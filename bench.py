@@ -2,8 +2,9 @@
 """bench.py — IA2C rollout-and-update throughput on B200 (agent-steps/s including the A2C update).
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA kernels through the C ABI)
-    python bench.py --impl reference --gpus N --steps K ...  # the UNMODIFIED reference loop (baseline/_ref/ia2c.py)
+    python bench.py --impl reference --gpus N --steps K ...  # the UNMODIFIED reference loop (oracle/_ref/ia2c.py)
                                                              # on the box's host cores
+    python bench.py --gpus 1 --steps K --dump-outputs DIR    # + the last timed headline step's outputs as DIR/*.npy
 
 A "step" is one IA2C episode: rollout of T=30 env steps for E envs x N agents (T+1 actor/belief evaluations)
 followed by the critic phase and the actor phase (ia2c.py:62-129).  The headline (`value`, `e2e`) is BASELINE.json
@@ -42,7 +43,9 @@ FLOPS_ROLLOUT, FLOPS_CRITIC, FLOPS_ACTOR = 210, 1512, 1044
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1000)
+    ap.add_argument("--steps", type=int, default=1000,
+                    help="timed steps per block of the headline; configs[] clamp K to their own range (cfg5 2..5 per GPU, cfg4 2..30, "
+                         "cfg3 3..30, cfg1 3..20) and report the steps they timed")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs-per-gpu", type=int, default=4096)
@@ -56,7 +59,13 @@ def parse():
     ap.add_argument("--skip-parity-check", action="store_true")
     ap.add_argument("--cpu-envs", type=int, default=4096, help="n_envs of the reference's ia2c.py CPU run")
     ap.add_argument("--cpu-budget-s", type=float, default=150.0, help="upper bound for the reference arm's CPU work")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed headline step computed to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs:
+        if args.impl != "ours":
+            ap.error("--dump-outputs needs --impl ours")
+        os.makedirs(args.dump_outputs, exist_ok=True)
+    return args
 
 
 def measured_peaks():
@@ -159,7 +168,7 @@ def cpu_port_rate(n_agents, sample_envs, min_seconds, max_steps=None, warmup=1):
 
 
 def ref_runner(*argv, timeout=900):
-    """Runs oracle/ref_runner.py (the UNMODIFIED reference files of baseline/_ref on the host CPU) in a fresh interpreter —
+    """Runs oracle/ref_runner.py (the UNMODIFIED reference files of oracle/_ref on the host CPU) in a fresh interpreter —
     the reference's module names (Org, ac_nets, belief_filter) must not meet the drop-in modules of this process.
     OMP/MKL thread limits that torchrun exports are dropped: the reference gets all the host threads it can use."""
     env = {k: v for k, v in os.environ.items() if k not in ("OMP_NUM_THREADS", "MKL_NUM_THREADS")}
@@ -191,7 +200,7 @@ def cpu_baseline_legs(n_envs):
 
 
 def run_reference(args):
-    """--impl reference: the reference's own CPU implementation of the path — baseline/_ref/ia2c.py, unmodified, executed by
+    """--impl reference: the reference's own CPU implementation of the path — oracle/_ref/ia2c.py, unmodified, executed by
     oracle/ref_runner.py at the headline config (n_envs = envs per GPU), every step one episode of its main loop."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -441,6 +450,30 @@ def make_trainer(ctx, E_total, N, fused=None, comm="auto", seed=1234, **kw):
                        rank=ctx.rank, world_size=ctx.world, fused_rollout=fused, comm=comm, **kw)
 
 
+DUMP_BYTES = 64_000_000
+NPY_HEADER_BYTES = 256   # allowance per file for the .npy header (128 bytes for these shapes)
+
+
+def dump_outputs(tr, out_dir, seed=0):
+    """Writes what the trainer's last episode handed its caller — losses, episode returns, updated parameters and the episode's
+    trajectory — as float32 / float64 DIR/<name>.npy, so that two builds can be compared output for output.  If the per-env
+    files would exceed DUMP_BYTES on disk in all, they keep a fixed, seeded sample of envs; env_index.npy holds the global indices kept."""
+    import numpy as np
+    h = lambda t: t.detach().cpu().numpy()
+    whole = {"critic_loss": h(tr.loss_out[0]), "actor_loss": h(tr.loss_out[1]),
+             "actor_params": h(tr.actor_params), "critic_params": h(tr.critic_params)}
+    per_env = {"ep_return": (h(tr.ep_return), 0), "obs": (h(tr.obs), 1), "reward": (h(tr.reward), 1),   # name -> (array, env axis)
+               "act": (h(tr.act).astype(np.float32), 1), "partner_pred": (h(tr.partner_pred).astype(np.float32), 1)}
+    env_bytes = sum(a.nbytes for a, _ in per_env.values()) // tr.E + 8
+    room = (DUMP_BYTES - sum(a.nbytes for a in whole.values()) - NPY_HEADER_BYTES * (len(whole) + len(per_env) + 1)) // env_bytes
+    keep = np.arange(tr.E) if tr.E <= room else np.sort(np.random.default_rng(seed).choice(tr.E, room, replace=False))
+    for name, a in whole.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    for name, (a, axis) in per_env.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.take(a, keep, axis=axis))
+    np.save(os.path.join(out_dir, "env_index.npy"), (tr.env_offset + keep).astype(np.float64))
+
+
 def parity_check(ctx, comm):
     """Multi-rank self-check INSIDE the bench run: the sharded trainer (same comm path as the timed run) against a
     single-rank trainer of the same total workload on every GPU, as tests/multigpu_parity.py does.  Trajectories of the
@@ -505,6 +538,8 @@ def bench_headline(ctx, args, _lib, peak_gbs, peak_src, sampler):
         blocks.append(ctx.max_over_ranks(total))
     launches = (_lib.launch_count() - launches0) // R
     tr.check_comm()
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(tr, args.dump_outputs)
     total_ms = statistics.median(blocks)
     # the rollout kernel on its own (single rank): the same steps as three calls with an event between the phases -- the
     # records cost the programmatic-launch overlap between the kernels (~2 us each), so this pass feeds `roofline` only
@@ -820,9 +855,11 @@ def bench_cfg1(ctx, updates, cpu):
     import contextlib
     import io
     from ia2c_b200 import launcher
-    path = os.path.join(ROOT, "baseline", "_ref", "a2c_org_test.py")
-    if not os.path.exists(path):
-        return {"config": "cfg1", "unavailable": "baseline/_ref/a2c_org_test.py not staged (python -m oracle.make_ref in the build container)"}
+    from oracle import ref_runner
+    ref, origin = ref_runner.find_reference()
+    if ref is None:
+        return {"config": "cfg1", "unavailable": f"the reference's a2c_org_test.py is not staged under oracle/_ref ({origin})"}
+    path = os.path.join(ref, "a2c_org_test.py")
     warm = 5
     stamps = []
     real_print = builtins.print
@@ -866,8 +903,11 @@ def run_ours(args):
     peaks, peak_src = measured_peaks()
     peak_gbs = float(peaks["hbm_gbs"])
     sampler = ClockSampler(ctx.local) if ctx.rank == 0 else None
-    line, comm, fused = bench_headline(ctx, args, _lib, peak_gbs, peak_src, sampler)
-    line["clocks"] = sampler.stop() if sampler else None
+    try:
+        line, comm, fused = bench_headline(ctx, args, _lib, peak_gbs, peak_src, sampler)
+    finally:   # the nvidia-smi sampler must not outlive a failed run
+        clocks = sampler.stop() if sampler else None
+    line["clocks"] = clocks
     single = ctx.world == 1
     # ---- multi-rank self-check on the same comm path the timed regions used
     if not single and not args.skip_parity_check:

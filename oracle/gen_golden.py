@@ -389,8 +389,23 @@ def gen_belief(out_name):
         out[f"{tag}/ap"] = np.stack(ap_l)
         out[f"{tag}/bprime"] = np.stack(b_l)
         out[f"{tag}/prediction"] = np.stack(p_l)
+        keep_envs(out, tag, BELIEF_KEEP_ENVS[tag])
     np.savez_compressed(os.path.join(OUT, out_name), **out)
     print("wrote", out_name)
+
+
+# envs stored per belief case: the class updates every env row on its own, so a fixed subset of rows is a complete record
+# of those rows, and it keeps belief_vectors.npz under 1 MB
+BELIEF_KEEP_ENVS = {"rand5": 64, "rand3": 32, "rand5x5": 16, "org_known": 32, "hvt_known": 16}
+
+
+def keep_envs(out, tag, n, seed=0):
+    """Keep a fixed, seeded subset of n envs (the second axis) in every per-step array of one belief case; prior0 stays
+    whole (it pins the class's initial prior), {tag}/env_index records the envs kept."""
+    keep = np.sort(np.random.RandomState(seed).choice(out[f"{tag}/obs"].shape[1], n, replace=False))
+    for k in ("other_action", "obs", "prev", "u", "ap", "bprime", "prediction"):
+        out[f"{tag}/{k}"] = out[f"{tag}/{k}"][:, keep]
+    out[f"{tag}/env_index"] = keep
 
 
 def gen_acnets(out_name):

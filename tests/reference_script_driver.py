@@ -4,7 +4,7 @@ Launched by tests/test_gpu_reference_scripts.py in a fresh interpreter whose mod
 ia2c_b200/compat and ia2c_b200/compat_gym, so the script's own ``from ac_nets import *``, ``from belief_filter
 import BeliefFilter``, ``import gymnasium`` and the gym entry point ``"Org:Org"`` (ia2c.py:20-38,
 a2c_org_test.py:16-19) resolve to the product's drop-in modules — the reference's module files are never on the path.
-The script source is read from baseline/_ref (or /root/reference), its loop length is set by text substitution on
+The script source is read from oracle/_ref (or the reference checkout), its loop length is set by text substitution on
 the in-memory source exactly as oracle/gen_golden.py did when it recorded the golden tapes, and it is exec'd as
 ``__main__``.
 

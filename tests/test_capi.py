@@ -86,19 +86,20 @@ def test_compat_modules_export_reference_names():
 
 
 @pytest.mark.parametrize("script", ["a2c_org_test.py", "ia2c.py"])
-def test_unmodified_reference_scripts_resolve_against_the_drop_in_modules(script):
-    """Build-container only: the reference's scripts, unmodified and run from where they lie, must import the drop-in
-    modules and reach the first CUDA call — where, without a GPU, the product raises its loud no-fallback error."""
+def test_unmodified_reference_scripts_resolve_against_the_drop_in_modules(script, tmp_path):
+    """Without a GPU: the reference's scripts, unmodified and run from where they lie, must import the drop-in
+    modules and reach the first CUDA call — where the product raises its loud no-fallback error."""
     import torch
-    ref = os.environ.get("IA2C_REFERENCE", "/root/reference")
-    if not os.path.exists(os.path.join(ref, script)):
-        pytest.skip("reference sources not present (GPU box)")
+    from oracle import ref_runner
+    ref, origin = ref_runner.find_reference()
+    if ref is None:
+        pytest.skip(f"reference sources not staged: {origin}")
     if torch.cuda.is_available():
         pytest.skip("CUDA present: the scripts would train for hours")
     env = dict(os.environ)
     env["PYTHONPATH"] = os.pathsep.join([ROOT, os.path.join(ROOT, "ia2c_b200", "compat"), os.path.join(ROOT, "ia2c_b200", "compat_gym")])
     # -P: do not put the script's own directory (which holds the reference modules) in front of PYTHONPATH
-    r = subprocess.run([sys.executable, "-P", os.path.join(ref, script)], capture_output=True, text=True, env=env, cwd="/tmp", timeout=300)
+    r = subprocess.run([sys.executable, "-P", os.path.join(ref, script)], capture_output=True, text=True, env=env, cwd=str(tmp_path), timeout=300)
     assert r.returncode != 0
     assert "no CPU fallback" in r.stderr, r.stderr[-2000:]
     assert "ModuleNotFoundError" not in r.stderr and "ImportError" not in r.stderr

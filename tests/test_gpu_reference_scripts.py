@@ -1,6 +1,6 @@
 """SURVEY.md §8 f1 / b1: the reference's own scripts, UNMODIFIED, executed on the GPU against the drop-in modules.
 
-tests/reference_script_driver.py exec's baseline/_ref/ia2c.py and baseline/_ref/a2c_org_test.py (staged by
+tests/reference_script_driver.py exec's oracle/_ref/ia2c.py and oracle/_ref/a2c_org_test.py (staged by
 oracle/make_ref.py, sha256-verified; loop length set by in-memory substitution as oracle/gen_golden.py did) in a
 fresh interpreter whose path resolves ``Org``, ``ac_nets``, ``belief_filter`` and ``gymnasium`` to
 ia2c_b200/compat(+compat_gym).  The golden run's sampled actions and np.random draws are replayed; everything the
@@ -27,7 +27,7 @@ def run_driver(script, golden_name, tmp_path):
     r = subprocess.run([sys.executable, "-P", os.path.join(ROOT, "tests", "reference_script_driver.py"), script,
                         os.path.join(GOLDEN, golden_name), out], capture_output=True, text=True, env=env, cwd=str(tmp_path), timeout=900)
     if r.returncode == 3 and "NO_REFERENCE" in r.stdout:
-        pytest.skip("baseline/_ref not staged (run python -m oracle.make_ref in the build container)")
+        pytest.skip("oracle/_ref not staged (IA2C_REFERENCE=<checkout of thinclab/IA2C> python -m oracle.make_ref)")
     assert r.returncode == 0 and "REFERENCE_SCRIPT_DONE" in r.stdout, r.stdout[-2000:] + r.stderr[-4000:]
     return np.load(out, allow_pickle=False), r.stdout
 

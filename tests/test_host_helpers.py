@@ -37,11 +37,11 @@ def test_staged_reference_manifest_detects_modification(tmp_path):
         make_ref.stage(str(tmp_path / "missing"), str(dst))
 
 
-def test_baseline_ref_is_git_ignored_but_travels_to_the_gpu_box():
+def test_staged_reference_is_git_ignored():
+    from oracle import make_ref
+
     ignore = open(os.path.join(ROOT, ".gitignore")).read().split()
-    assert "baseline/_ref/" in ignore
-    gpurunignore = os.path.join(ROOT, ".gpurunignore")
-    assert not os.path.exists(gpurunignore) or "baseline" not in open(gpurunignore).read()
+    assert make_ref.REF_DST == os.path.join(ROOT, "oracle", "_ref") and "oracle/_ref/" in ignore
 
 
 def test_hostmem_cpulist_parsing_and_bind_never_raises():

@@ -1,5 +1,5 @@
-import sys, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, numpy as np, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ia2c_b200.trainer import IA2CTrainer, reference_init
 E, N = 1024, 256
 init = reference_init(N, 5, seed=3)
