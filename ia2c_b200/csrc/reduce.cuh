@@ -45,12 +45,25 @@ __host__ __device__ inline ReduceArgs make_reduce_args(const ia2c_episode_desc& 
     return R;
 }
 
-// Adam's bias corrections for step t: {lr / (1 - b1^t) as float, sqrt(1 - b2^t) as float}.  Two fp64 pow() calls: computed by
-// ONE thread per block while the others' partial-row loads are in flight, and handed over through shared memory.
+// b^t by binary exponentiation: about 2 log2(t) DMULs, two of them per step independent, instead of pow()'s log/exp sequence.
+// Every multiply rounds once, so the relative error stays below 2 log2(t) * 2^-53 (< 7e-15 for any int32 t): far inside the
+// float rounding the bias corrections get below.
+__device__ __forceinline__ double pow_uint(double b, unsigned t) {
+    double r = 1.0;
+    for (; t; t >>= 1) {
+        if (t & 1u) r *= b;
+        b *= b;
+    }
+    return r;
+}
+
+// Adam's bias corrections for step t: {lr / (1 - b1^t) as float, sqrt(1 - b2^t) as float}.  They depend on the step counter the
+// gradient kernel has just bumped, so the reduce kernel computes them after its wait, in ONE thread per block whose result the
+// others pick up from shared memory: the powers by squaring keep that chain short.
 struct AdamBias { float step_size, bc2_sqrt; };
 __device__ __forceinline__ AdamBias adam_bias(int t, double lr) {
     const double b1 = 0.9, b2 = 0.999;
-    const double bc1 = 1.0 - pow(b1, (double)t), bc2 = 1.0 - pow(b2, (double)t);
+    const double bc1 = 1.0 - pow_uint(b1, (unsigned)t), bc2 = 1.0 - pow_uint(b2, (unsigned)t);
     AdamBias a;
     a.step_size = (float)(lr / bc1);
     a.bc2_sqrt = (float)sqrt(bc2);
@@ -68,8 +81,23 @@ __device__ __forceinline__ void adam_update(float& p, float& m, float& v, float 
 constexpr int kReduceSlices = 32;
 
 
-// what happens to entry i of agent n once its sum s is known (shared by both reduction routes)
-__device__ __forceinline__ void finish_entry(const ReduceArgs& R, int n, int i, float s, const AdamBias& bias) {
+// Adam operands of entry i of agent n (zero where the entry is not stepped).  Loaded right after the kernel's wait, together with
+// the partial rows, so that their memory round trip (from HBM when the cache is cold) is not a second one after the sum.
+struct AdamIn { float p, m, v, accum; };
+__device__ __forceinline__ AdamIn load_adam_in(const ReduceArgs& R, int n, int i) {
+    AdamIn a = {0.f, 0.f, 0.f, 0.f};
+    if (R.apply_adam && i < R.P) {
+        const int64_t k = (int64_t)n * R.P + i;
+        a.p = R.params[k];
+        a.m = R.m[k];
+        a.v = R.v[k];
+        if (R.grad_accum) a.accum = R.grad_accum[k];
+    }
+    return a;
+}
+
+// what happens to entry i of agent n once its sum s is known; `in` = load_adam_in(R, n, i)
+__device__ __forceinline__ void finish_entry(const ReduceArgs& R, int n, int i, float s, const AdamBias& bias, const AdamIn& in) {
     const int P = R.P;
     if (R.from_partials) {
         if (i == P) s *= R.loss_scale;
@@ -81,10 +109,14 @@ __device__ __forceinline__ void finish_entry(const ReduceArgs& R, int n, int i, 
         const int64_t k = (int64_t)n * P + i;
         float g = s;
         if (R.grad_accum) {                  // the reference's actor never zeroes its gradients (Q2)
-            g += R.grad_accum[k];
+            g += in.accum;
             R.grad_accum[k] = g;
         }
-        adam_update(R.params[k], R.m[k], R.v[k], g, bias);
+        float p = in.p, m = in.m, v = in.v;
+        adam_update(p, m, v, g, bias);
+        R.params[k] = p;
+        R.m[k] = m;
+        R.v[k] = v;
     }
 }
 

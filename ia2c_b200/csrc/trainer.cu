@@ -497,6 +497,8 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
 // grid (N, ceil((P+1)/32)); block 1024 = 32 entries x 32 slices of the partial blocks; fixed-order sums.
 // The partials are L2-resident, so a thread's chain of dependent adds costs one L2 round trip per term: many
 // short slices (<= 8 terms at 256 partial blocks, loads issued back to back) instead of few long ones.
+// Everything the update reads is requested right after the wait — the partial rows (every slice), the Adam operands (slice 0)
+// and the step counter (the bias thread) — so the kernel costs one memory round trip before its barrier and none after it.
 __global__ void __launch_bounds__(32 * kReduceSlices) reduce_adam_kernel(ReduceArgs R) {
     pdl_prologue();
     KSTAMP(g_kclock, R.P == kCriticP ? 0 : 10);
@@ -505,8 +507,9 @@ __global__ void __launch_bounds__(32 * kReduceSlices) reduce_adam_kernel(ReduceA
     const int i = blockIdx.y * 32 + col;
     __shared__ float part[kReduceSlices][33];
     __shared__ AdamBias bias;
-    if (threadIdx.x == blockDim.x - 1 && R.apply_adam)   // step[n] was already incremented by the gradient kernel / apply entry
-        bias = adam_bias(__ldcg(R.step + n), R.lr);
+    const bool bias_thread = threadIdx.x == blockDim.x - 1 && R.apply_adam;
+    const int t = bias_thread ? __ldcg(R.step + n) : 0;   // step[n] was already incremented by the gradient kernel / apply entry
+    const AdamIn in = (slice == 0 && i <= P) ? load_adam_in(R, n, i) : AdamIn{0.f, 0.f, 0.f, 0.f};
     float s = 0.f;
     if (i <= P) {
         if (R.from_partials) {
@@ -525,12 +528,13 @@ __global__ void __launch_bounds__(32 * kReduceSlices) reduce_adam_kernel(ReduceA
             s = R.grad[(int64_t)n * (P + 1) + i];
         }
     }
+    if (bias_thread) bias = adam_bias(t, R.lr);
     part[slice][col] = s;
     __syncthreads();
     if (slice != 0 || i > P) return;
 #pragma unroll
     for (int k = 1; k < kReduceSlices; ++k) s += part[k][col];
-    finish_entry(R, n, i, s, bias);
+    finish_entry(R, n, i, s, bias, in);
     KSTAMP(g_kclock, R.P == kCriticP ? 3 : 13);
 }
 
