@@ -25,4 +25,7 @@ def __getattr__(name):  # lazy: torch-dependent classes are imported on first us
     if name in ("IA2CTrainer", "reference_init"):
         from . import trainer
         return getattr(trainer, name)
+    if name == "IA2CRuns":
+        from .runs import IA2CRuns
+        return IA2CRuns
     raise AttributeError(name)

@@ -22,7 +22,8 @@ FLAG_ACTOR_COLUMNS = 16
 FLAG_BELIEF_PER_STEP = 32
 FLAG_ROLLOUT_PER_STEP = 64
 BELIEF_RECORD = 8
-ABI_VERSION = 2
+ABI_VERSION = 3
+MAX_RUN_NETS = 65535   # IA2C_MAX_RUN_NETS: runs * n_agents of one batch
 ACTOR_P = 105
 CRITIC_P = 147
 
@@ -55,6 +56,11 @@ class PeerDesc(C.Structure):
     """Mirror of ``ia2c_peer_desc``."""
     _fields_ = [("rank", i32), ("world", i32), ("inbox", vp * 8), ("mc_inbox", vp), ("error", vp * 8),
                 ("timeout_us", u32), ("reserved", u32)]
+
+
+class RunsDesc(C.Structure):
+    """Mirror of ``ia2c_runs_desc``: a batch of independent runs (ia2c_train_episode_runs)."""
+    _fields_ = [("runs", i32), ("reserved", i32), ("seed", vp), ("lr_actor", vp), ("lr_critic", vp), ("gamma", vp), ("beta", vp)]
 
 
 _DP = C.POINTER(EpisodeDesc)
@@ -106,6 +112,8 @@ SIGNATURES = {
     "ia2c_host_stage_stride": (C.c_size_t, [_DP]),
     "ia2c_train_episodes_host": (C.c_int, [_DP, vp, vp, vp, i32, C.POINTER(vp), vp, vp]),
     "ia2c_train_episodes_host_p2p": (C.c_int, [_DP, vp, C.POINTER(PeerDesc), u32, vp, vp, i32, C.POINTER(vp), vp, vp]),
+    "ia2c_runs_partials_floats": (C.c_size_t, [_DP, i32]),
+    "ia2c_train_episode_runs": (C.c_int, [_DP, C.POINTER(RunsDesc), vp]),
 }
 
 _lib = None

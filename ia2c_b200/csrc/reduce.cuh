@@ -45,6 +45,22 @@ __host__ __device__ inline ReduceArgs make_reduce_args(const ia2c_episode_desc& 
     return R;
 }
 
+// Per-run learning rates of a batch of runs (reduce_adam_kernel<true>): net n belongs to run n / N; lr == NULL -> ReduceArgs.lr.
+struct ReduceRuns {
+    const double* lr;
+    int N;
+};
+template <bool RUNS>
+using ReduceRunsArg = std::conditional_t<RUNS, ReduceRuns, NoRuns>;
+template <bool RUNS>
+__device__ __forceinline__ double reduce_lr(const ReduceArgs& R, const ReduceRunsArg<RUNS>& rr, int n) {
+    if constexpr (RUNS) {
+        return rr.lr ? rr.lr[n / rr.N] : R.lr;
+    } else {
+        return R.lr;
+    }
+}
+
 // b^t by binary exponentiation: about 2 log2(t) DMULs, two of them per step independent, instead of pow()'s log/exp sequence.
 // Every multiply rounds once, so the relative error stays below 2 log2(t) * 2^-53 (< 7e-15 for any int32 t): far inside the
 // float rounding the bias corrections get below.

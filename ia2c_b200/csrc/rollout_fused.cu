@@ -69,8 +69,9 @@ __device__ __forceinline__ void obs_from_cls(int packed, float (&x)[F]) {
     }
 }
 
-template <int N, int M, bool CRITIC>
-__global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc d, float* __restrict__ partials) {
+// RUNS: a batch of independent runs (ia2c_train_episode_runs), blockIdx.y = run; see `run` below.
+template <int N, int M, bool CRITIC, bool RUNS>
+__global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc d, float* __restrict__ partials, RunsArg<RUNS> ra) {
     constexpr int K = N - 1;
     constexpr int G = N <= 2 ? 2 : (N <= 4 ? 4 : 8);     // lanes per env
     constexpr int EPW = 32 / G;
@@ -88,10 +89,15 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
     __shared__ float4 dy_s[4][CRITIC ? 32 : 1];          // row t's output gradients {jt, dQ[jt], nja, dQ'[nja]}, slot t & 3
     __shared__ float red_s[CRITIC ? kCriticP + 1 : 1][33];   // per-lane gradient partials for the block-wide reduction at the end
     KCLOCK(sc_entry);
+    // A run of a batch owns net rows [run * N, (run + 1) * N) and env columns [run * E, (run + 1) * E) of an env axis of length
+    // R * E (stride ES); `e` stays the env's index within its run, which keys its Philox counters.  ia2c_train_episode_runs
+    // refuses replay tapes and parity dumps, so the code that indexes them by `e` and E never runs in a batch.
+    const int run = RUNS ? (int)blockIdx.y : 0;
+    const int net0 = run * N;
     pdl_release();
     // constants of the run (k/100, the agents' models): staged while the previous kernel of the stream may still be running
     for (int k = threadIdx.x; k <= 100; k += blockDim.x) tab[k] = __ddiv_rn((double)k, 100.0);
-    for (int k = threadIdx.x; k < N * M * A; k += blockDim.x) fa_s[k] = d.filter_action[k];
+    for (int k = threadIdx.x; k < N * M * A; k += blockDim.x) fa_s[k] = d.filter_action[(int64_t)net0 * M * A + k];
     __syncthreads();
     pdl_wait();   // parameters (updated by the previous episode's Adam steps) are read only after this
     KCLOCK(sc_waited);
@@ -102,6 +108,8 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
     const int leader = lane & ~(G - 1);
     const int64_t e = (int64_t)blockIdx.x * EPW + (lane / G);
     const int64_t E = d.E;
+    const int64_t ES = RUNS ? E * gridDim.y : E;
+    const int64_t ge = RUNS ? (int64_t)run * E + e : e;
     const bool live = e < E;            // uniform over the env's lane group
     const bool agent = live && sub < N; // this lane owns agent `sub`
     const int i = sub < N ? sub : 0;
@@ -131,7 +139,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
     auto draw_action_from = [&](float& ua, int t) {
         if (t <= T && agent)
             ua_s[t & 1][lane] = inj_a ? ua
-                                      : philox_uniform_f32(d.seed, kStreamAction, d.episode, (uint32_t)t,
+                                      : philox_uniform_f32(run_seed<RUNS>(d, ra, run), kStreamAction, d.episode, (uint32_t)t,
                                                            (uint64_t)((d.env_offset + e) * N + i));
         fetch_a(ua, t + 2);
     };
@@ -143,7 +151,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
             } else {
 #pragma unroll
                 for (int sl = 0; sl < (K + 3) / 4; ++sl) {
-                    const uint4 r = philox_belief_quad(d.seed, d.episode, (uint32_t)t, (uint64_t)((d.env_offset + e) * N + i), K, sl);
+                    const uint4 r = philox_belief_quad(run_seed<RUNS>(d, ra, run), d.episode, (uint32_t)t, (uint64_t)((d.env_offset + e) * N + i), K, sl);
                     ub_s[t & 3][4 * sl][lane] = belief_word_to_unit_f64(r.x);
                     if (4 * sl + 1 < K) ub_s[t & 3][4 * sl + 1][lane] = belief_word_to_unit_f64(r.y);
                     if (4 * sl + 2 < K) ub_s[t & 3][4 * sl + 2][lane] = belief_word_to_unit_f64(r.z);
@@ -163,17 +171,17 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
     if (role == 1) {
         // ================================================================ A: env + actor, step t = it - 1
         RegNet<A> net;
-        load_regnet<A>(net, d.actor_params + i * kActorP);
+        load_regnet<A>(net, d.actor_params + (net0 + i) * kActorP);
         int s = 2, prev_cls = 1, cur_cls = 1, elapsed = 0;   // env state, replicated in the group's lanes
         double hist = 0.0, ep_ret = 0.0;
         const double rcp10 = drcp_seq(10.0);
         int a = 0;
         // running output pointers (one bump per step instead of 64-bit index arithmetic)
-        float* obs_p = d.obs + e * F;
-        uint8_t* act_p = d.act + e * N + i;
-        uint8_t* ptrue_p = d.partner_true + e * N + i;
+        float* obs_p = d.obs + ge * F;
+        uint8_t* act_p = d.act + ge * N + i;
+        uint8_t* ptrue_p = d.partner_true + ge * N + i;
         const uint8_t* inj_p = d.inj_actions ? d.inj_actions + e * N + i : nullptr;
-        float* rew_p = d.reward + e;
+        float* rew_p = d.reward + ge;
         int32_t* trace_p = d.state_trace ? d.state_trace + e : nullptr;
         double* rew64_p = d.reward_f64 ? d.reward_f64 + e : nullptr;
         const int max_steps = d.max_episode_steps;
@@ -198,7 +206,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
                         if (trace_p) *trace_p = s2;
                         if (rew64_p) *rew64_p = r;
                     }
-                    rew_p += E;
+                    rew_p += ES;
                     if (trace_p) trace_p += E;
                     if (rew64_p) rew64_p += E;
                     ++elapsed;
@@ -219,7 +227,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
                     for (int k = 0; k < F; ++k)
                         if ((k % G) == sub) obs_p[k] = x[k];
                 }
-                obs_p += E * F;
+                obs_p += ES * F;
                 if (inj_p) {
                     a = agent ? *inj_p : 0;
                     inj_p += E * N;
@@ -242,18 +250,18 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
                     *act_p = (uint8_t)a;
                     *ptrue_p = (uint8_t)pt;
                 }
-                act_p += E * N;
-                ptrue_p += E * N;
+                act_p += ES * N;
+                ptrue_p += ES * N;
             }
             STAGE_SYNC();
         }
         KCLOCK(sc_loop_end);
         if (live && sub == 0) {   // persist the final env state exactly as the per-step path leaves it
-            d.env_state[e] = s;
-            d.env_hist[e] = hist;
-            d.env_elapsed[e] = elapsed;
-            d.ep_return[e] = ep_ret;
-            *reinterpret_cast<uchar2*>(d.env_cls + 2 * e) = make_uchar2((unsigned char)prev_cls, (unsigned char)cur_cls);
+            d.env_state[ge] = s;
+            d.env_hist[ge] = hist;
+            d.env_elapsed[ge] = elapsed;
+            d.ep_return[ge] = ep_ret;
+            *reinterpret_cast<uchar2*>(d.env_cls + 2 * ge) = make_uchar2((unsigned char)prev_cls, (unsigned char)cur_cls);
         }
         STAGE_CLOCK_EXIT("A");
     } else if (role == 2) {
@@ -268,7 +276,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
         int last_pred[K];
 #pragma unroll
         for (int jj = 0; jj < K; ++jj) last_pred[jj] = 0;
-        uint8_t* ppred_p = d.partner_pred + e * N + i;
+        uint8_t* ppred_p = d.partner_pred + ge * N + i;
         if (CRITIC) draw_action_init();
         STAGE_CLOCK_INIT;
         for (int it = 0; it < n_iter; ++it) {
@@ -330,7 +338,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
                 const int pp = mode3(pc0, pc1, pc2);
                 ppred_s[t & (kRing - 1)][lane] = pp;
                 if (agent) *ppred_p = (uint8_t)pp;
-                ppred_p += E * N;
+                ppred_p += ES * N;
             }
             STAGE_SYNC();
         }
@@ -344,7 +352,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
                     if (m < 4) lo |= (uint32_t)bel[jj][m] << (8 * m); else hi |= (uint32_t)bel[jj][m] << (8 * (m - 4));
                 }
                 hi |= (uint32_t)last_pred[jj] << 16;
-                *reinterpret_cast<uint2*>(d.belief_records + ((e * N + i) * (int64_t)K + jj) * IA2C_BELIEF_RECORD) = make_uint2(lo, hi);
+                *reinterpret_cast<uint2*>(d.belief_records + ((ge * N + i) * (int64_t)K + jj) * IA2C_BELIEF_RECORD) = make_uint2(lo, hi);
             }
         }
         STAGE_CLOCK_EXIT("B");
@@ -366,11 +374,11 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
         // One forward per observation: obs[t+1] is evaluated as the "next" observation of row t, its
         // activations are parked in shared memory for the backward stage, and the two Q values it will be
         // asked for (as bootstrap of row t, as Q(obs)[jt] of row t+1) are selected right away.
-        const float gamma = d.gamma;
+        const float gamma = run_gamma<RUNS>(d, ra, run);
         float loss = 0.f;
         float q_cur_jt = 0.f;
         RegNet<J> cnet;                      // this lane's critic, forward-paired weights in registers
-        load_regnet<J>(cnet, d.critic_params + (int64_t)i * kCriticP);
+        load_regnet<J>(cnet, d.critic_params + (int64_t)(net0 + i) * kCriticP);
         float2 gB[21];                       // W1 | b1 gradient (the backprop warp hands dz1 over, one iteration later)
 #pragma unroll
         for (int k = 0; k < 21; ++k) gB[k] = make_float2(0.f, 0.f);
@@ -428,7 +436,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
 #pragma unroll
         for (int k = 0; k < 21; ++k) { red_s[2 * k][lane] = gB[k].x; red_s[2 * k + 1][lane] = gB[k].y; }
         red_s[P][lane] = loss;
-        if (lane < N && blockIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.critic_step[lane] += 1;
+        if (lane < N && blockIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.critic_step[net0 + lane] += 1;
         STAGE_CLOCK_EXIT("Cf");
     } else {
     // ==================================================================== Cb: critic backward, observation t = it - 5
@@ -437,7 +445,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
     // stay in registers for the whole episode.
     constexpr int GA = GN - 21;          // float2 accumulators for flat entries [42, 148): W2 | b2 | W3 | b3 (| loss slot)
     RegBack<J> back;
-    load_regback<J>(back, d.critic_params + (int64_t)i * kCriticP);
+    load_regback<J>(back, d.critic_params + (int64_t)(net0 + i) * kCriticP);
     float2 gA[GA];
 #pragma unroll
     for (int k = 0; k < GA; ++k) gA[k] = make_float2(0.f, 0.f);
@@ -489,18 +497,23 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
             float sum = red_s[entry][a];
 #pragma unroll
             for (int j = 1; j < EPW; ++j) sum += red_s[entry][a + G * j];
-            partials[((int64_t)a * gridDim.x + blockIdx.x) * P1 + entry] = sum;
+            partials[((int64_t)(net0 + a) * gridDim.x + blockIdx.x) * P1 + entry] = sum;
         }
     }
 }
 
 template <int N, int M>
-int launch(const ia2c_episode_desc* d, cudaStream_t s) {
+int launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s) {
     constexpr int G = N <= 2 ? 2 : (N <= 4 ? 4 : 8);
     const int64_t blocks = (d->E + (32 / G) - 1) / (32 / G);   // one block = 4 stage warps over 32/G envs
+    if (runs)   // every run with its own row of blocks, partitioned as a standalone run of E envs
+        return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, true, true>, dim3((unsigned)blocks, (unsigned)runs->runs),
+                          dim3(kBlock), 0, s, *d, d->partials, *runs);
     if (d->flags & IA2C_FLAG_FUSED_CRITIC)
-        return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, true>, dim3((unsigned)blocks), dim3(kBlock), 0, s, *d, d->partials);
-    return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, false>, dim3((unsigned)blocks), dim3(kBlock), 0, s, *d, nullptr);
+        return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, true, false>, dim3((unsigned)blocks), dim3(kBlock), 0, s, *d,
+                          d->partials, NoRuns{});
+    return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, false, false>, dim3((unsigned)blocks), dim3(kBlock), 0, s, *d,
+                      nullptr, NoRuns{});
 }
 
 }  // namespace
@@ -514,16 +527,17 @@ int64_t rollout_fused_blocks(int64_t E, int N) {
     return (E + (32 / G) - 1) / (32 / G);
 }
 
-int rollout_fused_launch(const ia2c_episode_desc* d, cudaStream_t s) {
-    if (d->M == 3 && d->N == 2) return launch<2, 3>(d, s);
+// runs != nullptr: all runs of a batch (ia2c_train_episode_runs), always with the critic-gradient stage.
+int rollout_fused_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s) {
+    if (d->M == 3 && d->N == 2) return launch<2, 3>(d, runs, s);
     switch (d->N) {
-        case 2: return launch<2, 5>(d, s);
-        case 3: return launch<3, 5>(d, s);
-        case 4: return launch<4, 5>(d, s);
-        case 5: return launch<5, 5>(d, s);
-        case 6: return launch<6, 5>(d, s);
-        case 7: return launch<7, 5>(d, s);
-        case 8: return launch<8, 5>(d, s);
+        case 2: return launch<2, 5>(d, runs, s);
+        case 3: return launch<3, 5>(d, runs, s);
+        case 4: return launch<4, 5>(d, runs, s);
+        case 5: return launch<5, 5>(d, runs, s);
+        case 6: return launch<6, 5>(d, runs, s);
+        case 7: return launch<7, 5>(d, runs, s);
+        case 8: return launch<8, 5>(d, runs, s);
     }
     set_error("rollout_fused: no instantiation for N=%d M=%d", d->N, d->M);
     return IA2C_ERR_UNSUPPORTED;

@@ -33,7 +33,7 @@
 
 namespace ia2c {
 int rollout_fused_supported(int N, int M);                                  // rollout_fused.cu
-int rollout_fused_launch(const ia2c_episode_desc* d, cudaStream_t s);
+int rollout_fused_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s);
 int64_t rollout_fused_blocks(int64_t E, int N);
 int actor_pipe_launch(const ia2c_episode_desc* d, cudaStream_t s);
 int64_t actor_pipe_blocks(int64_t E, int N);
@@ -380,7 +380,10 @@ __global__ void __launch_bounds__(kGradThreads) critic_grad_kernel(ia2c_episode_
     block_reduce_store<P + 1>(reinterpret_cast<float(&)[P + 1]>(g), red, partials + ((int64_t)n * gridDim.x + blockIdx.x) * (P + 1));
 }
 
-__global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_desc d, float* __restrict__ partials) {
+// RUNS: a batch of independent runs (ia2c_train_episode_runs): blockIdx.y = run * N + agent is the net row, the run's envs are
+// columns [run * E, (run + 1) * E) of an env axis of length R * E (stride ES).
+template <bool RUNS>
+__global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_desc d, float* __restrict__ partials, RunsArg<RUNS> ra) {
     constexpr int P = kActorP, PC = kCriticP, GN = F2<A>::G2;   // 106 floats = 53 float2
     __shared__ __align__(16) float wc[SmemNet<J>::size];
     __shared__ __align__(16) float w[SmemNet<A>::size];
@@ -390,13 +393,15 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
     pdl_prologue();
     KCLOCK(k_waited);
     KSTAMP(g_kclock, 5);
-    const int n = blockIdx.y, N = d.N;
-    stage_smemnet<J>(wc, d.critic_params + (int64_t)n * PC);
-    stage_smemnet<A>(w, d.actor_params + (int64_t)n * P);
-    if (blockIdx.x == 0 && threadIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.actor_step[n] += 1;
+    const int N = d.N, n = RUNS ? (int)blockIdx.y % N : blockIdx.y;   // n: the agent
+    const int run = RUNS ? (int)blockIdx.y / N : 0;
+    stage_smemnet<J>(wc, d.critic_params + (int64_t)(RUNS ? blockIdx.y : n) * PC);
+    stage_smemnet<A>(w, d.actor_params + (int64_t)(RUNS ? blockIdx.y : n) * P);
+    if (blockIdx.x == 0 && threadIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.actor_step[RUNS ? blockIdx.y : n] += 1;
     __syncthreads();
     KCLOCK(k_staged);
     const int64_t E = d.E, rows = (int64_t)d.T * E;
+    const int64_t ES = RUNS ? E * (gridDim.y / N) : E;
     const ChunkPlan cp = chunk_plan(d.T, E, N);
     const int64_t items = E * cp.n_chunks;
     const float inv_b = 1.f / (float)((int64_t)d.T * d.E_total);
@@ -405,11 +410,11 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
     for (int i = 0; i < GN; ++i) g2[i] = make_float2(0.f, 0.f);
     float loss = 0.f;
     for (int64_t item = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; item < items; item += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t e = item % E;
+        const int64_t e = RUNS ? (int64_t)run * E + item % E : item % E;
         const int t0 = (int)(item / E) * cp.chunk_len;
         const int t1 = min(d.T, t0 + cp.chunk_len);
         float x[kIn], q[J];
-        load_obs6(d.obs + ((int64_t)t0 * E + e) * kIn, x);
+        load_obs6(d.obs + ((int64_t)t0 * ES + e) * kIn, x);
         {
             float2 h1[3], h2[3];
             fwd_f2<J>(wc, x, h1, h2, q);
@@ -419,17 +424,17 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
         // during iteration t-1 and carries its own action / predicted partner over from the previous row.
         struct RowIn { float xn[kIn]; int own_n, pp_n; float rew; };
         auto fetch = [&](int t, RowIn& in) {
-            const int64_t r = (int64_t)t * E + e;
-            load_obs6(d.obs + (r + E) * kIn, in.xn);                 // next_obs[t] = obs[t+1]
-            in.own_n = d.act[(r + E) * N + n];
-            in.pp_n = d.partner_pred[(r + E) * N + n];
+            const int64_t r = (int64_t)t * ES + e;
+            load_obs6(d.obs + (r + ES) * kIn, in.xn);                 // next_obs[t] = obs[t+1]
+            in.own_n = d.act[(r + ES) * N + n];
+            in.pp_n = d.partner_pred[(r + ES) * N + n];
             in.rew = d.reward[r];
         };
         RowIn cur;
         fetch(t0, cur);
-        int own = d.act[((int64_t)t0 * E + e) * N + n], pp = d.partner_pred[((int64_t)t0 * E + e) * N + n];
+        int own = d.act[((int64_t)t0 * ES + e) * N + n], pp = d.partner_pred[((int64_t)t0 * ES + e) * N + n];
         for (int t = t0; t < t1; ++t) {
-            const int64_t r = (int64_t)t * E + e;
+            const int64_t r = (int64_t)t * ES + e;
             RowIn nxt = cur;
             if (t + 1 < t1) fetch(t + 1, nxt);
             float qn[J];
@@ -440,8 +445,14 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
             const int own_n = cur.own_n;
             const int ja = joint_index(n, N, own, pp);                                   // ia2c.py:120-121
             const int nja = joint_index(n, N, own_n, cur.pp_n);
-            const float adv = (cur.rew + d.gamma * select_out<J>(qn, nja)) - select_out<J>(q, ja);
-            if (d.adv_dump) d.adv_dump[(int64_t)n * rows + r] = adv;
+            // RUNS spells out, with rounding intrinsics, the contractions nvcc 12.9 makes in the standalone instantiation (read
+            // off its SASS: FFMA for rew + gamma * Q', for adv * (-log q) - beta * H, for the entropy terms and for the own
+            // action's beta * (..) - adv / q except at the last action): with gamma / beta loaded per run instead of read from
+            // the parameter bank the compiler contracts differently, and the batch's runs would drift from the standalone runs
+            // in the last bit.  tests/test_gpu_runs.py checks the two byte for byte.
+            const float adv = RUNS ? __fmaf_rn(run_gamma<RUNS>(d, ra, run), select_out<J>(qn, nja), cur.rew) - select_out<J>(q, ja)
+                                   : (cur.rew + run_gamma<RUNS>(d, ra, run) * select_out<J>(qn, nja)) - select_out<J>(q, ja);
+            if (d.adv_dump) d.adv_dump[(int64_t)n * rows + r] = adv;   // never in a batch (refused)
             float2 h1[3], h2[3];
             float p[A];
             fwd_f2<A>(w, x, h1, h2, p);
@@ -456,17 +467,29 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
                 const float qv = p[o] / s;
                 const bool inside = (qv >= kEpsClamp) && (qv <= 1.f - kEpsClamp);
                 const float logit = logf(fminf(fmaxf(qv, kEpsClamp), 1.f - kEpsClamp));
-                ent -= logit * qv;
-                float go = d.beta * (logit + (inside ? 1.f : 0.f));
-                if (o == own) {
-                    neglogp = -logit;
-                    if (inside) go -= adv / qv;
+                float go;
+                if constexpr (RUNS) {
+                    const float beta = run_beta<RUNS>(d, ra, run), lc = logit + (inside ? 1.f : 0.f);
+                    ent = __fmaf_rn(-logit, qv, ent);
+                    if (o == own && inside)   // (the standalone build fuses this for the first two actions, not the last)
+                        go = o < A - 1 ? __fmaf_rn(beta, lc, -__fdiv_rn(adv, qv)) : __fsub_rn(__fmul_rn(beta, lc), __fdiv_rn(adv, qv));
+                    else
+                        go = __fmul_rn(beta, lc);
+                    if (o == own) neglogp = -logit;
+                } else {
+                    ent -= logit * qv;
+                    go = run_beta<RUNS>(d, ra, run) * (logit + (inside ? 1.f : 0.f));
+                    if (o == own) {
+                        neglogp = -logit;
+                        if (inside) go -= adv / qv;
+                    }
                 }
                 gq[o] = go;
                 qq[o] = qv;
                 qg = fmaf(qv, go, qg);
             }
-            loss += adv * neglogp - d.beta * ent;
+            if constexpr (RUNS) loss += __fmaf_rn(adv, neglogp, -__fmul_rn(run_beta<RUNS>(d, ra, run), ent));
+            else loss += adv * neglogp - run_beta<RUNS>(d, ra, run) * ent;
             float dy[A];
 #pragma unroll
             for (int o = 0; o < A; ++o) dy[o] = qq[o] * (gq[o] - qg) * inv_b;   // through normalise + softmax
@@ -485,7 +508,7 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
     float g[2 * GN];
     unpack_g2(g2, g);
     g[P] = loss;
-    block_reduce_store<P + 1>(reinterpret_cast<float(&)[P + 1]>(g), red, partials + ((int64_t)n * gridDim.x + blockIdx.x) * (P + 1));
+    block_reduce_store<P + 1>(reinterpret_cast<float(&)[P + 1]>(g), red, partials + ((int64_t)(RUNS ? blockIdx.y : n) * gridDim.x + blockIdx.x) * (P + 1));
     KSTAMP(g_kclock, 7);
     KCLOCK_PRINT(d.episode == 5 && (blockIdx.x == 0 || blockIdx.x == gridDim.x - 1) && blockIdx.y == 0 && threadIdx.x == 0,
                  "actor_grad block %3d entry %llu: waited +%llu, staged +%llu, rows done +%llu, exit +%llu ns\n", (int)blockIdx.x,
@@ -499,7 +522,9 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
 // short slices (<= 8 terms at 256 partial blocks, loads issued back to back) instead of few long ones.
 // Everything the update reads is requested right after the wait — the partial rows (every slice), the Adam operands (slice 0)
 // and the step counter (the bias thread) — so the kernel costs one memory round trip before its barrier and none after it.
-__global__ void __launch_bounds__(32 * kReduceSlices) reduce_adam_kernel(ReduceArgs R) {
+// RUNS: the R * N nets of a batch of runs (ia2c_train_episode_runs); net n belongs to run n / N and steps with that run's lr.
+template <bool RUNS>
+__global__ void __launch_bounds__(32 * kReduceSlices) reduce_adam_kernel(ReduceArgs R, ReduceRunsArg<RUNS> rr) {
     pdl_prologue();
     KSTAMP(g_kclock, R.P == kCriticP ? 0 : 10);
     const int n = blockIdx.x, P = R.P;
@@ -528,7 +553,7 @@ __global__ void __launch_bounds__(32 * kReduceSlices) reduce_adam_kernel(ReduceA
             s = R.grad[(int64_t)n * (P + 1) + i];
         }
     }
-    if (bias_thread) bias = adam_bias(t, R.lr);
+    if (bias_thread) bias = adam_bias(t, reduce_lr<RUNS>(R, rr, n));
     part[slice][col] = s;
     __syncthreads();
     if (slice != 0 || i > P) return;
@@ -585,7 +610,7 @@ static int actor_partial_blocks(const ia2c_episode_desc* d) {
 static int launch_actor_grad(const ia2c_episode_desc* d, cudaStream_t s) {
     if (!actor_columns(d)) return actor_pipe_launch(d, s);
     dim3 grid(grad_blocks(d), d->N);
-    return launch_pdl("actor_grad_kernel", actor_grad_kernel, grid, dim3(kGradThreads), 0, s, *d, d->partials);
+    return launch_pdl("actor_grad_kernel", actor_grad_kernel<false>, grid, dim3(kGradThreads), 0, s, *d, d->partials, NoRuns{});
 }
 
 extern "C" size_t ia2c_episode_partials_floats(const ia2c_episode_desc* d) {
@@ -608,7 +633,7 @@ extern "C" int ia2c_rollout(const ia2c_episode_desc* d, void* stream) {
             IA2C_REQUIRE(d->partials && d->partials_floats >= ia2c_episode_partials_floats(d) && d->critic_step,
                          "ia2c_rollout: IA2C_FLAG_FUSED_CRITIC needs the partials workspace and critic_step");
         }
-        return rollout_fused_launch(d, s);
+        return rollout_fused_launch(d, nullptr, s);
     }
     const bool episode_beliefs = !(d->flags & IA2C_FLAG_BELIEF_PER_STEP) && ia2c_belief_supports_episode(d->N, d->M);
     if (episode_beliefs && !(d->flags & IA2C_FLAG_ROLLOUT_PER_STEP) && d->N <= 256) {
@@ -677,7 +702,7 @@ static int run_reduce(const ia2c_episode_desc* d, int which, int from_partials, 
         if (int rc = check_launch("bump_steps_kernel")) return rc;
     }
     dim3 grid(d->N, ceil_div(R.P + 1, 32));
-    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel, grid, dim3(32 * kReduceSlices), 0, s, R);
+    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<false>, grid, dim3(32 * kReduceSlices), 0, s, R, NoRuns{});
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1188,6 +1213,67 @@ extern "C" int ia2c_allreduce_adam(const ia2c_episode_desc* d, int32_t which, co
     const int total = d->N * chunks_per_agent;
     const int grid = std::min(total, kSMs);          // persistent: every block is resident
     return launch_pdl("allreduce_adam_kernel", allreduce_adam_kernel, dim3(grid), dim3(32 * kReduceSlices), 0, s, R, X, total, chunks_per_agent);
+}
+
+// ------------------------------------------------------------------------------------------------
+// A batch of R independent runs in the four launches of one episode (include/ia2c_b200.h: ia2c_train_episode_runs).  Every
+// kernel takes the run as one more grid dimension and partitions each run as a standalone run of E envs is partitioned:
+// rollout grid (rollout_fused_blocks(E, N), R), actor-gradient grid (grad_blocks(E), R * N), reduce grid (R * N, chunks).
+extern "C" size_t ia2c_runs_partials_floats(const ia2c_episode_desc* d, int32_t runs) {
+    if (runs < 1) return 0;
+    return (size_t)runs * ia2c_episode_partials_floats(d);
+}
+
+static int validate_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r) {
+    const char* who = "ia2c_train_episode_runs";
+    if (int rc = validate(d, who)) return rc;
+    IA2C_REQUIRE(r != nullptr, "%s: null runs descriptor", who);
+    IA2C_REQUIRE(r->runs >= 1, "%s: runs=%d, need at least 1", who, r->runs);
+    IA2C_REQUIRE((int64_t)r->runs * d->N <= IA2C_MAX_RUN_NETS, "%s: runs * N = %lld above IA2C_MAX_RUN_NETS = %d", who,
+                 (long long)r->runs * d->N, IA2C_MAX_RUN_NETS);
+    IA2C_REQUIRE(r->seed != nullptr, "%s: null seed array (one Philox key per run)", who);
+    auto unsupported = [](const char* what, const char* who) {
+        set_error("%s: %s", who, what);
+        return IA2C_ERR_UNSUPPORTED;
+    };
+    if (!rollout_fused_supported(d->N, d->M)) {
+        set_error("%s: N=%d M=%d has no fused instantiation (batches need N <= 8 with M = 5, or N = 2 with M = 3)", who, d->N, d->M);
+        return IA2C_ERR_UNSUPPORTED;
+    }
+    if (d->env_offset != 0 || d->E_total != d->E)
+        return unsupported("batches run on one GPU: desc.env_offset must be 0 and desc.E_total == desc.E (envs per run)", who);
+    if (d->inj_actions || d->inj_u_action || d->inj_u_belief) return unsupported("injected replay tapes are not supported in batches", who);
+    if (d->state_trace || d->reward_f64 || d->pred_dump || d->belief_dump || d->adv_dump || d->target_dump)
+        return unsupported("parity dumps are not supported in batches", who);
+    if (d->flags & ~(IA2C_FLAG_FUSED_ROLLOUT | IA2C_FLAG_FUSED_CRITIC | IA2C_FLAG_ACTOR_COLUMNS))
+        return unsupported("desc.flags may carry only FUSED_ROLLOUT, FUSED_CRITIC and ACTOR_COLUMNS", who);
+    IA2C_REQUIRE(d->env_state && d->env_hist && d->env_cls && d->env_elapsed && d->ep_return && d->belief_records && d->filter_action,
+                 "%s: null env/belief pointer", who);
+    IA2C_REQUIRE(d->critic_grad && d->actor_grad && d->critic_m && d->critic_v && d->actor_m && d->actor_v && d->actor_grad_accum &&
+                     d->critic_step && d->actor_step && d->loss_out, "%s: null optimiser pointer", who);
+    IA2C_REQUIRE(d->partials && d->partials_floats >= ia2c_runs_partials_floats(d, r->runs), "%s: partials workspace too small (%zu < %zu)",
+                 who, d->partials_floats, ia2c_runs_partials_floats(d, r->runs));
+    return 0;
+}
+
+extern "C" int ia2c_train_episode_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream) {
+    if (int rc = validate_runs(d, r)) return rc;
+    cudaStream_t s = as_stream(stream);
+    const int R = r->runs, nets = R * d->N;
+    ia2c_episode_desc e = *d;
+    e.flags = IA2C_FLAG_FUSED_ROLLOUT | IA2C_FLAG_FUSED_CRITIC | IA2C_FLAG_ACTOR_COLUMNS;
+    auto reduce = [&](int which) {   // which = 0 critics, 1 actors: the R * N nets, each with its run's learning rate
+        ReduceArgs A = make_reduce_args(e, which, which == 0 ? critic_partial_blocks(&e) : actor_partial_blocks(&e));
+        A.loss_out = e.loss_out + (which == 0 ? 0 : nets);
+        const ReduceRuns rr = {which == 0 ? r->lr_critic : r->lr_actor, d->N};
+        dim3 grid(nets, ceil_div(A.P + 1, 32));
+        return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr);
+    };
+    if (int rc = rollout_fused_launch(&e, r, s)) return rc;
+    if (int rc = reduce(0)) return rc;
+    dim3 grid(grad_blocks(&e), nets);
+    if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
+    return reduce(1);
 }
 
 #ifdef IA2C_STAGE_CLOCKS

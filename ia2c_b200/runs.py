@@ -1,0 +1,200 @@
+"""IA2CRuns — many independent IA2C training runs (seeds, hyper-parameter sweeps) advanced together on one GPU.
+
+One episode of every run is ONE C call (``ia2c_train_episode_runs``) whose four launches each cover all R runs: the
+standalone episode is latency-bound and leaves most of the B200 idle, so R runs cost far less than R standalone
+episodes.  Run r computes byte for byte what ``IA2CTrainer(envs_per_run, seed=seeds[r], init=reference_init(N, M,
+seed=seeds[r]), <run r's hyper-parameters>)`` computes over the same episodes (include/ia2c_b200.h states the contract).
+
+The device buffers hold the runs stacked (DESIGN.md §3): per-net buffers have R*N rows, run r at rows [r*N, (r+1)*N);
+per-env buffers have an env axis of length R*E, run r at [r*E, (r+1)*E).  ``run_view(r)`` returns those slices and
+``run_state_dict(r)`` a checkpoint that a standalone ``IA2CTrainer`` loads, so the best run of a sweep can go on alone.
+"""
+from __future__ import annotations
+
+import ctypes as C
+import math
+
+import numpy as np
+import torch
+
+from . import _lib
+from .trainer import N_ACTIONS, N_FEATURES, IA2CTrainer, reference_init
+
+# buffers with one row per (run, agent), and buffers with an env axis (its position) of length R * E
+_NET = ("actor_params", "critic_params", "actor_grad", "critic_grad", "actor_grad_accum", "actor_m", "actor_v", "critic_m",
+        "critic_v", "actor_step", "critic_step", "filter_action")
+_ENV = {"env_state": 0, "env_hist": 0, "env_cls": 0, "env_elapsed": 0, "ep_return": 0, "belief_records": 0,
+        "obs": 1, "reward": 1, "act": 1, "partner_true": 1, "partner_pred": 1}
+
+
+def _per_run(name, value, R, dtype):
+    """A hyper-parameter given as a scalar (-> (None, value): the descriptor's scalar serves every run) or as a length-R
+    sequence (-> (array, value[0]))."""
+    if np.ndim(value) == 0:
+        v = float(value)
+        if not math.isfinite(v):
+            raise ValueError(f"{name} must be finite, got {value!r}")
+        return None, v
+    arr = np.asarray(value, dtype=np.float64)
+    if arr.ndim != 1 or arr.shape[0] != R:
+        raise ValueError(f"{name} must be a scalar or a sequence of one value per run ({R}), got shape {arr.shape}")
+    if not np.all(np.isfinite(arr)):
+        raise ValueError(f"{name} must be finite")
+    return arr.astype(dtype), float(arr[0])
+
+
+class IA2CRuns:
+    def __init__(self, envs_per_run, seeds, n_agents=2, n_models=5, steps_per_episode=30, max_episode_steps=30,
+                 lr_critic=0.0002, lr_actor=0.0001, beta=0.001, gamma=0.9, init=None, device=None):
+        self.lib = _lib.load()
+        seeds = [int(s) for s in seeds]
+        R, E, N, M, T = len(seeds), int(envs_per_run), int(n_agents), int(n_models), int(steps_per_episode)
+        if R < 1:
+            raise ValueError("seeds: need at least one run")
+        if any(s < 0 or s >= 1 << 64 for s in seeds):
+            raise ValueError("seeds must lie in [0, 2**64)")
+        if E < 1 or not 0 < T < 65535:
+            raise ValueError(f"envs_per_run={E} must be >= 1 and steps_per_episode={T} in 1..65534")
+        if not self.lib.ia2c_rollout_fused_supported(N, M):
+            raise ValueError(f"n_agents={N}, n_models={M}: batches of runs need the fused path (N <= 8 with M = 5, or N = 2 with M = 3)")
+        if R * N > _lib.MAX_RUN_NETS:
+            raise ValueError(f"runs * n_agents = {R * N} above the limit of {_lib.MAX_RUN_NETS}")
+        hyper = {name: _per_run(name, v, R, dt) for name, v, dt in
+                 (("lr_actor", lr_actor, np.float64), ("lr_critic", lr_critic, np.float64),
+                  ("gamma", gamma, np.float32), ("beta", beta, np.float32))}
+        if init is not None and len(init) != R:
+            raise ValueError(f"init: need one (actor, critic, filter_action) tuple per run ({R}), got {len(init)}")
+        _lib.require_cuda()
+        self.R, self.E, self.N, self.M, self.T, self.K = R, E, N, M, T, N - 1
+        self.seeds = seeds
+        self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+        self.episode = 0
+        dev, RN, RE, K = self.device, R * N, R * E, N - 1
+
+        def z(shape, dtype):
+            return torch.zeros(shape, dtype=dtype, device=dev)
+
+        f32, f64, u8, i32 = torch.float32, torch.float64, torch.uint8, torch.int32
+        self.actor_params, self.critic_params = z((RN, _lib.ACTOR_P), f32), z((RN, _lib.CRITIC_P), f32)
+        self.actor_grad, self.critic_grad = z((RN, _lib.ACTOR_P + 1), f32), z((RN, _lib.CRITIC_P + 1), f32)
+        self.actor_grad_accum = z((RN, _lib.ACTOR_P), f32)
+        self.actor_m, self.actor_v = z((RN, _lib.ACTOR_P), f32), z((RN, _lib.ACTOR_P), f32)
+        self.critic_m, self.critic_v = z((RN, _lib.CRITIC_P), f32), z((RN, _lib.CRITIC_P), f32)
+        self.actor_step, self.critic_step = z((RN,), i32), z((RN,), i32)
+        self.loss_out = z((2, RN), f32)
+        self.filter_action = z((RN, M, N_ACTIONS), f64)
+        self.env_state, self.env_hist = z((RE,), i32), z((RE,), f64)
+        self.env_cls, self.env_elapsed = z((RE, 2), u8), z((RE,), i32)
+        self.ep_return = z((RE,), f64)
+        self.obs, self.reward = z((T + 1, RE, N_FEATURES), f32), z((T, RE), f32)
+        self.act, self.partner_true, self.partner_pred = z((T + 1, RE, N), u8), z((T + 1, RE, N), u8), z((T + 1, RE, N), u8)
+        self.belief_records = z((RE, N, K, _lib.BELIEF_RECORD), u8)
+        self._seed = torch.from_numpy(np.asarray(seeds, dtype=np.uint64).view(np.int64)).to(dev)
+        self._hyper = {k: (torch.from_numpy(a).to(dev) if a is not None else None) for k, (a, _) in hyper.items()}
+
+        d = self.desc = _lib.EpisodeDesc()
+        d.E, d.E_total, d.env_offset = E, E, 0
+        d.N, d.T, d.M, d.max_episode_steps = N, T, M, int(max_episode_steps or 0)
+        d.lr_actor, d.lr_critic = hyper["lr_actor"][1], hyper["lr_critic"][1]
+        d.gamma, d.beta = hyper["gamma"][1], hyper["beta"][1]
+        d.flags = _lib.FLAG_FUSED_ROLLOUT | _lib.FLAG_FUSED_CRITIC | _lib.FLAG_ACTOR_COLUMNS
+        for name in _NET + tuple(_ENV) + ("loss_out",):
+            setattr(d, name, getattr(self, name).data_ptr())
+        n_part = int(self.lib.ia2c_runs_partials_floats(C.byref(d), R))
+        self.partials = z((n_part,), f32)
+        d.partials, d.partials_floats = self.partials.data_ptr(), n_part
+        r = self.runs_desc = _lib.RunsDesc()
+        r.runs, r.seed = R, self._seed.data_ptr()
+        for k, t in self._hyper.items():
+            setattr(r, k, t.data_ptr() if t is not None else None)
+
+        self.critic_losses, self.actor_losses, self.reward_lst = [], [], []
+        for k in range(R):
+            self._load_init(k, *(init[k] if init is not None else reference_init(N, M, seed=seeds[k])))
+
+    def _load_init(self, r, actor, critic, filter_action):
+        rows = slice(r * self.N, (r + 1) * self.N)
+        self.actor_params[rows].copy_(torch.as_tensor(np.asarray(actor), dtype=torch.float32))
+        self.critic_params[rows].copy_(torch.as_tensor(np.asarray(critic), dtype=torch.float32))
+        self.filter_action[rows].copy_(torch.as_tensor(np.asarray(filter_action), dtype=torch.float64))
+
+    # ------------------------------------------------------------------ episodes
+    def train_episode(self, sync_stats=False):
+        """One episode of every run in one C call; asynchronous unless ``sync_stats``."""
+        self.desc.episode = self.episode
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ia2c_train_episode_runs(C.byref(self.desc), C.byref(self.runs_desc),
+                                                        torch.cuda.current_stream(self.device).cuda_stream),
+                       "ia2c_train_episode_runs")
+        self.episode += 1
+        if sync_stats:
+            return self.read_stats()
+
+    def read_stats(self):
+        """The last episode's losses ``[R, N]`` and returns ``[R, E]``, appended to each run's windows as
+        ``IA2CTrainer._record_stats`` does (20-deep loss windows, last-50 returns); the window means are per run."""
+        R, N, E = self.R, self.N, self.E
+        loss = self.loss_out.cpu().numpy()
+        ret = self.ep_return.cpu().numpy().reshape(R, E)
+        critic, actor = loss[0].reshape(R, N), loss[1].reshape(R, N)
+        self.critic_losses.append(critic), self.actor_losses.append(actor)
+        del self.critic_losses[:-20], self.actor_losses[:-20]
+        self.reward_lst.append(ret)
+        del self.reward_lst[:-50]
+        return dict(critic_loss=critic, actor_loss=actor, ep_return=ret,
+                    critic_loss_window=np.mean(self.critic_losses, axis=0), actor_loss_window=np.mean(self.actor_losses, axis=0),
+                    mean_return=np.array([np.mean([x[r] for x in self.reward_lst]) for r in range(R)]))
+
+    # ------------------------------------------------------------------ one run's slice
+    def run_view(self, r):
+        """Views (no copies) of run r's slices of every device buffer, under the names ``IA2CTrainer`` uses."""
+        if not 0 <= r < self.R:
+            raise IndexError(f"run {r} of {self.R}")
+        N, E = self.N, self.E
+        v = {k: getattr(self, k)[r * N:(r + 1) * N] for k in _NET}
+        for k, axis in _ENV.items():
+            v[k] = getattr(self, k).narrow(axis, r * E, E)
+        v["loss_out"] = self.loss_out[:, r * N:(r + 1) * N]
+        return v
+
+    def run_state_dict(self, r):
+        """Run r as a checkpoint of a standalone ``IA2CTrainer(envs_per_run, ..., seed=seeds[r])``: its
+        ``load_state_dict`` accepts it and the run continues alone bit-identically."""
+        torch.cuda.current_stream(self.device).synchronize()
+        v = self.run_view(r)
+        sd = {k: v[k].detach().cpu().clone() for k in IA2CTrainer._CKPT_TENSORS}
+        sd.update(episode=self.episode, seed=self.seeds[r], dims=(self.E, self.E, self.N, self.M, self.T), rank=0, world=1,
+                  critic_losses=[x[r].copy() for x in self.critic_losses], actor_losses=[x[r].copy() for x in self.actor_losses],
+                  reward_lst=[x[r].copy() for x in self.reward_lst])
+        return sd
+
+    # ------------------------------------------------------------------ checkpoint / resume of the whole batch
+    def state_dict(self):
+        torch.cuda.current_stream(self.device).synchronize()
+        sd = {k: getattr(self, k).detach().cpu().clone() for k in IA2CTrainer._CKPT_TENSORS}
+        sd.update(episode=self.episode, seeds=list(self.seeds), dims=(self.R, self.E, self.N, self.M, self.T),
+                  critic_losses=[x.copy() for x in self.critic_losses], actor_losses=[x.copy() for x in self.actor_losses],
+                  reward_lst=[x.copy() for x in self.reward_lst])
+        return sd
+
+    def load_state_dict(self, sd):
+        """Restores parameters, optimiser, env and belief state, the episode counter, the runs' seeds and the windows; the
+        hyper-parameters stay those this batch was built with (as ``IA2CTrainer.load_state_dict``)."""
+        if tuple(sd["dims"]) != (self.R, self.E, self.N, self.M, self.T):
+            raise ValueError(f"checkpoint is for (runs, E, N, M, T) = {tuple(sd['dims'])}, batch has {(self.R, self.E, self.N, self.M, self.T)}")
+        for k in IA2CTrainer._CKPT_TENSORS:
+            getattr(self, k).copy_(sd[k])
+        self.episode = int(sd["episode"])
+        self.seeds = [int(s) for s in sd["seeds"]]
+        self._seed.copy_(torch.from_numpy(np.asarray(self.seeds, dtype=np.uint64).view(np.int64)))
+        self.critic_losses, self.actor_losses = list(sd["critic_losses"]), list(sd["actor_losses"])
+        self.reward_lst = list(sd["reward_lst"])
+
+    def save(self, path):
+        torch.save(self.state_dict(), path)
+
+    def load(self, path):
+        self.load_state_dict(torch.load(path, map_location="cpu", weights_only=False))
+
+    def agent_steps_per_episode(self):
+        return self.R * self.E * self.N * self.T

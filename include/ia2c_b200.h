@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define IA2C_ABI_VERSION 2
+#define IA2C_ABI_VERSION 3
 #define IA2C_HIDDEN 6          /* ac_nets.py:24 */
 #define IA2C_OBS_FEATURES 6    /* Org observation: [onehot3(prev class), onehot3(class)]  Org.py:37,112-114 */
 #define IA2C_AGENT_ACTIONS 3   /* ia2c.py:44 */
@@ -360,6 +360,46 @@ int ia2c_train_episodes_host(const ia2c_episode_desc* d, ia2c_host_pipe* pipe, v
 int ia2c_train_episodes_host_p2p(const ia2c_episode_desc* d, ia2c_host_pipe* pipe, const ia2c_peer_desc* peers,
                                  uint32_t epoch0, void* stage_b, void* result_b, int32_t n_episodes,
                                  const void* const* host_tapes, void* host_results, void* stream);
+
+/* ------------------------------------------------------------------ batches of independent runs -- */
+/* R independent IA2C training runs (seeds, hyper-parameter sweeps) advanced together, one episode number for all, in the
+ * launches of ONE episode.  All runs share N, M, T, max_episode_steps and E = envs per run; run r has its own Philox key
+ * seed[r], its own parameters, belief models and Adam state, and its own lr_actor / lr_critic / gamma / beta.
+ *
+ * Contract: run r computes byte for byte what ia2c_train_episode computes for a standalone run of E envs with
+ * desc.seed = seed[r], flags FUSED_ROLLOUT | FUSED_CRITIC | ACTOR_COLUMNS and the run's hyper-parameters — trajectory,
+ * beliefs, returns, losses, gradients, Adam moments, step counters, actor grad_accum and parameters.  Philox counters use
+ * the env's index WITHIN its run, the means divide by T * E, and every run's gradient partial rows are partitioned as a
+ * standalone run of E envs partitions them, so every fixed-order sum is the same sum.
+ *
+ * `d` describes ONE run's shape (E = E_total = envs per run, env_offset = 0; desc.seed is not used); its pointers hold all
+ * R runs stacked:
+ *   per-net buffers  (params, grads, Adam m / v, step counters, actor_grad_accum, filter_action): R*N rows, run r at rows
+ *                    [r*N, (r+1)*N);
+ *   per-env buffers  (env state, ep_return, belief_records, and the trajectory obs[T+1, R*E, 6], reward[T, R*E],
+ *                    act / partner_true / partner_pred [T+1, R*E, N]): the env axis has length R*E, run r at [r*E, (r+1)*E);
+ *   loss_out         float[2, R*N] (critic losses of all nets, then actor losses);
+ *   partials         ia2c_runs_partials_floats(d, R) floats.
+ * Supported: the fused path only (ia2c_rollout_fused_supported(N, M): N <= 8), one GPU, Philox sampling.  desc.flags may
+ * carry only FUSED_ROLLOUT, FUSED_CRITIC and ACTOR_COLUMNS (the path is always that one).  Refused with
+ * IA2C_ERR_UNSUPPORTED: other (N, M), a non-zero env_offset or E_total != E (multi-GPU), injected replay tapes, parity
+ * dumps, other flags.  Refused with IA2C_ERR_INVALID: runs < 1, runs * N > IA2C_MAX_RUN_NETS (the actor-gradient grid
+ * has one block row per net), a NULL seed array, missing buffers.  Every check runs before the first CUDA call.
+ * The host-tape pipelines have no batched form. */
+#define IA2C_MAX_RUN_NETS 65535
+typedef struct ia2c_runs_desc {
+    int32_t runs;              /* R >= 1, R * N <= IA2C_MAX_RUN_NETS */
+    int32_t reserved;
+    const uint64_t* seed;      /* device uint64[R]: Philox key of run r (desc.seed is not used) */
+    const double* lr_actor;    /* device double[R], or NULL -> desc.lr_actor for every run */
+    const double* lr_critic;   /* device double[R], or NULL -> desc.lr_critic */
+    const float* gamma;        /* device float[R],  or NULL -> desc.gamma */
+    const float* beta;         /* device float[R],  or NULL -> desc.beta */
+} ia2c_runs_desc;
+size_t ia2c_runs_partials_floats(const ia2c_episode_desc* d, int32_t runs);
+/* One episode of every run: fused rollout + critic gradient, critic reduce + Adam, actor gradient, actor reduce + Adam —
+ * the four launches of a standalone episode, each covering all R runs. */
+int ia2c_train_episode_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream);
 
 #ifdef __cplusplus
 }
