@@ -28,4 +28,7 @@ def __getattr__(name):  # lazy: torch-dependent classes are imported on first us
     if name == "IA2CRuns":
         from .runs import IA2CRuns
         return IA2CRuns
+    if name in ("A2COrgTrainer", "a2c_reference_init"):
+        from . import a2c
+        return getattr(a2c, name)
     raise AttributeError(name)

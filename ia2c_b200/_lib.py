@@ -22,10 +22,13 @@ FLAG_ACTOR_COLUMNS = 16
 FLAG_BELIEF_PER_STEP = 32
 FLAG_ROLLOUT_PER_STEP = 64
 BELIEF_RECORD = 8
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAX_RUN_NETS = 65535   # IA2C_MAX_RUN_NETS: runs * n_agents of one batch
 ACTOR_P = 105
 CRITIC_P = 147
+A2C_MAX_RUNS = 65535          # IA2C_A2C_MAX_RUNS
+A2C_MAX_ENVS = 1 << 30        # IA2C_A2C_MAX_ENVS: envs per run and runs * envs
+A2C_MAX_STEPS = 65534         # IA2C_A2C_MAX_STEPS
 
 
 class EpisodeDesc(C.Structure):
@@ -61,6 +64,20 @@ class PeerDesc(C.Structure):
 class RunsDesc(C.Structure):
     """Mirror of ``ia2c_runs_desc``: a batch of independent runs (ia2c_train_episode_runs)."""
     _fields_ = [("runs", i32), ("reserved", i32), ("seed", vp), ("lr_actor", vp), ("lr_critic", vp), ("gamma", vp), ("beta", vp)]
+
+
+class A2CDesc(C.Structure):
+    """Mirror of ``ia2c_a2c_desc``: one update of the native A2C trainer (ia2c_a2c_train_update)."""
+    _fields_ = [
+        ("E", i64), ("R", i32), ("T", i32), ("update", u32), ("beta", f32), ("lr_actor", f64), ("lr_critic", f64),
+        ("seed", vp), ("lr_actor_run", vp), ("lr_critic_run", vp), ("beta_run", vp),
+        ("actor_params", vp), ("actor_grad", vp), ("actor_grad_accum", vp), ("actor_m", vp), ("actor_v", vp),
+        ("critic_params", vp), ("critic_grad", vp), ("critic_m", vp), ("critic_v", vp),
+        ("actor_step", vp), ("critic_step", vp),
+        ("env_state", vp), ("env_hist", vp), ("env_cls", vp), ("env_elapsed", vp), ("pending_action", vp), ("ep_return", vp),
+        ("obs", vp), ("act", vp), ("reward", vp), ("loss_out", vp), ("inj_actions", vp),
+        ("partials", vp), ("partials_floats", C.c_size_t),
+    ]
 
 
 _DP = C.POINTER(EpisodeDesc)
@@ -114,6 +131,8 @@ SIGNATURES = {
     "ia2c_train_episodes_host_p2p": (C.c_int, [_DP, vp, C.POINTER(PeerDesc), u32, vp, vp, i32, C.POINTER(vp), vp, vp]),
     "ia2c_runs_partials_floats": (C.c_size_t, [_DP, i32]),
     "ia2c_train_episode_runs": (C.c_int, [_DP, C.POINTER(RunsDesc), vp]),
+    "ia2c_a2c_partials_floats": (C.c_size_t, [C.POINTER(A2CDesc)]),
+    "ia2c_a2c_train_update": (C.c_int, [C.POINTER(A2CDesc), vp]),
 }
 
 _lib = None

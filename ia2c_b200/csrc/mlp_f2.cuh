@@ -341,6 +341,13 @@ __device__ __forceinline__ void load_obs6(const float* __restrict__ p, float (&x
     x[0] = a.x; x[1] = a.y; x[2] = b.x; x[3] = b.y; x[4] = c.x; x[5] = c.y;
 }
 
+// float2 gradient accumulators -> the flat gradient vector (+ loss slot) that block_reduce_store takes
+template <int GN>
+__device__ __forceinline__ void unpack_g2(const float2 (&g2)[GN], float (&g)[2 * GN]) {
+#pragma unroll
+    for (int i = 0; i < GN; ++i) { g[2 * i] = g2[i].x; g[2 * i + 1] = g2[i].y; }
+}
+
 template <int O>
 __device__ __forceinline__ float select_out(const float (&q)[O], int idx) {
     float v = 0.f;

@@ -36,6 +36,7 @@ int rollout_fused_supported(int N, int M);                                  // r
 int rollout_fused_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s);
 int64_t rollout_fused_blocks(int64_t E, int N);
 int actor_pipe_launch(const ia2c_episode_desc* d, cudaStream_t s);
+int reduce_adam_runs_launch(const ReduceArgs& A, const double* lr_per_net, int nets, cudaStream_t s);   // used by a2c.cu
 int64_t actor_pipe_blocks(int64_t E, int N);
 
 namespace {
@@ -312,12 +313,6 @@ __host__ __device__ inline ChunkPlan chunk_plan(int T, int64_t E, int N) {
     p.chunk_len = (int)((T + c - 1) / c);
     p.n_chunks = (T + p.chunk_len - 1) / p.chunk_len;
     return p;
-}
-
-template <int GN>
-__device__ __forceinline__ void unpack_g2(const float2 (&g2)[GN], float (&g)[2 * GN]) {
-#pragma unroll
-    for (int i = 0; i < GN; ++i) { g[2 * i] = g2[i].x; g[2 * i + 1] = g2[i].y; }
 }
 
 // partial row layout: P gradient entries then the loss partial.
@@ -1274,6 +1269,14 @@ extern "C" int ia2c_train_episode_runs(const ia2c_episode_desc* d, const ia2c_ru
     dim3 grid(grad_blocks(&e), nets);
     if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
     return reduce(1);
+}
+
+// reduce_adam_kernel<true> for `nets` nets of P entries with one learning rate per net (lr_per_net, or A.lr where NULL): the
+// native A2C trainer (a2c.cu) reduces and steps its R actor and R critic rows with it.
+int ia2c::reduce_adam_runs_launch(const ReduceArgs& A, const double* lr_per_net, int nets, cudaStream_t s) {
+    const ReduceRuns rr = {lr_per_net, 1};
+    const dim3 grid(nets, ceil_div(A.P + 1, 32));
+    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr);
 }
 
 #ifdef IA2C_STAGE_CLOCKS

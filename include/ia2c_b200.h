@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define IA2C_ABI_VERSION 3
+#define IA2C_ABI_VERSION 4
 #define IA2C_HIDDEN 6          /* ac_nets.py:24 */
 #define IA2C_OBS_FEATURES 6    /* Org observation: [onehot3(prev class), onehot3(class)]  Org.py:37,112-114 */
 #define IA2C_AGENT_ACTIONS 3   /* ia2c.py:44 */
@@ -400,6 +400,57 @@ size_t ia2c_runs_partials_floats(const ia2c_episode_desc* d, int32_t runs);
 /* One episode of every run: fused rollout + critic gradient, critic reduce + Adam, actor gradient, actor reduce + Adam —
  * the four launches of a standalone episode, each covering all R runs. */
 int ia2c_train_episode_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream);
+
+/* ------------------------------------------------------------------ native A2C trainer (a2c_org_test.py) -- */
+/* One update of a2c_org_test.py:43-92 for R independent runs x E envs: a single joint agent with 9 actions, actor and
+ * critic both 6 -> 6 -> 6 -> 9 MLPs (147 parameters each, the actor ending in a softmax), Org envs that are never reset
+ * after ia2c_org_reset and have no TimeLimit (SURVEY.md Q6).  Per env and update: T steps of Org.step(pending action)
+ * followed by a sample of the next action from the post-step observation; the stored pair is (post-step obs, action
+ * taken) (Q4).  Critic: target = reward (masks = 0, Q5), L = mean((r - Q(S)[a])^2), Adam.  Actor: Q from the UPDATED
+ * critic, V = sum(Q * pi), adv = Q[a] - V with gradient through pi (Q7), policy gradient + beta * entropy, Adam on the
+ * never-zeroed running sum of the gradients (Q2).  One row per env (the reference's two buffer rows are copies of one
+ * env); the means divide by T * E.  gamma is absent on purpose: with masks = 0 it multiplies zero.
+ *
+ * Sampling: inj_actions == NULL -> Philox stream 3, key = seed[r], counter = (env index within its run,
+ * slot | 3 << 16, update), the 24-bit uniform of the inverse-CDF sampler; slot 0 is update 0's first draw from the reset
+ * observation, slot t + 1 the draw after step t.  inj_actions uint8[T+1, R*E] replays actions (codes 0..8) in the same
+ * slot order; slot 0 is read at update 0 only.
+ *
+ * Layout (stacked like ia2c_runs_desc): per-net buffers have R rows (params / Adam m, v / grad_accum float[R,147],
+ * grads float[R,148] with this update's loss in the trailing slot, step counters int32[R]); per-env buffers have an
+ * env axis of length R*E, run r at [r*E, (r+1)*E): env_state int32, env_hist double, env_cls uint8[.,2], env_elapsed
+ * int32 (steps since reset), pending_action uint8, ep_return double (fp64 sum of the update's T rewards); trajectory
+ * obs float[T, R*E, 6], act uint8[T, R*E], reward float[T, R*E]; loss_out float[2, R] (critic losses, then actor).
+ *
+ * Contract: run r computes byte for byte what a call with R = 1, seed[0] = seed[r] and run r's hyper-parameters computes
+ * on run r's slices.  One update is FOUR launches: rollout + critic gradient, critic reduce + Adam, actor gradient, actor
+ * reduce + Adam.  Every check (ranges, NULL seed or buffers, workspace size) runs before the first CUDA call. */
+#define IA2C_A2C_MAX_RUNS 65535           /* R: one grid row per run */
+#define IA2C_A2C_MAX_ENVS 1073741824      /* E and R * E */
+#define IA2C_A2C_MAX_STEPS 65534          /* T: the slot field of the Philox counter is 16 bits */
+typedef struct ia2c_a2c_desc {
+    int64_t E;                 /* envs per run */
+    int32_t R, T;              /* runs, steps per update */
+    uint32_t update;           /* update number (Philox counter; update 0 draws the first action) */
+    float beta;                /* entropy weight when beta_run is NULL */
+    double lr_actor, lr_critic;            /* learning rates when the per-run arrays are NULL */
+    const uint64_t* seed;                  /* uint64[R]: Philox key of run r */
+    const double* lr_actor_run;            /* double[R] or NULL */
+    const double* lr_critic_run;           /* double[R] or NULL */
+    const float* beta_run;                 /* float[R] or NULL */
+    float *actor_params, *actor_grad, *actor_grad_accum, *actor_m, *actor_v;
+    float *critic_params, *critic_grad, *critic_m, *critic_v;
+    int32_t *actor_step, *critic_step;
+    int32_t* env_state; double* env_hist; uint8_t* env_cls; int32_t* env_elapsed;
+    uint8_t* pending_action;
+    double* ep_return;
+    float* obs; uint8_t* act; float* reward;
+    float* loss_out;
+    const uint8_t* inj_actions;            /* uint8[T+1, R*E] or NULL */
+    float* partials; size_t partials_floats;  /* ia2c_a2c_partials_floats(desc) */
+} ia2c_a2c_desc;
+size_t ia2c_a2c_partials_floats(const ia2c_a2c_desc* d);
+int ia2c_a2c_train_update(const ia2c_a2c_desc* d, void* stream);
 
 #ifdef __cplusplus
 }
