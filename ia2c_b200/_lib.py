@@ -22,13 +22,16 @@ FLAG_ACTOR_COLUMNS = 16
 FLAG_BELIEF_PER_STEP = 32
 FLAG_ROLLOUT_PER_STEP = 64
 BELIEF_RECORD = 8
-ABI_VERSION = 4
+ABI_VERSION = 5
 MAX_RUN_NETS = 65535   # IA2C_MAX_RUN_NETS: runs * n_agents of one batch
 ACTOR_P = 105
 CRITIC_P = 147
 A2C_MAX_RUNS = 65535          # IA2C_A2C_MAX_RUNS
 A2C_MAX_ENVS = 1 << 30        # IA2C_A2C_MAX_ENVS: envs per run and runs * envs
 A2C_MAX_STEPS = 65534         # IA2C_A2C_MAX_STEPS
+EVAL_MAX_RUNS = 65535         # IA2C_EVAL_MAX_RUNS
+EVAL_MAX_AGENTS = 1023        # IA2C_EVAL_MAX_AGENTS
+EVAL_MAX_STEPS = 65535        # IA2C_EVAL_MAX_STEPS
 
 
 class EpisodeDesc(C.Structure):
@@ -77,6 +80,16 @@ class A2CDesc(C.Structure):
         ("env_state", vp), ("env_hist", vp), ("env_cls", vp), ("env_elapsed", vp), ("pending_action", vp), ("ep_return", vp),
         ("obs", vp), ("act", vp), ("reward", vp), ("loss_out", vp), ("inj_actions", vp),
         ("partials", vp), ("partials_floats", C.c_size_t),
+    ]
+
+
+class EvalDesc(C.Structure):
+    """Mirror of ``ia2c_eval_desc``: a frozen-policy evaluation of R runs' actors (ia2c_evaluate)."""
+    _fields_ = [
+        ("actor_params", vp), ("R", i32), ("N", i32), ("E", i64),
+        ("episodes", i32), ("T", i32), ("max_episode_steps", i32), ("greedy", i32),
+        ("seed", u64), ("episode0", u32), ("inj_u_action", vp),
+        ("policy", vp), ("policy_floats", C.c_size_t), ("returns", vp), ("action_counts", vp),
     ]
 
 
@@ -133,6 +146,8 @@ SIGNATURES = {
     "ia2c_train_episode_runs": (C.c_int, [_DP, C.POINTER(RunsDesc), vp]),
     "ia2c_a2c_partials_floats": (C.c_size_t, [C.POINTER(A2CDesc)]),
     "ia2c_a2c_train_update": (C.c_int, [C.POINTER(A2CDesc), vp]),
+    "ia2c_eval_policy_floats": (C.c_size_t, [C.POINTER(EvalDesc)]),
+    "ia2c_evaluate": (C.c_int, [C.POINTER(EvalDesc), vp]),
 }
 
 _lib = None

@@ -196,5 +196,16 @@ class IA2CRuns:
     def load(self, path):
         self.load_state_dict(torch.load(path, map_location="cpu", weights_only=False))
 
+    # ------------------------------------------------------------------ frozen-policy evaluation
+    def evaluate(self, episodes=1, num_envs=None, greedy=False, seed=0, first_episode=0):
+        """``IA2CTrainer.evaluate`` for every run at once (default ``num_envs``: envs_per_run; greedy: 1), with a leading
+        run axis on every result (returns [R, K, E], mean_return [R], ...).  All runs see the same random numbers, so their
+        returns are paired samples, and run r's results equal those of a standalone trainer holding ``run_state_dict(r)``."""
+        from .evaluate import evaluate_actors
+
+        E = (1 if greedy else self.E) if num_envs is None else num_envs
+        return evaluate_actors(self.actor_params, self.R, self.N, E, episodes, self.T, self.desc.max_episode_steps, greedy,
+                               seed, first_episode, self.device)
+
     def agent_steps_per_episode(self):
         return self.R * self.E * self.N * self.T

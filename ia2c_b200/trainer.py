@@ -510,6 +510,21 @@ class IA2CTrainer:
     def load(self, path):
         self.load_state_dict(torch.load(path, map_location="cpu", weights_only=False))
 
+    # ------------------------------------------------------------------ frozen-policy evaluation
+    def evaluate(self, episodes=1, num_envs=None, greedy=False, seed=0, first_episode=0):
+        """Evaluate the current actors without training: ``episodes`` episodes of T steps in each of ``num_envs`` envs
+        (default E_total; greedy: 1) from the reset state, with this trainer's max_episode_steps.  Actions are sampled from
+        the actors with Philox stream 4 keyed by ``seed`` (episodes ``first_episode`` onwards) or, with ``greedy``, are their
+        argmax.  Reads ``actor_params`` on the trainer's stream and writes no trainer buffer; at world > 1 it runs on the
+        calling rank alone, with its replicated parameters.  Returns returns [K, E], mean_return, std_return,
+        action_counts / action_freq [N, 3] (freq = counts / (K * E * T)), policy [N, 9, 3] and, greedy, greedy_actions [N, 9]."""
+        from .evaluate import evaluate_actors
+
+        E = (1 if greedy else self.E_total) if num_envs is None else num_envs
+        out = evaluate_actors(self.actor_params, 1, self.N, E, episodes, self.T, self.desc.max_episode_steps, greedy, seed,
+                              first_episode, self.device)
+        return {k: v[0] for k, v in out.items()}
+
     # ------------------------------------------------------------------ accounting
     def agent_steps_per_episode(self):
         return self.E_total * self.N * self.T

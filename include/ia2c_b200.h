@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define IA2C_ABI_VERSION 4
+#define IA2C_ABI_VERSION 5
 #define IA2C_HIDDEN 6          /* ac_nets.py:24 */
 #define IA2C_OBS_FEATURES 6    /* Org observation: [onehot3(prev class), onehot3(class)]  Org.py:37,112-114 */
 #define IA2C_AGENT_ACTIONS 3   /* ia2c.py:44 */
@@ -451,6 +451,51 @@ typedef struct ia2c_a2c_desc {
 } ia2c_a2c_desc;
 size_t ia2c_a2c_partials_floats(const ia2c_a2c_desc* d);
 int ia2c_a2c_train_update(const ia2c_a2c_desc* d, void* stream);
+
+/* ------------------------------------------------------------------ frozen-policy evaluation of IA2C actors -- */
+/* Plays `episodes` episodes of T Org-N steps in each of E envs of each of R runs with the runs' actors frozen: no belief
+ * filter, no critic, no update (the IA2C actor reads only the observation).  Every item (episode k, env e) starts from
+ * the reset state, steps with the same-step autoreset at max_episode_steps (0: no limit) and sums its fp64 rewards in step
+ * order.  Actions are sampled by the inverse CDF at a uniform or, with greedy != 0, are the argmax of the distribution
+ * (ties to the lowest action, as torch.argmax).
+ *
+ * Layout: actor_params f32[R*N, 105], run r at rows [r*N, (r+1)*N) (as ia2c_runs_desc stacks them);
+ *   policy        out f32[R*N, 9, 3]: each actor's softmax at observation class c = 3 * prev_cls + cur_cls (the one-hot
+ *                 [onehot3(prev_cls), onehot3(cur_cls)]), bit-identical to the probabilities the training samplers draw from;
+ *   returns       out f64[R, episodes, E] (greedy: f64[R]);
+ *   action_counts out u64[R*N, 3], overwritten: how often each agent took each action over all items and steps;
+ *   inj_u_action  f32[episodes, T, R*E, N] or NULL: the uniforms, instead of Philox (parity and tests; not with greedy).
+ * Sampling without a tape: Philox stream 4, key = seed (the same for every run), counter = (index, t | 4 << 16,
+ * episode0 + k) with index = e * ceil(N/4) + agent / 4 for env e within its run; agent i takes word i mod 4 and converts it
+ * as the training sampler converts its word: (w >> 8) * 2^-24.  All runs and all evaluations with the same seed / episode0
+ * thus see the same numbers: comparisons between runs are paired.
+ *
+ * Two launches: the policy table (which also zeroes action_counts), then the episodes.
+ * Contract: run r computes byte for byte what an R = 1 call with run r's actor rows computes.  For fixed actor parameters
+ * and an injected tape, returns and action counts are byte-identical to the env part of ia2c_rollout (ep_return, and the
+ * counts of act[0..T-1]) fed U[t] = inj_u_action[0, t] with one episode.  Nothing outside policy, returns and
+ * action_counts is written.
+ * Every check runs before the first CUDA call: a NULL descriptor or output pointer, R, N, E, episodes or T out of range,
+ * R * N above IA2C_MAX_RUN_NETS, E * episodes beyond one grid, episode0 + episodes above 2^32, greedy with
+ * E * episodes != 1 (Org is deterministic: every greedy episode of a run is the same) or with a tape, and a policy
+ * workspace smaller than ia2c_eval_policy_floats(desc). */
+#define IA2C_EVAL_MAX_RUNS 65535     /* R: one grid row per run */
+#define IA2C_EVAL_MAX_AGENTS 1023    /* a step's action counts are packed in 10-bit fields */
+#define IA2C_EVAL_MAX_STEPS 65535    /* T: the t field of the Philox counter is 16 bits */
+typedef struct ia2c_eval_desc {
+    const float* actor_params;       /* f32[R*N, 105] */
+    int32_t R, N;                    /* 1 <= R, 2 <= N <= 1023, R * N <= IA2C_MAX_RUN_NETS */
+    int64_t E;                       /* envs per run */
+    int32_t episodes, T, max_episode_steps, greedy;
+    uint64_t seed;                   /* Philox key (stream 4) */
+    uint32_t episode0;               /* Philox episode of item k is episode0 + k; episode0 + episodes <= 2^32 */
+    const float* inj_u_action;       /* f32[episodes, T, R*E, N] or NULL */
+    float* policy; size_t policy_floats;   /* out and workspace: f32[R*N, 9, 3], ia2c_eval_policy_floats(desc) */
+    double* returns;                 /* out: f64[R, episodes, E] (greedy: f64[R]) */
+    unsigned long long* action_counts;     /* out: u64[R*N, 3] */
+} ia2c_eval_desc;
+size_t ia2c_eval_policy_floats(const ia2c_eval_desc* d);
+int ia2c_evaluate(const ia2c_eval_desc* d, void* stream);
 
 #ifdef __cplusplus
 }
