@@ -25,9 +25,9 @@ def __getattr__(name):  # lazy: torch-dependent classes are imported on first us
     if name in ("IA2CTrainer", "reference_init"):
         from . import trainer
         return getattr(trainer, name)
-    if name == "IA2CRuns":
-        from .runs import IA2CRuns
-        return IA2CRuns
+    if name in ("IA2CRuns", "IA2CRunsMany"):
+        from . import runs
+        return getattr(runs, name)
     if name in ("A2COrgTrainer", "a2c_reference_init"):
         from . import a2c
         return getattr(a2c, name)

@@ -22,7 +22,7 @@ FLAG_ACTOR_COLUMNS = 16
 FLAG_BELIEF_PER_STEP = 32
 FLAG_ROLLOUT_PER_STEP = 64
 BELIEF_RECORD = 8
-ABI_VERSION = 5
+ABI_VERSION = 6
 MAX_RUN_NETS = 65535   # IA2C_MAX_RUN_NETS: runs * n_agents of one batch
 ACTOR_P = 105
 CRITIC_P = 147
@@ -65,7 +65,7 @@ class PeerDesc(C.Structure):
 
 
 class RunsDesc(C.Structure):
-    """Mirror of ``ia2c_runs_desc``: a batch of independent runs (ia2c_train_episode_runs)."""
+    """Mirror of ``ia2c_runs_desc``: a batch of independent runs (ia2c_train_episode_runs, ia2c_train_episode_runs_many)."""
     _fields_ = [("runs", i32), ("reserved", i32), ("seed", vp), ("lr_actor", vp), ("lr_critic", vp), ("gamma", vp), ("beta", vp)]
 
 
@@ -144,6 +144,7 @@ SIGNATURES = {
     "ia2c_train_episodes_host_p2p": (C.c_int, [_DP, vp, C.POINTER(PeerDesc), u32, vp, vp, i32, C.POINTER(vp), vp, vp]),
     "ia2c_runs_partials_floats": (C.c_size_t, [_DP, i32]),
     "ia2c_train_episode_runs": (C.c_int, [_DP, C.POINTER(RunsDesc), vp]),
+    "ia2c_train_episode_runs_many": (C.c_int, [_DP, C.POINTER(RunsDesc), vp]),
     "ia2c_a2c_partials_floats": (C.c_size_t, [C.POINTER(A2CDesc)]),
     "ia2c_a2c_train_update": (C.c_int, [C.POINTER(A2CDesc), vp]),
     "ia2c_eval_policy_floats": (C.c_size_t, [C.POINTER(EvalDesc)]),

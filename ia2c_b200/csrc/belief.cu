@@ -20,6 +20,7 @@
 #include "common.cuh"
 
 namespace ia2c {
+int belief_pairs_episode_runs_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s);   // trainer.cu
 namespace {
 
 constexpr int kThreads = 256;
@@ -748,19 +749,28 @@ constexpr int kEpQuads = 4;                    // quads per lane
 constexpr int kEpWarps = kThreads / 32;
 constexpr int kEpWarpQuads = 32 * kEpQuads;    // quad slots of a warp: an env's KQ quads must fit (N <= 512)
 
-template <int M, bool FAST>
-__global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const __grid_constant__ EpisodePairsArgs P) {
+// RUNS (FAST only): a batch of independent runs (ia2c_train_episode_runs_many), blockIdx.y = run * N + agent is the filter row; the
+// run's envs are columns [run * E, (run + 1) * E) of an env axis of length R * E, `e0` stays the env's index within the run
+// (Philox counters), and the Philox key is the run's seed, read after the wait.
+template <int M, bool FAST, bool RUNS>
+__global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const __grid_constant__ EpisodePairsArgs P, RunsArg<RUNS> ra) {
+    static_assert(FAST || !RUNS, "batches have no dumps or tapes");
     constexpr int A = IA2C_AGENT_ACTIONS;
     const double* const u_injected = FAST ? nullptr : P.u_injected;
     uint8_t* const belief_dump = FAST ? nullptr : P.belief_dump;
     uint8_t* const pred_dump = FAST ? nullptr : P.pred_dump;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int queue_n_w[kEpWarps];   // flagged records of the warp's current step
-    const int N = P.N, K = P.K, i = blockIdx.y;
+    const int N = P.N, K = P.K, i = RUNS ? (int)blockIdx.y % N : blockIdx.y;   // i: the agent
+    const int run = RUNS ? (int)blockIdx.y / N : 0;
     const int KQ = (K + 3) >> 2;
     const int EW = P.envs_per_warp, EWp = (EW + 3) & ~3;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int64_t e0 = ((int64_t)blockIdx.x * kEpWarps + warp) * EW;                 // the warp's first env
+    const int64_t e0 = ((int64_t)blockIdx.x * kEpWarps + warp) * EW;                 // the warp's first env (within its run)
+    // the env axis has n_runs * E columns, the run's start at col0 (both folded away in the standalone form, which thus reads P.E
+    // where it always did)
+    const int n_runs = RUNS ? (int)gridDim.y / N : 1;
+    const int64_t col0 = RUNS ? (int64_t)run * P.E : 0;
     const int n_envs = (int)max((int64_t)0, min((int64_t)EW, P.E - e0));
     double* tab = reinterpret_cast<double*>(smem_raw);               // [104]   k/100
     double* bpt = tab + 104;                                         // [A][M][101]
@@ -773,7 +783,7 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
     uint32_t* seen4 = reinterpret_cast<uint32_t*>(queue - warp * (4 * kEpWarpQuads) + 4 * kEpQuads * kThreads);    // [kEpQuads][kThreads] the others' actions
     pdl_release();
     for (int k = threadIdx.x; k <= 100; k += blockDim.x) tab[k] = __ddiv_rn((double)k, 100.0);
-    for (int k = threadIdx.x; k < M * A; k += blockDim.x) fa[k] = P.filter_action[(int64_t)i * M * A + k];
+    for (int k = threadIdx.x; k < M * A; k += blockDim.x) fa[k] = P.filter_action[(int64_t)(RUNS ? blockIdx.y : i) * M * A + k];
     if (threadIdx.x < kEpWarps) queue_n_w[threadIdx.x] = 0;
     for (int k = threadIdx.x; k < kEpWarps * EWp; k += blockDim.x) (counts - warp * EWp)[k] = 0u;
     __syncthreads();
@@ -793,6 +803,17 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
     pdl_wait();
     __syncthreads();   // the last block-wide barrier: from here on the warps run independently
     if (n_envs == 0) return;
+    // Philox with the round keys of P.rk or, in a batch, keyed by the run's seed: philox4x32_10 derives key_r = key_0 + r * W as
+    // it goes, the formula the host fills P.rk with, so the numbers are the same
+    uint2 run_key = make_uint2(0u, 0u);
+    if constexpr (RUNS) {
+        const uint64_t seed = ra.seed[run];
+        run_key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+    }
+    auto philox = [&](uint4 c) -> uint4 {
+        if constexpr (RUNS) return philox4x32_10(c, run_key);
+        else return philox4x32_10_rk(c, P.rk);
+    };
     float f0[M], f01[M];
 #pragma unroll
     for (int m = 0; m < M; ++m) { f0[m] = fcum[m]; f01[m] = fcum[M + m]; }
@@ -900,7 +921,7 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
     }
     // the actions are written by the kernel before this one: coherent loads (an ld.global.nc may be hoisted above griddepcontrol.wait)
     auto stage_load = [&](int t) {
-        const uint8_t* src8 = P.act + ((int64_t)t * P.E + e0) * N;
+        const uint8_t* src8 = P.act + ((int64_t)t * P.E * n_runs + col0 + e0) * N;
         if (aligned) {
             const uint32_t* src = reinterpret_cast<const uint32_t*>(src8);
 #pragma unroll
@@ -956,7 +977,7 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
             uint32_t words[4] = {0u, 0u, 0u, 0u};
             if (!u_injected) {
                 const uint64_t index = ctr0 + (uint32_t)(live ? el : 0) * row_ctr + (uint32_t)sq;
-                const uint4 rnd = philox4x32_10_rk(make_uint4((uint32_t)index, (uint32_t)(index >> 32), c2, P.episode), P.rk);
+                const uint4 rnd = philox(make_uint4((uint32_t)index, (uint32_t)(index >> 32), c2, P.episode));
                 words[0] = rnd.x; words[1] = rnd.y; words[2] = rnd.z; words[3] = rnd.w;
             }
             const uint32_t seen_w = live ? seen4[s_ * kThreads + threadIdx.x] : 0u;
@@ -1022,7 +1043,7 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
                 u = u_injected[trec];
             } else {
                 const uint64_t index = ctr0 + (uint32_t)el_ * row_ctr + (uint32_t)sq_;
-                const uint4 rnd = philox4x32_10_rk(make_uint4((uint32_t)index, (uint32_t)(index >> 32), c2, P.episode), P.rk);
+                const uint4 rnd = philox(make_uint4((uint32_t)index, (uint32_t)(index >> 32), c2, P.episode));
                 u = belief_word_to_unit_f64(w == 0 ? rnd.x : (w == 1 ? rnd.y : (w == 2 ? rnd.z : rnd.w)));
             }
             const uint32_t seen = (seen4[(ql >> 5) * kThreads + (warp << 5) + (ql & 31)] >> (8 * w)) & 0xFFu;
@@ -1040,7 +1061,7 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
             int best = 0, bc = n0;
             if (n1 > bc) { best = 1; bc = n1; }
             if (n2 > bc) best = 2;                                   // ties -> lowest action
-            P.partner_pred[((int64_t)t * P.E + e0 + x) * N + i] = (uint8_t)best;
+            P.partner_pred[((int64_t)t * P.E * n_runs + col0 + e0 + x) * N + i] = (uint8_t)best;
             counts[x] = 0u;
         }
         if (lane == 0) queue_n_w[warp] = 0;
@@ -1052,7 +1073,7 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
 #pragma unroll
         for (int s_ = 0; s_ < kEpQuads; ++s_) {
             if (lane + 32 * s_ < total) {
-                uint2* wp = reinterpret_cast<uint2*>(P.records + (((e0 + el) * N + i) * (int64_t)K + 4 * sq) * IA2C_BELIEF_RECORD);
+                uint2* wp = reinterpret_cast<uint2*>(P.records + (((col0 + e0 + el) * N + i) * (int64_t)K + 4 * sq) * IA2C_BELIEF_RECORD);
 #pragma unroll
                 for (int w = 0; w < 4; ++w)
                     if (4 * sq + w < K) wp[w] = st_mem[(4 * s_ + w) * kThreads + threadIdx.x];
@@ -1063,24 +1084,46 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
     }
 }
 
+// Launch shape of belief_pairs_episode_kernel for P.E envs (of one run): sets P.envs_per_warp, returns the env blocks (grid x)
+// and the dynamic shared memory.  The standalone and the batched launcher share it, so the batch's shared memory always
+// matches what the kernel carves out of it.
+struct EpisodeShape { int64_t env_blocks; size_t smem; };
 template <int M>
-int launch_pairs_episode(EpisodePairsArgs& P, cudaStream_t stream) {
+EpisodeShape episode_shape(EpisodePairsArgs& P) {
     const int KQ = (P.K + 3) / 4;
     P.envs_per_warp = std::max(1, kEpWarpQuads / KQ);              // whole envs per warp, <= kEpQuads quads per lane
     const int64_t envs_per_block = (int64_t)P.envs_per_warp * kEpWarps;
-    const int64_t env_blocks = (P.E + envs_per_block - 1) / envs_per_block;
-    size_t smem = (104 + 3 * M * 101 + M * 3) * sizeof(double) + (((3 * M * 101 + 3) & ~3) + ((2 * M + 3) & ~3)) * sizeof(float) +
-                  (size_t)kEpWarps * ((P.envs_per_warp + 3) & ~3) * sizeof(uint32_t) +
-                  (size_t)4 * kEpQuads * kThreads * (sizeof(uint2) + sizeof(uint16_t)) + (size_t)kEpQuads * kThreads * sizeof(uint32_t);
-    smem = (smem + 15) & ~size_t(15);
-    dim3 grid((unsigned)env_blocks, P.N);
+    EpisodeShape sh;
+    sh.env_blocks = (P.E + envs_per_block - 1) / envs_per_block;
+    sh.smem = (104 + 3 * M * 101 + M * 3) * sizeof(double) + (((3 * M * 101 + 3) & ~3) + ((2 * M + 3) & ~3)) * sizeof(float) +
+              (size_t)kEpWarps * ((P.envs_per_warp + 3) & ~3) * sizeof(uint32_t) +
+              (size_t)4 * kEpQuads * kThreads * (sizeof(uint2) + sizeof(uint16_t)) + (size_t)kEpQuads * kThreads * sizeof(uint32_t);
+    sh.smem = (sh.smem + 15) & ~size_t(15);
+    return sh;
+}
+
+template <int M>
+int launch_pairs_episode(EpisodePairsArgs& P, cudaStream_t stream) {
+    const EpisodeShape sh = episode_shape<M>(P);
+    const size_t smem = sh.smem;
+    dim3 grid((unsigned)sh.env_blocks, P.N);
     const bool fast = !P.u_injected && !P.belief_dump && !P.pred_dump;
     if (fast) {
-        if (smem > 48 * 1024) cudaFuncSetAttribute(belief_pairs_episode_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, true>, grid, dim3(kThreads), smem, stream, P);
+        if (smem > 48 * 1024) cudaFuncSetAttribute(belief_pairs_episode_kernel<M, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, true, false>, grid, dim3(kThreads), smem, stream, P, NoRuns{});
     }
-    if (smem > 48 * 1024) cudaFuncSetAttribute(belief_pairs_episode_kernel<M, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, false>, grid, dim3(kThreads), smem, stream, P);
+    if (smem > 48 * 1024) cudaFuncSetAttribute(belief_pairs_episode_kernel<M, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, false, false>, grid, dim3(kThreads), smem, stream, P, NoRuns{});
+}
+
+// The batched form (ia2c_train_episode_runs_many): one run's shape, grid (env blocks of one run, R * N).
+template <int M>
+int launch_pairs_episode_runs(EpisodePairsArgs& P, const ia2c_runs_desc& runs, cudaStream_t stream) {
+    const EpisodeShape sh = episode_shape<M>(P);
+    dim3 grid((unsigned)sh.env_blocks, (unsigned)(runs.runs * P.N));
+    if (sh.smem > 48 * 1024)
+        cudaFuncSetAttribute(belief_pairs_episode_kernel<M, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh.smem);
+    return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, true, true>, grid, dim3(kThreads), sh.smem, stream, P, runs);
 }
 
 template <int M>
@@ -1182,5 +1225,19 @@ extern "C" int ia2c_belief_update_pairs_episode(uint8_t* records, const double* 
         case 4: return launch_pairs_episode<4>(P, s);
         case 5: return launch_pairs_episode<5>(P, s);
         default: return launch_pairs_episode<6>(P, s);
+    }
+}
+
+// The whole-episode belief update of a batch of runs (ia2c_train_episode_runs_many, which has validated both descriptors): the
+// stacked trajectory of d (env axis R * E), one filter row per net, each run's seed as its Philox key.
+int ia2c::belief_pairs_episode_runs_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s) {
+    EpisodePairsArgs P{d->belief_records, d->filter_action, d->act, nullptr, nullptr, nullptr, d->partner_pred, d->E, 0, d->N, d->N - 1,
+                       d->T + 1, 0, d->episode, {}};
+    switch (d->M) {
+        case 2: return launch_pairs_episode_runs<2>(P, *runs, s);
+        case 3: return launch_pairs_episode_runs<3>(P, *runs, s);
+        case 4: return launch_pairs_episode_runs<4>(P, *runs, s);
+        case 5: return launch_pairs_episode_runs<5>(P, *runs, s);
+        default: return launch_pairs_episode_runs<6>(P, *runs, s);
     }
 }

@@ -38,6 +38,7 @@ int64_t rollout_fused_blocks(int64_t E, int N);
 int actor_pipe_launch(const ia2c_episode_desc* d, cudaStream_t s);
 int reduce_adam_runs_launch(const ReduceArgs& A, const double* lr_per_net, int nets, cudaStream_t s);   // used by a2c.cu
 int64_t actor_pipe_blocks(int64_t E, int N);
+int belief_pairs_episode_runs_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s);   // belief.cu
 
 namespace {
 
@@ -186,11 +187,17 @@ __global__ void __launch_bounds__(kActorThreads) actor_step_kernel(StepArgs S) {
 //       same-step autoreset) and publish the next observation classes;
 //   (3) every agent derives the mode of the OTHERS' actions (partner_true)
 // with two block barriers per step.  The belief update of the whole episode follows as one kernel (belief.cu).
+// RUNS: a batch of independent runs (ia2c_train_episode_runs_many), blockIdx.y = run.  A block's chunk lies inside one run (its
+// threads hold that run's actors, rows run * N + i); the run's envs are columns [run * E, (run + 1) * E) of an env axis of
+// length R * E (stride ES), and `e` stays the env's index within its run, which keys its Philox counters.
 constexpr int kManyMaxEnvs = 32;     // envs per block
-__global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant__ ia2c_episode_desc d, int envs_per_block) {
+template <bool RUNS>
+__global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant__ ia2c_episode_desc d, int envs_per_block, RunsArg<RUNS> ra) {
     extern __shared__ __align__(16) unsigned char many_smem[];
     const int N = d.N, T = d.T, i = threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
     const int64_t E = d.E, e0 = (int64_t)blockIdx.x * envs_per_block;
+    const int run = RUNS ? (int)blockIdx.y : 0;
+    const int64_t ES = RUNS ? E * gridDim.y : E, g0 = RUNS ? (int64_t)run * E + e0 : e0;   // g0: the chunk's first column
     const int EC = (int)min((int64_t)envs_per_block, E - e0);
     uint32_t* warp_cnt = reinterpret_cast<uint32_t*>(many_smem);                 // [EC][n_warps] packed 3 x 10 bits
     uint32_t* tot_cnt = warp_cnt + kManyMaxEnvs * 8;                              // [EC]
@@ -199,14 +206,14 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
     pdl_prologue();
     const bool agent = i < N;
     RegNet<A> net;
-    if (agent && !d.inj_actions) load_regnet<A>(net, d.actor_params + (int64_t)i * kActorP);
+    if (agent && !d.inj_actions) load_regnet<A>(net, d.actor_params + (int64_t)(RUNS ? run * N + i : i) * kActorP);
     // env state of env el lives in the registers of thread el
     int s = 2, prev_cls = 1, cur_cls = 1, elapsed = 0;
     double hist = 0.0, ep_ret = 0.0;
     const bool owner = i < EC;
     if (owner) {
         cls_s[i] = 1 | (1 << 2);
-        float* o = d.obs + (e0 + i) * F;
+        float* o = d.obs + (g0 + i) * F;
 #pragma unroll
         for (int k = 0; k < F; ++k) o[k] = (k == 1 || k == 4) ? 1.f : 0.f;        // reset observation [0,1,0,0,1,0] (Org.py:128-148)
     }
@@ -217,7 +224,7 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
             const int64_t e = e0 + el;
             int a = 3;   // no action (threads beyond N)
             if (agent) {
-                const int64_t row = ((int64_t)t * E + e) * N + i;
+                const int64_t row = ((int64_t)t * ES + (RUNS ? g0 + el : e)) * N + i;
                 if (d.inj_actions) {
                     a = d.inj_actions[row];
                 } else {
@@ -231,7 +238,7 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
                     forward_regnet<A>(net, x, y);
                     softmax_inplace<A>(y);
                     const float u = d.inj_u_action ? d.inj_u_action[row]
-                                                   : philox_uniform_f32(d.seed, kStreamAction, d.episode, (uint32_t)t,
+                                                   : philox_uniform_f32(run_seed<RUNS>(d, ra, run), kStreamAction, d.episode, (uint32_t)t,
                                                                         (uint64_t)((d.env_offset + e) * N + i));
                     a = sample_inverse_cdf<A>(y, u);
                 }
@@ -249,7 +256,7 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
             for (int w = 0; w < n_warps; ++w) packed += warp_cnt[i * 8 + w];
             tot_cnt[i] = packed;
             if (t < T) {
-                const int64_t e = e0 + i;
+                const int64_t e = g0 + i;
                 const int c0 = packed & 1023, c1 = (packed >> 10) & 1023, c2 = (packed >> 20) & 1023;
                 int s2;
                 double base;
@@ -257,10 +264,10 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
                 double r = org_reward(base, hist);
                 prev_cls = cur_cls;
                 cur_cls = org_obs_class(s2);
-                d.reward[(int64_t)t * E + e] = (float)r;          // float32(r) as stored by ia2c.py:99
+                d.reward[(int64_t)t * ES + e] = (float)r;         // float32(r) as stored by ia2c.py:99
                 ep_ret += r;                                     // fp64, in step order (ia2c.py:102)
-                if (d.state_trace) d.state_trace[(int64_t)t * E + e] = s2;
-                if (d.reward_f64) d.reward_f64[(int64_t)t * E + e] = r;
+                if (d.state_trace) d.state_trace[(int64_t)t * ES + e] = s2;
+                if (d.reward_f64) d.reward_f64[(int64_t)t * ES + e] = r;
                 ++elapsed;
                 if (d.max_episode_steps > 0 && elapsed >= d.max_episode_steps) {   // same-step autoreset (Q14)
                     s2 = 2; r = 0.0; prev_cls = 1; cur_cls = 1; elapsed = 0;
@@ -268,7 +275,7 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
                 s = s2;
                 hist = r;
                 cls_s[i] = prev_cls | (cur_cls << 2);
-                float* o = d.obs + ((int64_t)(t + 1) * E + e) * F;
+                float* o = d.obs + ((int64_t)(t + 1) * ES + e) * F;
 #pragma unroll
                 for (int k = 0; k < F; ++k) o[k] = (k < 3 ? k == prev_cls : k - 3 == cur_cls) ? 1.f : 0.f;
             }
@@ -280,14 +287,14 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
                 const uint32_t packed = tot_cnt[el];
                 const int a = act_s[el * blockDim.x + i];
                 const int c0 = packed & 1023, c1 = (packed >> 10) & 1023, c2 = (packed >> 20) & 1023;
-                d.partner_true[((int64_t)t * E + e0 + el) * N + i] = (uint8_t)mode3(c0 - (a == 0), c1 - (a == 1), c2 - (a == 2));
+                d.partner_true[((int64_t)t * ES + g0 + el) * N + i] = (uint8_t)mode3(c0 - (a == 0), c1 - (a == 1), c2 - (a == 2));
             }
         }
         // (the next step's writes to warp_cnt / act_s come after these reads only per thread for act_s — own entries — and after
         //  the next barrier for tot_cnt; warp_cnt is rewritten before that barrier but was last read before this step's second one)
     }
     if (owner) {   // persist the final env state exactly as the per-step path leaves it
-        const int64_t e = e0 + i;
+        const int64_t e = g0 + i;
         d.env_state[e] = s;
         d.env_hist[e] = hist;
         d.env_elapsed[e] = elapsed;
@@ -316,16 +323,21 @@ __host__ __device__ inline ChunkPlan chunk_plan(int T, int64_t E, int N) {
 }
 
 // partial row layout: P gradient entries then the loss partial.
-__global__ void __launch_bounds__(kGradThreads) critic_grad_kernel(ia2c_episode_desc d, float* __restrict__ partials) {
+// RUNS: a batch of independent runs (ia2c_train_episode_runs_many), laid out as actor_grad_kernel<true> lays them out:
+// blockIdx.y = run * N + agent is the net row, the run's envs are columns [run * E, (run + 1) * E) of an env axis of length R * E.
+template <bool RUNS>
+__global__ void __launch_bounds__(kGradThreads) critic_grad_kernel(ia2c_episode_desc d, float* __restrict__ partials, RunsArg<RUNS> ra) {
     constexpr int P = kCriticP, GN = F2<J>::G2;   // 148 floats = 74 float2
     __shared__ __align__(16) float w[SmemNet<J>::size];
     __shared__ float red[(kGradThreads / 32) * (P + 1)];
     pdl_prologue();
-    const int n = blockIdx.y, N = d.N;
-    stage_smemnet<J>(w, d.critic_params + (int64_t)n * P);
-    if (blockIdx.x == 0 && threadIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.critic_step[n] += 1;
+    const int N = d.N, n = RUNS ? (int)blockIdx.y % N : blockIdx.y;   // n: the agent
+    const int run = RUNS ? (int)blockIdx.y / N : 0;
+    stage_smemnet<J>(w, d.critic_params + (int64_t)(RUNS ? blockIdx.y : n) * P);
+    if (blockIdx.x == 0 && threadIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.critic_step[RUNS ? blockIdx.y : n] += 1;
     __syncthreads();
     const int64_t E = d.E, rows = (int64_t)d.T * E;
+    const int64_t ES = RUNS ? E * (gridDim.y / N) : E;
     const ChunkPlan cp = chunk_plan(d.T, E, N);
     const int64_t items = E * cp.n_chunks;
     const float inv_b = 1.f / (float)((int64_t)d.T * d.E_total);
@@ -334,32 +346,38 @@ __global__ void __launch_bounds__(kGradThreads) critic_grad_kernel(ia2c_episode_
     for (int i = 0; i < GN; ++i) g2[i] = make_float2(0.f, 0.f);
     float loss = 0.f;
     for (int64_t item = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; item < items; item += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t e = item % E;
+        const int64_t e = RUNS ? (int64_t)run * E + item % E : item % E;
         const int t0 = (int)(item / E) * cp.chunk_len;
         const int t1 = min(d.T, t0 + cp.chunk_len);
         float x[kIn], q[J];
         float2 h1[3], h2[3];
-        load_obs6(d.obs + ((int64_t)t0 * E + e) * kIn, x);
+        load_obs6(d.obs + ((int64_t)t0 * ES + e) * kIn, x);
         fwd_f2<J>(w, x, h1, h2, q);
         int carry_idx = -1;          // pending bootstrap gradient for the CURRENT observation (from row t-1)
         float carry_val = 0.f;
         for (int t = t0; t < t1; ++t) {
-            const int64_t r = (int64_t)t * E + e;
+            const int64_t r = (int64_t)t * ES + e;
             float xn[kIn], qn[J];
             float2 h1n[3], h2n[3];
-            load_obs6(d.obs + (r + E) * kIn, xn);                    // next_obs[t] = obs[t+1]
+            load_obs6(d.obs + (r + ES) * kIn, xn);                   // next_obs[t] = obs[t+1]
             fwd_f2<J>(w, xn, h1n, h2n, qn);
-            const int own = d.act[r * N + n], own_n = d.act[(r + E) * N + n];
+            const int own = d.act[r * N + n], own_n = d.act[(r + ES) * N + n];
             const int jt = joint_index(n, N, own, d.partner_true[r * N + n]);            // ia2c.py:112
-            const int nja = joint_index(n, N, own_n, d.partner_pred[(r + E) * N + n]);   // ia2c.py:104-105
-            const float target = d.reward[r] + d.gamma * select_out<J>(qn, nja);         // ia2c.py:110 (Q8)
+            const int nja = joint_index(n, N, own_n, d.partner_pred[(r + ES) * N + n]);  // ia2c.py:104-105
+            // RUNS spells out, with rounding intrinsics, what nvcc 12.9 makes of the standalone instantiation (read off its SASS:
+            // FFMA for reward + gamma * Q', FMULs rounding 2 * gamma * delta and then * inv_b): with gamma loaded per run the
+            // compiler may contract differently, and the batch's runs would drift from the standalone runs in the last bit.
+            const float gamma = run_gamma<RUNS>(d, ra, run);
+            const float target = RUNS ? __fmaf_rn(gamma, select_out<J>(qn, nja), d.reward[r])
+                                      : d.reward[r] + gamma * select_out<J>(qn, nja);   // ia2c.py:110 (Q8)
             const float delta = target - select_out<J>(q, jt);
-            if (d.target_dump) d.target_dump[(int64_t)n * rows + r] = target;
+            if (d.target_dump) d.target_dump[(int64_t)n * rows + r] = target;   // never in a batch (refused)
             loss = fmaf(delta, delta, loss);
-            const float gq = -2.f * delta * inv_b;                   // dL/dQ(obs_t)[jt]
+            const float gq = RUNS ? __fmul_rn(-2.f * delta, inv_b) : -2.f * delta * inv_b;   // dL/dQ(obs_t)[jt]
             bwd_f2<J>(w, x, h1, h2, [&](int o) { return (o == jt ? gq : 0.f) + (o == carry_idx ? carry_val : 0.f); }, g2);
             carry_idx = nja;
-            carry_val = 2.f * d.gamma * delta * inv_b;               // dL/dQ(next_obs_t)[nja]: residual gradient
+            carry_val = RUNS ? __fmul_rn(__fmul_rn(2.f * gamma, delta), inv_b)   // dL/dQ(next_obs_t)[nja]: residual gradient
+                             : 2.f * gamma * delta * inv_b;
 #pragma unroll
             for (int k = 0; k < kIn; ++k) x[k] = xn[k];
 #pragma unroll
@@ -372,7 +390,7 @@ __global__ void __launch_bounds__(kGradThreads) critic_grad_kernel(ia2c_episode_
     float g[2 * GN];
     unpack_g2(g2, g);
     g[P] = loss;
-    block_reduce_store<P + 1>(reinterpret_cast<float(&)[P + 1]>(g), red, partials + ((int64_t)n * gridDim.x + blockIdx.x) * (P + 1));
+    block_reduce_store<P + 1>(reinterpret_cast<float(&)[P + 1]>(g), red, partials + ((int64_t)(RUNS ? blockIdx.y : n) * gridDim.x + blockIdx.x) * (P + 1));
 }
 
 // RUNS: a batch of independent runs (ia2c_train_episode_runs): blockIdx.y = run * N + agent is the net row, the run's envs are
@@ -573,6 +591,30 @@ int grad_blocks(const ia2c_episode_desc* d) {
     return (int)std::max<int64_t>(1, std::min(by_items, by_wave));
 }
 
+// Launch shape of rollout_many_kernel for `runs` runs of d->E envs.  A block walks its envs one after the other, so an episode
+// costs (waves of resident blocks) x (envs per block) — take the envs per block c that minimises it over all runs * ceil(E / c)
+// blocks (1024 x 256: 7 envs = one wave of 147 blocks instead of two waves of 4).  Envs are independent (no sum crosses an env),
+// so the choice changes no result.
+struct ManyPlan { int threads, envs_per_block; size_t smem; int64_t blocks; };   // blocks: per run (grid x)
+template <bool RUNS>
+ManyPlan many_plan(const ia2c_episode_desc* d, int runs) {
+    ManyPlan p;
+    p.threads = ((d->N + 31) / 32) * 32;
+    p.smem = (size_t)kManyMaxEnvs * (8 + 1 + 1) * 4 + (size_t)kManyMaxEnvs * p.threads;
+    static int resident_per_sm[9] = {0};     // per instantiation, by threads / 32; the same on every B200 of the box
+    int& per_sm = resident_per_sm[p.threads / 32];
+    if (per_sm == 0 && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_many_kernel<RUNS>, p.threads, p.smem) != cudaSuccess) per_sm = 1;
+    const int64_t resident = (int64_t)kSMs * std::max(1, per_sm);
+    p.envs_per_block = 1;
+    int64_t best = INT64_MAX;
+    for (int c = 1; c <= std::min(kManyMaxEnvs, p.threads); ++c) {   // one owner thread per env of the chunk
+        const int64_t blocks = runs * ((d->E + c - 1) / c), cost = ((blocks + resident - 1) / resident) * c;
+        if (cost <= best) { best = cost; p.envs_per_block = c; }   // ties: the larger chunk (fewer blocks, weights loaded once per more envs)
+    }
+    p.blocks = (d->E + p.envs_per_block - 1) / p.envs_per_block;
+    return p;
+}
+
 int validate(const ia2c_episode_desc* d, const char* who) {
     IA2C_REQUIRE(d != nullptr, "%s: null descriptor", who);
     IA2C_REQUIRE(d->E > 0 && d->E_total >= d->E && d->T > 0 && d->T < 65535, "%s: E=%lld E_total=%lld T=%d", who,
@@ -633,22 +675,10 @@ extern "C" int ia2c_rollout(const ia2c_episode_desc* d, void* stream) {
     const bool episode_beliefs = !(d->flags & IA2C_FLAG_BELIEF_PER_STEP) && ia2c_belief_supports_episode(d->N, d->M);
     if (episode_beliefs && !(d->flags & IA2C_FLAG_ROLLOUT_PER_STEP) && d->N <= 256) {
         // ONE persistent kernel for the T+1 env / actor steps, then ONE kernel for the episode's belief updates
-        const int threads = ((d->N + 31) / 32) * 32;
-        const size_t smem = (size_t)kManyMaxEnvs * (8 + 1 + 1) * 4 + (size_t)kManyMaxEnvs * threads;
-        // envs per block: a block walks its envs one after the other, so an episode costs (waves of resident blocks) x (envs per
-        // block) — take the split that minimises it (1024 x 256: 7 envs = one wave of 147 blocks instead of two waves of 4)
-        static int resident_per_sm[9] = {0};     // by threads / 32; the same on every B200 of the box
-        int& per_sm = resident_per_sm[threads / 32];
-        if (per_sm == 0 && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_many_kernel, threads, smem) != cudaSuccess) per_sm = 1;
-        const int64_t resident = (int64_t)kSMs * std::max(1, per_sm);
-        int epb = 1;
-        int64_t best = INT64_MAX;
-        for (int c = 1; c <= std::min(kManyMaxEnvs, threads); ++c) {   // one owner thread per env of the chunk
-            const int64_t blocks = (d->E + c - 1) / c, cost = ((blocks + resident - 1) / resident) * c;
-            if (cost <= best) { best = cost; epb = c; }   // ties: the larger chunk (fewer blocks, weights loaded once per more envs)
-        }
-        const int64_t grid = (d->E + epb - 1) / epb;
-        if (int rc = launch_pdl("rollout_many_kernel", rollout_many_kernel, dim3((unsigned)grid), dim3(threads), smem, s, *d, epb)) return rc;
+        const ManyPlan mp = many_plan<false>(d, 1);
+        if (int rc = launch_pdl("rollout_many_kernel", rollout_many_kernel<false>, dim3((unsigned)mp.blocks), dim3(mp.threads), mp.smem, s,
+                                *d, mp.envs_per_block, NoRuns{}))
+            return rc;
         return ia2c_belief_update_pairs_episode(d->belief_records, d->filter_action, d->act, d->inj_u_belief, d->pred_dump, d->belief_dump,
                                                 d->partner_pred, d->E, d->N, d->M, d->T + 1, d->seed, d->episode, d->env_offset, stream);
     }
@@ -867,7 +897,7 @@ extern "C" int ia2c_critic_phase(const ia2c_episode_desc* d, void* stream) {
     cudaStream_t s = as_stream(stream);
     if (!fused_critic(d)) {   // otherwise the rollout kernel's critic stage already wrote the partials
         dim3 grid(grad_blocks(d), d->N);
-        if (int rc = launch_pdl("critic_grad_kernel", critic_grad_kernel, grid, dim3(kGradThreads), 0, s, *d, d->partials)) return rc;
+        if (int rc = launch_pdl("critic_grad_kernel", critic_grad_kernel<false>, grid, dim3(kGradThreads), 0, s, *d, d->partials, NoRuns{})) return rc;
     }
     if (d->flags & IA2C_FLAG_GRAD_ONLY) return 0;
     return run_reduce(d, 0, 1, !(d->flags & IA2C_FLAG_SKIP_ADAM), s);
@@ -1159,7 +1189,7 @@ extern "C" int ia2c_train_episode_timed(const ia2c_episode_desc* d, float* host_
     cudaEventRecord(ev[0], s);
     rc = ia2c_rollout(d, stream);
     cudaEventRecord(ev[1], s);
-    if (!rc && !fused_critic(d)) { critic_grad_kernel<<<grid, kGradThreads, 0, s>>>(*d, d->partials); rc = check_launch("critic_grad_kernel"); }
+    if (!rc && !fused_critic(d)) { critic_grad_kernel<false><<<grid, kGradThreads, 0, s>>>(*d, d->partials, NoRuns{}); rc = check_launch("critic_grad_kernel"); }
     cudaEventRecord(ev[2], s);
     if (!rc) rc = run_reduce(d, 0, 1, apply, s);
     cudaEventRecord(ev[3], s);
@@ -1251,24 +1281,86 @@ static int validate_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r) {
     return 0;
 }
 
+// reduce + Adam of a batch's R * N critics (which = 0) or actors (1), each net with its run's learning rate; `e` carries the
+// internal flags, which select the partial-row count of the producing kernel
+static int reduce_runs(const ia2c_episode_desc& e, const ia2c_runs_desc* r, int which, cudaStream_t s) {
+    const int nets = r->runs * e.N;
+    ReduceArgs A = make_reduce_args(e, which, which == 0 ? critic_partial_blocks(&e) : actor_partial_blocks(&e));
+    A.loss_out = e.loss_out + (which == 0 ? 0 : nets);
+    const ReduceRuns rr = {which == 0 ? r->lr_critic : r->lr_actor, e.N};
+    dim3 grid(nets, ceil_div(A.P + 1, 32));
+    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr);
+}
+
 extern "C" int ia2c_train_episode_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream) {
     if (int rc = validate_runs(d, r)) return rc;
     cudaStream_t s = as_stream(stream);
     const int R = r->runs, nets = R * d->N;
     ia2c_episode_desc e = *d;
     e.flags = IA2C_FLAG_FUSED_ROLLOUT | IA2C_FLAG_FUSED_CRITIC | IA2C_FLAG_ACTOR_COLUMNS;
-    auto reduce = [&](int which) {   // which = 0 critics, 1 actors: the R * N nets, each with its run's learning rate
-        ReduceArgs A = make_reduce_args(e, which, which == 0 ? critic_partial_blocks(&e) : actor_partial_blocks(&e));
-        A.loss_out = e.loss_out + (which == 0 ? 0 : nets);
-        const ReduceRuns rr = {which == 0 ? r->lr_critic : r->lr_actor, d->N};
-        dim3 grid(nets, ceil_div(A.P + 1, 32));
-        return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr);
-    };
     if (int rc = rollout_fused_launch(&e, r, s)) return rc;
-    if (int rc = reduce(0)) return rc;
+    if (int rc = reduce_runs(e, r, 0, s)) return rc;
     dim3 grid(grad_blocks(&e), nets);
     if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
-    return reduce(1);
+    return reduce_runs(e, r, 1, s);
+}
+
+// ------------------------------------------------------------------------------------------------
+// A batch of R independent Org-N runs (9 <= N <= 256) in the six launches of one episode (include/ia2c_b200.h:
+// ia2c_train_episode_runs_many): the standalone N > 8 path of ia2c_rollout + the column actor kernel, every kernel with the run as
+// one more grid dimension and each run partitioned exactly as a standalone run of E envs.
+static int validate_runs_many(const ia2c_episode_desc* d, const ia2c_runs_desc* r) {
+    const char* who = "ia2c_train_episode_runs_many";
+    if (int rc = validate(d, who)) return rc;
+    IA2C_REQUIRE(r != nullptr, "%s: null runs descriptor", who);
+    IA2C_REQUIRE(r->runs >= 1, "%s: runs=%d, need at least 1", who, r->runs);
+    IA2C_REQUIRE((int64_t)r->runs * d->N <= IA2C_MAX_RUN_NETS, "%s: runs * N = %lld above IA2C_MAX_RUN_NETS = %d", who,
+                 (long long)r->runs * d->N, IA2C_MAX_RUN_NETS);
+    IA2C_REQUIRE(r->seed != nullptr, "%s: null seed array (one Philox key per run)", who);
+    auto unsupported = [](const char* what, const char* who) {
+        set_error("%s: %s", who, what);
+        return IA2C_ERR_UNSUPPORTED;
+    };
+    if (d->N <= 8) {
+        set_error("%s: N=%d: batches of N <= 8 agents run on the fused path, ia2c_train_episode_runs", who, d->N);
+        return IA2C_ERR_UNSUPPORTED;
+    }
+    if (d->N > 256) {
+        set_error("%s: N=%d above 256 (the per-step env / actor kernels have no batched form)", who, d->N);
+        return IA2C_ERR_UNSUPPORTED;
+    }
+    if (d->env_offset != 0 || d->E_total != d->E)
+        return unsupported("batches run on one GPU: desc.env_offset must be 0 and desc.E_total == desc.E (envs per run)", who);
+    if (d->inj_actions || d->inj_u_action || d->inj_u_belief) return unsupported("injected replay tapes are not supported in batches", who);
+    if (d->state_trace || d->reward_f64 || d->pred_dump || d->belief_dump || d->adv_dump || d->target_dump)
+        return unsupported("parity dumps are not supported in batches", who);
+    if (d->flags != IA2C_FLAG_ACTOR_COLUMNS)
+        return unsupported("desc.flags must be exactly ACTOR_COLUMNS (the batch runs the column actor kernel)", who);
+    IA2C_REQUIRE(d->env_state && d->env_hist && d->env_cls && d->env_elapsed && d->ep_return && d->belief_records && d->filter_action,
+                 "%s: null env/belief pointer", who);
+    IA2C_REQUIRE(d->critic_grad && d->actor_grad && d->critic_m && d->critic_v && d->actor_m && d->actor_v && d->actor_grad_accum &&
+                     d->critic_step && d->actor_step && d->loss_out, "%s: null optimiser pointer", who);
+    IA2C_REQUIRE(d->partials && d->partials_floats >= ia2c_runs_partials_floats(d, r->runs), "%s: partials workspace too small (%zu < %zu)",
+                 who, d->partials_floats, ia2c_runs_partials_floats(d, r->runs));
+    return 0;
+}
+
+extern "C" int ia2c_train_episode_runs_many(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream) {
+    if (int rc = validate_runs_many(d, r)) return rc;
+    cudaStream_t s = as_stream(stream);
+    const int R = r->runs, nets = R * d->N;
+    ia2c_episode_desc e = *d;
+    e.flags = IA2C_FLAG_ACTOR_COLUMNS;   // both reductions sum grad_blocks(E) partial rows per net
+    const ManyPlan mp = many_plan<true>(&e, R);
+    if (int rc = launch_pdl("rollout_many_kernel", rollout_many_kernel<true>, dim3((unsigned)mp.blocks, (unsigned)R), dim3(mp.threads), mp.smem,
+                            s, e, mp.envs_per_block, *r))
+        return rc;
+    if (int rc = belief_pairs_episode_runs_launch(&e, r, s)) return rc;
+    const dim3 grid(grad_blocks(&e), nets);
+    if (int rc = launch_pdl("critic_grad_kernel", critic_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
+    if (int rc = reduce_runs(e, r, 0, s)) return rc;
+    if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
+    return reduce_runs(e, r, 1, s);
 }
 
 // reduce_adam_kernel<true> for `nets` nets of P entries with one learning rate per net (lr_per_net, or A.lr where NULL): the

@@ -4,6 +4,8 @@ One episode of every run is ONE C call (``ia2c_train_episode_runs``) whose four 
 standalone episode is latency-bound and leaves most of the B200 idle, so R runs cost far less than R standalone
 episodes.  Run r computes byte for byte what ``IA2CTrainer(envs_per_run, seed=seeds[r], init=reference_init(N, M,
 seed=seeds[r]), <run r's hyper-parameters>)`` computes over the same episodes (include/ia2c_b200.h states the contract).
+``IA2CRunsMany`` does the same for Org-N runs of 9 to 256 agents in SIX launches per episode (``ia2c_train_episode_runs_many``);
+its run r is byte-identical to that trainer with ``actor_kernel="columns"``.
 
 The device buffers hold the runs stacked (DESIGN.md §3): per-net buffers have R*N rows, run r at rows [r*N, (r+1)*N);
 per-env buffers have an env axis of length R*E, run r at [r*E, (r+1)*E).  ``run_view(r)`` returns those slices and
@@ -44,6 +46,16 @@ def _per_run(name, value, R, dtype):
 
 
 class IA2CRuns:
+    # the C entry point of one batched episode and the descriptor flags it takes
+    _ENTRY = "ia2c_train_episode_runs"
+    _FLAGS = _lib.FLAG_FUSED_ROLLOUT | _lib.FLAG_FUSED_CRITIC | _lib.FLAG_ACTOR_COLUMNS
+
+    @classmethod
+    def _check_shape(cls, lib, N, M):
+        """Raises ValueError, before any device work, for an (n_agents, n_models) the entry point has no kernels for."""
+        if not lib.ia2c_rollout_fused_supported(N, M):
+            raise ValueError(f"n_agents={N}, n_models={M}: batches of runs need the fused path (N <= 8 with M = 5, or N = 2 with M = 3)")
+
     def __init__(self, envs_per_run, seeds, n_agents=2, n_models=5, steps_per_episode=30, max_episode_steps=30,
                  lr_critic=0.0002, lr_actor=0.0001, beta=0.001, gamma=0.9, init=None, device=None):
         self.lib = _lib.load()
@@ -55,8 +67,7 @@ class IA2CRuns:
             raise ValueError("seeds must lie in [0, 2**64)")
         if E < 1 or not 0 < T < 65535:
             raise ValueError(f"envs_per_run={E} must be >= 1 and steps_per_episode={T} in 1..65534")
-        if not self.lib.ia2c_rollout_fused_supported(N, M):
-            raise ValueError(f"n_agents={N}, n_models={M}: batches of runs need the fused path (N <= 8 with M = 5, or N = 2 with M = 3)")
+        self._check_shape(self.lib, N, M)
         if R * N > _lib.MAX_RUN_NETS:
             raise ValueError(f"runs * n_agents = {R * N} above the limit of {_lib.MAX_RUN_NETS}")
         hyper = {name: _per_run(name, v, R, dt) for name, v, dt in
@@ -97,7 +108,7 @@ class IA2CRuns:
         d.N, d.T, d.M, d.max_episode_steps = N, T, M, int(max_episode_steps or 0)
         d.lr_actor, d.lr_critic = hyper["lr_actor"][1], hyper["lr_critic"][1]
         d.gamma, d.beta = hyper["gamma"][1], hyper["beta"][1]
-        d.flags = _lib.FLAG_FUSED_ROLLOUT | _lib.FLAG_FUSED_CRITIC | _lib.FLAG_ACTOR_COLUMNS
+        d.flags = self._FLAGS
         for name in _NET + tuple(_ENV) + ("loss_out",):
             setattr(d, name, getattr(self, name).data_ptr())
         n_part = int(self.lib.ia2c_runs_partials_floats(C.byref(d), R))
@@ -123,9 +134,9 @@ class IA2CRuns:
         """One episode of every run in one C call; asynchronous unless ``sync_stats``."""
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.ia2c_train_episode_runs(C.byref(self.desc), C.byref(self.runs_desc),
-                                                        torch.cuda.current_stream(self.device).cuda_stream),
-                       "ia2c_train_episode_runs")
+            _lib.check(getattr(self.lib, self._ENTRY)(C.byref(self.desc), C.byref(self.runs_desc),
+                                                      torch.cuda.current_stream(self.device).cuda_stream),
+                       self._ENTRY)
         self.episode += 1
         if sync_stats:
             return self.read_stats()
@@ -159,7 +170,8 @@ class IA2CRuns:
 
     def run_state_dict(self, r):
         """Run r as a checkpoint of a standalone ``IA2CTrainer(envs_per_run, ..., seed=seeds[r])``: its
-        ``load_state_dict`` accepts it and the run continues alone bit-identically."""
+        ``load_state_dict`` accepts it and the run continues alone bit-identically in
+        ``IA2CTrainer(..., actor_kernel="columns")`` (the default up to 64 agents)."""
         torch.cuda.current_stream(self.device).synchronize()
         v = self.run_view(r)
         sd = {k: v[k].detach().cpu().clone() for k in IA2CTrainer._CKPT_TENSORS}
@@ -209,3 +221,31 @@ class IA2CRuns:
 
     def agent_steps_per_episode(self):
         return self.R * self.E * self.N * self.T
+
+
+class IA2CRunsMany(IA2CRuns):
+    """R independent Org-N runs with 9 <= n_agents <= 256 (cfg4: 64 agents, cfg5: 256) in the six launches of one episode
+    (``ia2c_train_episode_runs_many``): the whole-episode rollout and belief kernels, the critic gradient, the column actor
+    gradient and both reduce + Adam steps, each covering all runs.  Run r computes byte for byte what
+    ``IA2CTrainer(envs_per_run, n_agents=N, n_models=M, seed=seeds[r], init=reference_init(N, M, seed=seeds[r]),
+    actor_kernel="columns", <run r's hyper-parameters>)`` computes.  Above 64 agents a standalone trainer defaults to the
+    pipelined actor kernel, whose sums are ordered differently: the contract is with the column kernel.
+
+    Layout, statistics, ``run_view`` / ``run_state_dict``, checkpoints and ``evaluate`` are those of ``IA2CRuns``."""
+    _ENTRY = "ia2c_train_episode_runs_many"
+    _FLAGS = _lib.FLAG_ACTOR_COLUMNS
+
+    @classmethod
+    def _check_shape(cls, lib, N, M):
+        if N <= 8:
+            raise ValueError(f"n_agents={N}: batches of N <= 8 agents run on the fused path, IA2CRuns")
+        if N > 256:
+            raise ValueError(f"n_agents={N} above 256: batches of runs cover 9..256 agents")
+        if not lib.ia2c_belief_supports_episode(N, M):
+            raise ValueError(f"n_models={M} outside 2..6")
+
+    def __init__(self, envs_per_run, seeds, n_agents, n_models=5, steps_per_episode=30, max_episode_steps=30,
+                 lr_critic=0.0002, lr_actor=0.0001, beta=0.001, gamma=0.9, init=None, device=None):
+        super().__init__(envs_per_run, seeds, n_agents=n_agents, n_models=n_models, steps_per_episode=steps_per_episode,
+                         max_episode_steps=max_episode_steps, lr_critic=lr_critic, lr_actor=lr_actor, beta=beta, gamma=gamma,
+                         init=init, device=device)

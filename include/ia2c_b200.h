@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define IA2C_ABI_VERSION 5
+#define IA2C_ABI_VERSION 6
 #define IA2C_HIDDEN 6          /* ac_nets.py:24 */
 #define IA2C_OBS_FEATURES 6    /* Org observation: [onehot3(prev class), onehot3(class)]  Org.py:37,112-114 */
 #define IA2C_AGENT_ACTIONS 3   /* ia2c.py:44 */
@@ -380,7 +380,8 @@ int ia2c_train_episodes_host_p2p(const ia2c_episode_desc* d, ia2c_host_pipe* pip
  *                    act / partner_true / partner_pred [T+1, R*E, N]): the env axis has length R*E, run r at [r*E, (r+1)*E);
  *   loss_out         float[2, R*N] (critic losses of all nets, then actor losses);
  *   partials         ia2c_runs_partials_floats(d, R) floats.
- * Supported: the fused path only (ia2c_rollout_fused_supported(N, M): N <= 8), one GPU, Philox sampling.  desc.flags may
+ * Supported: the fused path only (ia2c_rollout_fused_supported(N, M): N <= 8), one GPU, Philox sampling; batches of
+ * 9 <= N <= 256 agents have their own entry point, ia2c_train_episode_runs_many (below).  desc.flags may
  * carry only FUSED_ROLLOUT, FUSED_CRITIC and ACTOR_COLUMNS (the path is always that one).  Refused with
  * IA2C_ERR_UNSUPPORTED: other (N, M), a non-zero env_offset or E_total != E (multi-GPU), injected replay tapes, parity
  * dumps, other flags.  Refused with IA2C_ERR_INVALID: runs < 1, runs * N > IA2C_MAX_RUN_NETS (the actor-gradient grid
@@ -400,6 +401,30 @@ size_t ia2c_runs_partials_floats(const ia2c_episode_desc* d, int32_t runs);
 /* One episode of every run: fused rollout + critic gradient, critic reduce + Adam, actor gradient, actor reduce + Adam —
  * the four launches of a standalone episode, each covering all R runs. */
 int ia2c_train_episode_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream);
+
+/* A batch of R independent Org-N runs with 9 <= N <= 256 agents, in SIX launches per episode whatever R is.  Same descriptors
+ * and the same stacked layout as ia2c_train_episode_runs (above): per-net rows R*N, env axis R*E, loss_out float[2, R*N],
+ * partials ia2c_runs_partials_floats(d, R) floats; desc.flags = IA2C_FLAG_ACTOR_COLUMNS.
+ *
+ * Contract: run r computes byte for byte what ia2c_train_episode computes for a standalone run of E envs with desc.seed =
+ * seed[r], flags = ACTOR_COLUMNS (the whole-episode rollout and belief kernels, then the column actor kernel) and the run's
+ * lr_actor / lr_critic / gamma / beta — trajectory, belief records, partner_pred, returns, losses, gradients, Adam moments, step
+ * counters, actor grad_accum and parameters.  (Above N = 64 a standalone trainer defaults to the pipelined actor kernel, whose
+ * sums are ordered differently: the contract is with the column kernel.)  Philox counters use the env's index within its run.
+ *
+ * Launches (grid x, y; each run partitioned exactly as a standalone run of E envs, so every fixed-order sum is the same sum):
+ *   1. rollout_many_kernel          (ceil(E / c), R): c envs per block, chosen once for the batch (waves over R * ceil(E / c)
+ *                                   blocks x c); one block's envs lie in one run;
+ *   2. belief_pairs_episode_kernel  (env blocks of one run, R*N): blockIdx.y = run*N + agent is the filter row;
+ *   3. critic_grad_kernel           (grad_blocks(E), R*N);
+ *   4. reduce_adam_kernel (critics) (R*N, ceil(148 / 32));
+ *   5. actor_grad_kernel            (grad_blocks(E), R*N), the column kernel;
+ *   6. reduce_adam_kernel (actors)  (R*N, ceil(106 / 32)).
+ * Refused with IA2C_ERR_UNSUPPORTED: N <= 8 (use ia2c_train_episode_runs), N > 256, a non-zero env_offset or E_total != E,
+ * injected replay tapes, parity dumps, flags other than exactly IA2C_FLAG_ACTOR_COLUMNS.  Refused with IA2C_ERR_INVALID:
+ * runs < 1, runs * N > IA2C_MAX_RUN_NETS, a NULL seed array, M outside 2..6, missing buffers, a workspace smaller than
+ * ia2c_runs_partials_floats(d, R).  Every check runs before the first CUDA call. */
+int ia2c_train_episode_runs_many(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream);
 
 /* ------------------------------------------------------------------ native A2C trainer (a2c_org_test.py) -- */
 /* One update of a2c_org_test.py:43-92 for R independent runs x E envs: a single joint agent with 9 actions, actor and
