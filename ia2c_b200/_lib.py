@@ -93,6 +93,11 @@ class EvalDesc(C.Structure):
     ]
 
 
+class HistoryDesc(C.Structure):
+    """Mirror of ``ia2c_history_desc``: the device ring of per-episode statistics (ia2c_record_episode)."""
+    _fields_ = [("capacity", i32), ("return_sum", vp), ("loss", vp), ("action_counts", vp), ("partner_hits", vp)]
+
+
 _DP = C.POINTER(EpisodeDesc)
 
 # name -> (restype, argtypes); every symbol declared in include/ia2c_b200.h
@@ -149,6 +154,7 @@ SIGNATURES = {
     "ia2c_a2c_train_update": (C.c_int, [C.POINTER(A2CDesc), vp]),
     "ia2c_eval_policy_floats": (C.c_size_t, [C.POINTER(EvalDesc)]),
     "ia2c_evaluate": (C.c_int, [C.POINTER(EvalDesc), vp]),
+    "ia2c_record_episode": (C.c_int, [_DP, i32, C.POINTER(HistoryDesc), i32, vp]),
 }
 
 _lib = None

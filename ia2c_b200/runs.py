@@ -20,6 +20,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .history import RecordsHistory
 from .trainer import N_ACTIONS, N_FEATURES, IA2CTrainer, reference_init
 
 # buffers with one row per (run, agent), and buffers with an env axis (its position) of length R * E
@@ -45,7 +46,7 @@ def _per_run(name, value, R, dtype):
     return arr.astype(dtype), float(arr[0])
 
 
-class IA2CRuns:
+class IA2CRuns(RecordsHistory):
     # the C entry point of one batched episode and the descriptor flags it takes
     _ENTRY = "ia2c_train_episode_runs"
     _FLAGS = _lib.FLAG_FUSED_ROLLOUT | _lib.FLAG_FUSED_CRITIC | _lib.FLAG_ACTOR_COLUMNS
@@ -131,7 +132,9 @@ class IA2CRuns:
 
     # ------------------------------------------------------------------ episodes
     def train_episode(self, sync_stats=False):
-        """One episode of every run in one C call; asynchronous unless ``sync_stats``."""
+        """One episode of every run in one C call; asynchronous unless ``sync_stats``.  ``train_episodes(n)`` trains n
+        episodes and records their statistics on the device for ``history()``; those episodes do not enter the
+        ``read_stats`` windows."""
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):
             _lib.check(getattr(self.lib, self._ENTRY)(C.byref(self.desc), C.byref(self.runs_desc),
@@ -140,6 +143,12 @@ class IA2CRuns:
         self.episode += 1
         if sync_stats:
             return self.read_stats()
+
+    def _history_dims(self):
+        return self.R, self.N, self.E, self.T, False
+
+    def _enqueue_episode(self, desc_ref, stream):
+        _lib.check(getattr(self.lib, self._ENTRY)(desc_ref, C.byref(self.runs_desc), stream), self._ENTRY)
 
     def read_stats(self):
         """The last episode's losses ``[R, N]`` and returns ``[R, E]``, appended to each run's windows as
@@ -231,7 +240,8 @@ class IA2CRunsMany(IA2CRuns):
     actor_kernel="columns", <run r's hyper-parameters>)`` computes.  Above 64 agents a standalone trainer defaults to the
     pipelined actor kernel, whose sums are ordered differently: the contract is with the column kernel.
 
-    Layout, statistics, ``run_view`` / ``run_state_dict``, checkpoints and ``evaluate`` are those of ``IA2CRuns``."""
+    Layout, statistics, recorded histories (``train_episodes`` / ``history``), ``run_view`` / ``run_state_dict``, checkpoints
+    and ``evaluate`` are those of ``IA2CRuns``."""
     _ENTRY = "ia2c_train_episode_runs_many"
     _FLAGS = _lib.FLAG_ACTOR_COLUMNS
 

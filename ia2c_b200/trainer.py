@@ -18,6 +18,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
+from .history import RecordsHistory
 from .nets import hidden_size
 from .sharding import shard_envs
 
@@ -46,7 +47,7 @@ def reference_init(n_agents, n_models, seed=None):
     return actor, critic, np.stack(fa)
 
 
-class IA2CTrainer:
+class IA2CTrainer(RecordsHistory):
     def __init__(self, num_envs, n_agents=2, n_models=5, steps_per_episode=30, max_episode_steps=30,
                  lr_critic=0.0002, lr_actor=0.0001, beta=0.001, gamma=0.9, seed=0, device=None,
                  rank=0, world_size=1, process_group=None, dumps=False, fused_rollout=None, fused_critic=None,
@@ -264,7 +265,9 @@ class IA2CTrainer:
         dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=self.pg)
 
     def train_episode(self, sync_stats=False):
-        """One episode: rollout, critic update, actor update.  Asynchronous unless ``sync_stats``."""
+        """One episode: rollout, critic update, actor update.  Asynchronous unless ``sync_stats``.  ``train_episodes(n)``
+        (one GPU) trains n episodes and records their statistics on the device for ``history()``; those episodes do not
+        enter the ``read_stats`` windows."""
         if self.world == 1:   # one C call for the whole episode
             self.desc.episode = self.episode
             with torch.cuda.device(self.device):
@@ -281,6 +284,17 @@ class IA2CTrainer:
         self.episode += 1
         if sync_stats:
             return self.read_stats()
+
+    # ---- learning curves recorded on the device (ia2c_b200/history.py: train_episodes, history) --------------------
+    def _check_history(self):
+        if self.world > 1:
+            raise _lib.IA2CError("train_episodes records histories on one GPU (a rank sees only its env shard)")
+
+    def _history_dims(self):
+        return 1, self.N, self.E, self.T, True
+
+    def _enqueue_episode(self, desc_ref, stream):
+        _lib.check(self.lib.ia2c_train_episode(desc_ref, stream), "ia2c_train_episode")
 
     def train_episode_host(self, host_u_action, host_u_belief):
         """End-to-end form with HOST inputs/outputs: pinned uniforms in, losses + episode returns out;

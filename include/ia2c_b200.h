@@ -522,6 +522,40 @@ typedef struct ia2c_eval_desc {
 size_t ia2c_eval_policy_floats(const ia2c_eval_desc* d);
 int ia2c_evaluate(const ia2c_eval_desc* d, void* stream);
 
+/* ------------------------------------------------------------------ learning curves: per-episode statistics on the device -- */
+/* Reduces the trajectory an episode just left into slot `slot` of a caller-owned ring, in ONE launch, so that learning curves
+ * are read back in bulk instead of with a stream synchronisation per episode.  `d` is the descriptor the episode ran with: a
+ * standalone trainer's (runs = 1) or a batch's stacked one (ia2c_runs_desc layout, E = envs per run, runs = R).  Read:
+ * act, partner_true, partner_pred u8[T+1, R*E, N], ep_return f64[R*E], loss_out f32[2, R*N]; any path that fills them
+ * (fused, whole-episode, per-step, injected tapes) is covered.  Nothing else of `d` is read and nothing of it is written.
+ *
+ * Definitions, for run r, agent i (net n = r*N + i) and all steps 0 <= t < T (the T steps the env took) and envs 0 <= e < E:
+ *   action_counts[slot, n, a] = #{ act[t, r*E+e, i] == a }                                   (a = 0, 1, 2)
+ *   partner_hits[slot, n]     = #{ partner_pred[t, r*E+e, i] == partner_true[t, r*E+e, i] }  (the belief filter's hit count)
+ *   loss[slot]                = loss_out, byte for byte (critic row, then actor row)
+ *   return_sum[slot, r]       = the run's E returns summed in a fixed order: lane j of 256 adds ep_return[r*E + j],
+ *                               [r*E + j + 256], [r*E + j + 512], ... in increasing order from +0.0, then a halving tree
+ *                               combines the lanes (s[j] += s[j + w] for j < w, w = 128, 64, ..., 1) and the sum is s[0];
+ *                               every addition is one IEEE fp64 add, round to nearest.  The same bytes from run to run.
+ *
+ * The ring (device, allocated zeroed by the caller): capacity >= 2 slots of each array.  The call writes return_sum and
+ * loss of slot s, ADDS the counts and hits of this episode into slot s with integer atomics, and zeroes the counts and hits
+ * of slot (s + 1) mod capacity for the next call; it writes nothing else.  So slot s must hold zero counts when the call
+ * runs (a zeroed ring, or the previous call on slot s - 1), and slot (s + 1) mod capacity must have been read before the call
+ * on slot s is enqueued: the ring holds at most capacity - 1 episodes that have not been read.
+ * Launched with programmatic dependent launch; the trajectory is read after the wait through L2.
+ * Every check runs before the first CUDA call: a NULL descriptor or pointer, runs < 1, N, T or E < 1, runs * N above
+ * IA2C_MAX_RUN_NETS, capacity < 2 and a slot outside [0, capacity) (IA2C_ERR_INVALID); env_offset != 0 or E_total != E
+ * (a multi-GPU shard; IA2C_ERR_UNSUPPORTED); T * E >= 2^32 (u32 counts; IA2C_ERR_INVALID). */
+typedef struct ia2c_history_desc {
+    int32_t capacity;                 /* episodes the ring holds, >= 2 */
+    double* return_sum;               /* out f64[capacity, R]: sum of ep_return over the run's E envs */
+    float* loss;                      /* out f32[capacity, 2, R*N]: copy of loss_out (critic row, actor row) */
+    uint32_t* action_counts;          /* out u32[capacity, R*N, 3] */
+    uint32_t* partner_hits;           /* out u32[capacity, R*N] */
+} ia2c_history_desc;
+int ia2c_record_episode(const ia2c_episode_desc* d, int32_t runs, const ia2c_history_desc* h, int32_t slot, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
