@@ -111,7 +111,10 @@ def ia2c_rollout(st: IA2CState, E, actions=None, u_act=None, u_belief=None):
                 BEL[t, :, i, jj] = bprime
                 prior[:, i, jj] = bprime                                    # rounded posterior is next prior (Q10)
     return dict(obs=OBS, reward=REW, state=STATE, act=ACT, pred=PRED, belief=BEL, probs=PROBS,
-                ep_return=REW.sum(0))
+                ep_return=REW.sum(0),
+                # env state after the episode's T steps (and their autoresets), in the device's layout
+                env_state=env.state.astype(np.int32), env_hist=env.reward.copy(),
+                env_cls=np.stack([env.prev_cls, env.cls], axis=-1).astype(np.uint8), env_elapsed=env.elapsed.astype(np.int32))
 
 
 def partner_actions(traj, n):
