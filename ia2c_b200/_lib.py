@@ -98,6 +98,17 @@ class HistoryDesc(C.Structure):
     _fields_ = [("capacity", i32), ("return_sum", vp), ("loss", vp), ("action_counts", vp), ("partner_hits", vp)]
 
 
+class PbtDesc(C.Structure):
+    """Mirror of ``ia2c_pbt_desc``: one population-based-training generation of a batch (ia2c_pbt_step)."""
+    _fields_ = [("window", i32), ("slot", i32), ("q", i32), ("perturb", u32), ("factor_lo", f64), ("factor_hi", f64),
+                ("seed", u64), ("generation", u32), ("reserved", i32),
+                ("lr_actor", vp), ("lr_critic", vp), ("gamma", vp), ("beta", vp),
+                ("log_fitness", vp), ("log_rank", vp), ("log_donor", vp), ("log_lr_actor", vp), ("log_lr_critic", vp),
+                ("log_gamma", vp), ("log_beta", vp), ("workspace", vp), ("workspace_bytes", C.c_size_t)]
+
+
+PBT_LR_ACTOR, PBT_LR_CRITIC, PBT_BETA = 1, 2, 4   # IA2C_PBT_* bits of PbtDesc.perturb
+
 _DP = C.POINTER(EpisodeDesc)
 
 # name -> (restype, argtypes); every symbol declared in include/ia2c_b200.h
@@ -155,6 +166,8 @@ SIGNATURES = {
     "ia2c_eval_policy_floats": (C.c_size_t, [C.POINTER(EvalDesc)]),
     "ia2c_evaluate": (C.c_int, [C.POINTER(EvalDesc), vp]),
     "ia2c_record_episode": (C.c_int, [_DP, i32, C.POINTER(HistoryDesc), i32, vp]),
+    "ia2c_pbt_workspace_bytes": (C.c_size_t, [i32]),
+    "ia2c_pbt_step": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(HistoryDesc), C.POINTER(PbtDesc), vp]),
 }
 
 _lib = None

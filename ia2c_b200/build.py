@@ -17,7 +17,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 BUILD = os.path.join(PKG, "build")
 LIB = os.path.join(PKG, "libia2c_b200.so")
-SOURCES = ["runtime.cu", "org_env.cu", "belief.cu", "mlp.cu", "loss.cu", "trainer.cu", "rollout_fused.cu", "actor_pipe.cu", "debug.cu", "net_update.cu", "a2c.cu", "evaluate.cu", "history.cu"]
+SOURCES = ["runtime.cu", "org_env.cu", "belief.cu", "mlp.cu", "loss.cu", "trainer.cu", "rollout_fused.cu", "actor_pipe.cu", "debug.cu", "net_update.cu", "a2c.cu", "evaluate.cu", "history.cu", "pbt.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
          "--expt-relaxed-constexpr"]

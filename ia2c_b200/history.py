@@ -22,71 +22,101 @@ import torch
 from . import _lib
 
 
-class EpisodeHistory:
-    """The device ring of one trainer or batch (runs R, N agents, E envs per run, T steps) and the drained host rows.
+class DeviceRing:
+    """``capacity`` slots of fixed-size device rows, one array per field, carved in order from one zeroed device buffer, so
+    that a drain is one copy of the byte span that holds the slots to read (the whole buffer when the range wraps).
+    ``fields``: (name, numpy dtype, row shape) per array, field k at ``ptr[name]`` as ``dtype[capacity, *shape]``;
+    ``tags``: names of host-side integers kept per slot (the episode number of a record, ...).
 
-    The four ring arrays of ``ia2c_history_desc`` are carved, in order, from one zeroed device buffer, so that a drain is one
-    copy of the byte span that holds the slots to read (the whole buffer when the range wraps)."""
+    A writer takes ``free_slot()``, enqueues its launch on that slot and then ``commit(**tags)``.  At most ``capacity - 1``
+    records wait undrained (a history record clears the slot after its own): ``free_slot`` drains, which synchronises the
+    device's current stream, when that many are pending."""
 
-    def __init__(self, lib, device, runs, N, E, T, capacity):
+    def __init__(self, device, capacity, fields, tags):
         cap = int(capacity)
         if cap < 2:
-            raise ValueError(f"HISTORY_CAPACITY={capacity} must be >= 2")
-        self.lib, self.device, self.capacity = lib, device, cap
-        self.R, self.N, self.E, self.T = int(runs), int(N), int(E), int(T)
-        RN = self.R * self.N
-        # bytes per slot of return_sum f64[R], loss f32[2, RN], action_counts u32[RN, 3], partner_hits u32[RN]
-        self._row = (self.R * 8, 2 * RN * 4, 3 * RN * 4, RN * 4)
+            raise ValueError(f"capacity={capacity} must be >= 2")
+        self.device, self.capacity = device, cap
+        self._fields = tuple((name, np.dtype(dt), tuple(shape)) for name, dt, shape in fields)
+        self._row = tuple(int(np.prod(shape, dtype=np.int64)) * dt.itemsize for _, dt, shape in self._fields)   # bytes per slot
         self._off = tuple(int(x) for x in np.concatenate([[0], np.cumsum([cap * b for b in self._row])]))
         self._dev = torch.zeros(self._off[-1], dtype=torch.uint8, device=device)
         self._host = torch.empty(self._off[-1], dtype=torch.uint8).pin_memory()
         base = self._dev.data_ptr()
-        h = self.desc = _lib.HistoryDesc()
-        h.capacity = cap
-        h.return_sum, h.loss, h.action_counts, h.partner_hits = (base + o for o in self._off[:4])
-        self._href = C.byref(h)
+        self.ptr = {name: base + o for (name, _, _), o in zip(self._fields, self._off)}
+        self.row_bytes = {name: b for (name, _, _), b in zip(self._fields, self._row)}
+        self._tags = tuple(tags)
+        self._tag_of_slot = np.zeros((len(self._tags), cap), dtype=np.int64)
         self.head = self.tail = 0                       # records enqueued / drained since the ring was made
-        self._episode_of_slot = np.zeros(cap, dtype=np.int64)
         self._chunks = []
 
-    def record(self, desc_ref, episode, stream):
-        """Enqueue the record of the episode ``desc_ref`` just ran (``episode`` is its number) on ``stream``."""
-        if self.head - self.tail >= self.capacity - 1:   # the call clears the next slot: it must have been read
+    def free_slot(self):
+        """The slot of the next record (draining first if capacity - 1 records are pending)."""
+        if self.head - self.tail >= self.capacity - 1:
             self.drain()
+        return self.head % self.capacity
+
+    def commit(self, **tags):
+        """Count the record just enqueued on ``free_slot()`` and keep its tags."""
         slot = self.head % self.capacity
-        _lib.check(self.lib.ia2c_record_episode(desc_ref, self.R, self._href, slot, stream), "ia2c_record_episode")
-        self._episode_of_slot[slot] = episode
+        for i, k in enumerate(self._tags):
+            self._tag_of_slot[i, slot] = tags[k]
         self.head += 1
 
     def drain(self):
-        """Synchronise the device's current stream and move the recorded slots to host arrays."""
+        """Synchronise the device's current stream and move the pending slots to host arrays."""
         n = self.head - self.tail
         if n == 0:
             return
         cap, first = self.capacity, self.tail % self.capacity
         lo, hi = 0, self._off[-1]
-        if first + n <= cap:   # one contiguous run of slots: from its return_sum row to its partner_hits row
-            lo, hi = self._off[0] + first * self._row[0], self._off[3] + (first + n) * self._row[3]
+        if first + n <= cap:   # one contiguous run of slots: from its row of the first field to its row of the last one
+            lo, hi = self._off[0] + first * self._row[0], self._off[-2] + (first + n) * self._row[-1]
         with torch.cuda.device(self.device):
             self._host[lo:hi].copy_(self._dev[lo:hi], non_blocking=True)
             torch.cuda.current_stream(self.device).synchronize()
         slots = (first + np.arange(n)) % cap
         buf = self._host.numpy()
-        R, RN = self.R, self.R * self.N
-
-        def rows(k, dtype, shape):
-            return buf[self._off[k]:self._off[k + 1]].view(dtype).reshape(cap, *shape)[slots]
-
-        self._chunks.append(dict(episode=self._episode_of_slot[slots], return_sum=rows(0, np.float64, (R,)),
-                                 loss=rows(1, np.float32, (2, RN)), action_counts=rows(2, np.uint32, (RN, 3)),
-                                 partner_hits=rows(3, np.uint32, (RN,))))
+        chunk = {k: self._tag_of_slot[i, slots] for i, k in enumerate(self._tags)}
+        for (name, dt, shape), o0, o1 in zip(self._fields, self._off[:-1], self._off[1:]):
+            chunk[name] = buf[o0:o1].view(dt).reshape(cap, *shape)[slots]
+        self._chunks.append(chunk)
         self.tail = self.head
+
+    def take_chunks(self):
+        """Drain, then return and forget every chunk drained so far (a list of dicts of tag and field arrays)."""
+        self.drain()
+        chunks, self._chunks = self._chunks, []
+        return chunks
+
+
+class EpisodeHistory(DeviceRing):
+    """The device ring of one trainer or batch (runs R, N agents, E envs per run, T steps): the four arrays of
+    ``ia2c_history_desc``, and the drained host rows."""
+
+    def __init__(self, lib, device, runs, N, E, T, capacity):
+        if int(capacity) < 2:
+            raise ValueError(f"HISTORY_CAPACITY={capacity} must be >= 2")
+        R, RN = int(runs), int(runs) * int(N)
+        super().__init__(device, capacity, (("return_sum", np.float64, (R,)), ("loss", np.float32, (2, RN)),
+                                            ("action_counts", np.uint32, (RN, 3)), ("partner_hits", np.uint32, (RN,))),
+                         ("episode",))
+        self.lib, self.R, self.N, self.E, self.T = lib, R, int(N), int(E), int(T)
+        h = self.desc = _lib.HistoryDesc()
+        h.capacity = self.capacity
+        h.return_sum, h.loss, h.action_counts, h.partner_hits = (self.ptr[k] for k in
+                                                                 ("return_sum", "loss", "action_counts", "partner_hits"))
+        self._href = C.byref(h)
+
+    def record(self, desc_ref, episode, stream):
+        """Enqueue the record of the episode ``desc_ref`` just ran (``episode`` is its number) on ``stream``."""
+        slot = self.free_slot()
+        _lib.check(self.lib.ia2c_record_episode(desc_ref, self.R, self._href, slot, stream), "ia2c_record_episode")
+        self.commit(episode=episode)
 
     def take(self):
         """Drain, then return and forget every row drained so far (see ``history_arrays``)."""
-        self.drain()
-        chunks, self._chunks = self._chunks, []
-        return history_arrays(chunks, self.R, self.N, self.E, self.T)
+        return history_arrays(self.take_chunks(), self.R, self.N, self.E, self.T)
 
 
 def history_arrays(chunks, R, N, E, T):

@@ -10,6 +10,10 @@ its run r is byte-identical to that trainer with ``actor_kernel="columns"``.
 The device buffers hold the runs stacked (DESIGN.md §3): per-net buffers have R*N rows, run r at rows [r*N, (r+1)*N);
 per-env buffers have an env axis of length R*E, run r at [r*E, (r+1)*E).  ``run_view(r)`` returns those slices and
 ``run_state_dict(r)`` a checkpoint that a standalone ``IA2CTrainer`` loads, so the best run of a sweep can go on alone.
+
+``exploit_explore`` runs one generation of population-based training on the device between episodes (``ia2c_pbt_step``):
+the worst runs by recent recorded returns take copies of the best runs' state and perturbed copies of their
+hyper-parameters; ``pbt_history`` reads back what each generation did.
 """
 from __future__ import annotations
 
@@ -20,7 +24,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .history import RecordsHistory
+from .history import DeviceRing, RecordsHistory
 from .trainer import N_ACTIONS, N_FEATURES, IA2CTrainer, reference_init
 
 # buffers with one row per (run, agent), and buffers with an env axis (its position) of length R * E
@@ -28,6 +32,9 @@ _NET = ("actor_params", "critic_params", "actor_grad", "critic_grad", "actor_gra
         "critic_v", "actor_step", "critic_step", "filter_action")
 _ENV = {"env_state": 0, "env_hist": 0, "env_cls": 0, "env_elapsed": 0, "ep_return": 0, "belief_records": 0,
         "obs": 1, "reward": 1, "act": 1, "partner_true": 1, "partner_pred": 1}
+# the per-run hyper-parameters, in ia2c_runs_desc order, with their device dtype
+_HYPER = (("lr_actor", torch.float64), ("lr_critic", torch.float64), ("gamma", torch.float32), ("beta", torch.float32))
+_PERTURB = {"lr_actor": _lib.PBT_LR_ACTOR, "lr_critic": _lib.PBT_LR_CRITIC, "beta": _lib.PBT_BETA}
 
 
 def _per_run(name, value, R, dtype):
@@ -50,6 +57,10 @@ class IA2CRuns(RecordsHistory):
     # the C entry point of one batched episode and the descriptor flags it takes
     _ENTRY = "ia2c_train_episode_runs"
     _FLAGS = _lib.FLAG_FUSED_ROLLOUT | _lib.FLAG_FUSED_CRITIC | _lib.FLAG_ACTOR_COLUMNS
+    PBT_LOG_CAPACITY = 16   # generations the device log holds before it drains (allocated on first use)
+    _pbt_log = None
+    _pbt_generation = 0     # generations run so far: the Philox counter of the next one
+    _pbt_mark = 0           # the history ring's record count at the previous generation
 
     @classmethod
     def _check_shape(cls, lib, N, M):
@@ -103,6 +114,7 @@ class IA2CRuns(RecordsHistory):
         self.belief_records = z((RE, N, K, _lib.BELIEF_RECORD), u8)
         self._seed = torch.from_numpy(np.asarray(seeds, dtype=np.uint64).view(np.int64)).to(dev)
         self._hyper = {k: (torch.from_numpy(a).to(dev) if a is not None else None) for k, (a, _) in hyper.items()}
+        self._built_hyper = {k: a for k, (a, _) in hyper.items()}   # per-run arrays as given, None for a scalar (desc holds it)
 
         d = self.desc = _lib.EpisodeDesc()
         d.E, d.E_total, d.env_offset = E, E, 0
@@ -196,11 +208,16 @@ class IA2CRuns(RecordsHistory):
         sd.update(episode=self.episode, seeds=list(self.seeds), dims=(self.R, self.E, self.N, self.M, self.T),
                   critic_losses=[x.copy() for x in self.critic_losses], actor_losses=[x.copy() for x in self.actor_losses],
                   reward_lst=[x.copy() for x in self.reward_lst])
+        if self._pbt_generation > 0:   # PBT changed the hyper-parameters: they are part of the runs' state now
+            sd.update(hyper={k: self._hyper[k].detach().cpu().clone() for k, _ in _HYPER}, pbt_generation=self._pbt_generation)
         return sd
 
     def load_state_dict(self, sd):
-        """Restores parameters, optimiser, env and belief state, the episode counter, the runs' seeds and the windows; the
-        hyper-parameters stay those this batch was built with (as ``IA2CTrainer.load_state_dict``)."""
+        """Restores parameters, optimiser, env and belief state, the episode counter, the runs' seeds and the windows.  A
+        checkpoint taken after a PBT generation also restores the per-run hyper-parameters and the generation counter; one
+        taken before any generation sets the hyper-parameters back to those this batch was built with (as
+        ``IA2CTrainer.load_state_dict`` keeps them) and the generation counter to 0.  Either way the next ``exploit_explore``
+        counts only episodes recorded after the load."""
         if tuple(sd["dims"]) != (self.R, self.E, self.N, self.M, self.T):
             raise ValueError(f"checkpoint is for (runs, E, N, M, T) = {tuple(sd['dims'])}, batch has {(self.R, self.E, self.N, self.M, self.T)}")
         for k in IA2CTrainer._CKPT_TENSORS:
@@ -210,6 +227,21 @@ class IA2CRuns(RecordsHistory):
         self._seed.copy_(torch.from_numpy(np.asarray(self.seeds, dtype=np.uint64).view(np.int64)))
         self.critic_losses, self.actor_losses = list(sd["critic_losses"]), list(sd["actor_losses"])
         self.reward_lst = list(sd["reward_lst"])
+        if "pbt_generation" in sd:
+            with torch.cuda.device(self.device):
+                self._materialise_hyper()
+            for k, _ in _HYPER:
+                self._hyper[k].copy_(sd["hyper"][k])
+            self._pbt_generation = int(sd["pbt_generation"])
+        elif self._pbt_generation > 0:   # PBT changed this batch's hyper-parameters; the checkpoint predates any generation
+            for k, _ in _HYPER:
+                built = self._built_hyper[k]
+                if built is None:
+                    self._hyper[k].fill_(getattr(self.desc, k))   # the array holds the scalar, as _materialise_hyper fills it
+                else:
+                    self._hyper[k].copy_(torch.from_numpy(built))
+            self._pbt_generation = 0
+        self._pbt_mark = self._history.head if self._history is not None else 0   # the ring's records predate the load
 
     def save(self, path):
         torch.save(self.state_dict(), path)
@@ -230,6 +262,100 @@ class IA2CRuns(RecordsHistory):
 
     def agent_steps_per_episode(self):
         return self.R * self.E * self.N * self.T
+
+    # ------------------------------------------------------------------ population-based training
+    def run_hyper(self, r):
+        """Run r's current lr_actor, lr_critic, gamma and beta as Python floats (synchronises once PBT has changed them):
+        ``IA2CTrainer(envs_per_run, n_agents=N, n_models=M, seed=seeds[r], **run_hyper(r))`` loaded with
+        ``run_state_dict(r)`` continues run r bit-identically."""
+        if not 0 <= r < self.R:
+            raise IndexError(f"run {r} of {self.R}")
+        return {k: float(self._hyper[k][r].item()) if self._hyper[k] is not None else float(getattr(self.desc, k))
+                for k, _ in _HYPER}
+
+    def _materialise_hyper(self):
+        """Give every hyper-parameter a device array (filled from the scalar where the batch was built with one) and point
+        the runs descriptor at it; the kernels compute the same bytes from the array as from the scalar."""
+        for k, dtype in _HYPER:
+            if self._hyper[k] is None:
+                self._hyper[k] = torch.full((self.R,), getattr(self.desc, k), dtype=dtype, device=self.device)
+                setattr(self.runs_desc, k, self._hyper[k].data_ptr())
+
+    def _pbt_args(self, window, fraction, perturb, factors, seed):
+        """exploit_explore's checks, all before any device work -> (window, q, perturb mask, factors, seed)."""
+        window, fraction, seed = int(window), float(fraction), int(seed)
+        cap = self._history.capacity if self._history is not None else self.HISTORY_CAPACITY
+        if not 1 <= window <= cap - 1:
+            raise ValueError(f"window={window} outside [1, HISTORY_CAPACITY - 1 = {cap - 1}]")
+        if not 0.0 <= fraction <= 0.5:
+            raise ValueError(f"fraction={fraction} outside [0, 0.5]: donors and recipients must be disjoint")
+        mask = 0
+        for name in ((perturb,) if isinstance(perturb, str) else perturb):
+            if name == "gamma":
+                raise ValueError("perturb: gamma is inherited from the donor, never perturbed")
+            if name not in _PERTURB:
+                raise ValueError(f"perturb: unknown hyper-parameter {name!r} (lr_actor, lr_critic, beta)")
+            mask |= _PERTURB[name]
+        factors = tuple(float(f) for f in factors)
+        if len(factors) != 2 or not all(math.isfinite(f) and f > 0 for f in factors):
+            raise ValueError(f"factors={factors}: need two finite factors > 0")
+        if not 0 <= seed < 1 << 64:
+            raise ValueError(f"seed={seed} outside [0, 2**64)")
+        if self._history is None:
+            raise ValueError("exploit_explore ranks runs by the returns train_episodes records: this batch has no history ring yet")
+        recorded = self._history.head - self._pbt_mark
+        if recorded < window:
+            raise ValueError(f"window={window}: only {recorded} episodes recorded by train_episodes since the previous generation")
+        return window, int(math.floor(fraction * self.R)), mask, factors, seed
+
+    def exploit_explore(self, window, fraction=0.25, perturb=("lr_actor", "lr_critic", "beta"), factors=(0.8, 1.2), seed=0):
+        """One generation of population-based training, on the device and asynchronous (include/ia2c_b200.h,
+        ia2c_pbt_step, states the definitions).  Run r's fitness is the fp64 sum of its return_sum over the last ``window``
+        episodes recorded by ``train_episodes``, oldest first; runs rank by fitness, higher first, NaN last, ties to the lower
+        index.  Each of the bottom q = floor(fraction * R) runs takes a donor from the top q (Philox stream 5 keyed by
+        ``seed``, counter word 3 the generation): its parameters, Adam moments and steps, actor gradient sum and belief
+        models become a byte copy of the donor's, and it inherits the donor's hyper-parameters, each name in ``perturb``
+        multiplied by factors[0] or factors[1].  A recipient keeps its seed, env state and statistics windows.  Afterwards
+        run r equals ``IA2CTrainer(E, n_agents=N, n_models=M, seed=seeds[r], **run_hyper(r))`` (``actor_kernel="columns"``
+        for N > 8) loaded with ``run_state_dict(r)``.  Two launches; the log (``pbt_history``) drains, synchronising, once
+        every ``PBT_LOG_CAPACITY - 1`` generations that ``pbt_history`` has not read."""
+        window, q, mask, (lo, hi), seed = self._pbt_args(window, fraction, perturb, factors, seed)
+        ring, R = self._history, self.R
+        with torch.cuda.device(self.device):
+            self._materialise_hyper()
+            if self._pbt_log is None:
+                self._pbt_log = DeviceRing(self.device, self.PBT_LOG_CAPACITY, (
+                    ("fitness", np.float64, (R,)), ("rank", np.int32, (R,)), ("donor", np.int32, (R,)),
+                    ("lr_actor", np.float64, (R,)), ("lr_critic", np.float64, (R,)), ("gamma", np.float32, (R,)),
+                    ("beta", np.float32, (R,))), ("generation", "episode"))
+                self._pbt_ws = torch.empty(int(self.lib.ia2c_pbt_workspace_bytes(R)), dtype=torch.uint8, device=self.device)
+            log = self._pbt_log
+            slot = log.free_slot()
+            p = _lib.PbtDesc()
+            p.window, p.slot, p.q, p.perturb = window, (ring.head - 1) % ring.capacity, q, mask
+            p.factor_lo, p.factor_hi, p.seed, p.generation = lo, hi, seed, self._pbt_generation
+            for k, _ in _HYPER:
+                setattr(p, k, self._hyper[k].data_ptr())
+            for k in ("fitness", "rank", "donor", "lr_actor", "lr_critic", "gamma", "beta"):
+                setattr(p, "log_" + k, log.ptr[k] + slot * log.row_bytes[k])
+            p.workspace, p.workspace_bytes = self._pbt_ws.data_ptr(), self._pbt_ws.numel()
+            _lib.check(self.lib.ia2c_pbt_step(C.byref(self.desc), C.byref(self.runs_desc), ring._href, C.byref(p),
+                                              torch.cuda.current_stream(self.device).cuda_stream), "ia2c_pbt_step")
+        log.commit(generation=self._pbt_generation, episode=self.episode)
+        self._pbt_generation += 1
+        self._pbt_mark = ring.head
+
+    def pbt_history(self):
+        """Synchronise and return every PBT generation since the previous call, generation axis first: ``generation`` and
+        ``episode`` (the episode counter at the call) [g]; ``fitness`` f64, ``rank`` i32 and ``donor`` i32 (-1: the run kept
+        its own state) [g, R]; ``lr_actor``, ``lr_critic`` (f64), ``beta`` and ``gamma`` (f32) [g, R] after the step.  The log
+        is not part of a checkpoint: call this before ``save``."""
+        chunks = self._pbt_log.take_chunks() if self._pbt_log is not None else []
+        shapes = dict(generation=(np.int64, ()), episode=(np.int64, ()), fitness=(np.float64, (self.R,)),
+                      rank=(np.int32, (self.R,)), donor=(np.int32, (self.R,)), lr_actor=(np.float64, (self.R,)),
+                      lr_critic=(np.float64, (self.R,)), beta=(np.float32, (self.R,)), gamma=(np.float32, (self.R,)))
+        return {k: (np.concatenate([c[k] for c in chunks]) if chunks else np.zeros((0,) + shape, dtype=dt))
+                for k, (dt, shape) in shapes.items()}
 
 
 class IA2CRunsMany(IA2CRuns):

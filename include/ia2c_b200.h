@@ -556,6 +556,79 @@ typedef struct ia2c_history_desc {
 } ia2c_history_desc;
 int ia2c_record_episode(const ia2c_episode_desc* d, int32_t runs, const ia2c_history_desc* h, int32_t slot, void* stream);
 
+/* ------------------------------------------------------------------ population-based training of a batch of runs -- */
+/* One generation of population-based training (PBT) on a batch of R runs (ia2c_runs_desc layout, `d` the batch's episode
+ * descriptor, `h` its history ring as ia2c_record_episode fills it), entirely on the device: rank the runs by their recent
+ * training returns, overwrite the worst q with copies of runs drawn from the best q, and perturb the copies'
+ * hyper-parameters.  Called between episodes; nothing is read back to the host.
+ *
+ * Definitions (R runs of N agents, w = p->window, s = p->slot the ring slot of the newest record, C = h->capacity):
+ *   fitness[r]  = the fp64 sum of return_sum[(s - w + 1 + k) mod C, r] for k = 0 .. w - 1, oldest first, added in that
+ *                 order from +0.0 with one IEEE fp64 add each (round to nearest).  The same bytes from run to run.
+ *   order       the runs sorted by fitness, higher first; a NaN fitness ranks below every non-NaN one; ties (equal
+ *                 fitness, both NaN included; -0.0 == +0.0) go to the lower run index.  A total order: rank[r] is r's
+ *                 position in it, order[rank[r]] = r.
+ *   recipients  the bottom q runs, order[R - q + j] for j = 0 .. q - 1; donors are drawn from the top q, order[0 .. q-1].
+ *                 2q <= R, so the two sets are disjoint.
+ *   donor       recipient v draws ONE Philox block, stream 5: key = p->seed, counter = (v, 0, 0 | 5 << 16,
+ *                 p->generation) (the layout of the other streams: index v, t = 0, episode = generation) -> words
+ *                 (x, y, z, w); donor = order[((x >> 8) * q) >> 24], in unsigned 64-bit integer arithmetic.
+ *   copy        every byte of the recipient's rows [v*N, (v+1)*N) of actor_params, critic_params, actor_m, actor_v,
+ *                 critic_m, critic_v, actor_step, critic_step, actor_grad_accum and filter_action becomes the byte of the
+ *                 donor's rows as it was before the call.  Nothing else of `d` is written: not the env state, trajectory,
+ *                 ep_return, belief_records, loss_out, actor_grad or critic_grad, and no row of a run that is not a
+ *                 recipient.  The recipient keeps its seed.
+ *   explore     the recipient takes the donor's lr_actor, lr_critic, gamma and beta; then, for each set bit of
+ *                 p->perturb, f = p->factor_hi if the top bit of the word is set, else p->factor_lo, and
+ *                   lr_actor  = __dmul_rn(lr_actor, f)                       (bit 0, IA2C_PBT_LR_ACTOR, word y)
+ *                   lr_critic = __dmul_rn(lr_critic, f)                      (bit 1, IA2C_PBT_LR_CRITIC, word z)
+ *                   beta      = __double2float_rn(__dmul_rn((double)beta, f)) (bit 2, IA2C_PBT_BETA, word w)
+ *                 gamma is inherited, never perturbed.  Other runs' hyper-parameters are unchanged.
+ * The hyper-parameters live in the four device arrays of `p` (read and written), which must be the arrays the batch's
+ * ia2c_runs_desc points at for its next episode to train with them.
+ *
+ * Log (device, written for every run r): log_fitness[r], log_rank[r], log_donor[r] (-1: not a recipient) and the four
+ * hyper-parameters of run r after the step.  workspace: ia2c_pbt_workspace_bytes(R) bytes, int32 order[R].
+ *
+ * Two launches, both with programmatic dependent launch (ring rows, parameters and hyper-parameters are read after the wait
+ * through L2): pbt_rank_kernel (ceil(R / 256) blocks of 256 threads, one thread per run, O(R^2) compares over fitness tiles
+ * staged in shared memory) and pbt_apply_kernel (q x ceil(N / agents per block) blocks: the draw, the log row and the
+ * hyper-parameters of recipient j in block (j, 0), the row copies in 16-byte words where donor and recipient rows share
+ * their 16-byte alignment, else 4-byte words).  q = 0 launches both kernels, logs, and changes no training byte.
+ * Every check runs before the first CUDA call: a NULL descriptor or pointer (the ten buffers above, h->return_sum, the
+ * four hyper-parameter arrays, the seven log arrays, the workspace), R < 1, N < 1, R * N above IA2C_MAX_RUN_NETS, capacity
+ * < 2, window outside [1, capacity - 1], a slot outside [0, capacity), q < 0 or 2q > R, perturb bits other than the three
+ * above, a factor that is not finite and > 0, a workspace smaller than ia2c_pbt_workspace_bytes(R) (IA2C_ERR_INVALID);
+ * env_offset != 0 or E_total != E (a multi-GPU shard; IA2C_ERR_UNSUPPORTED). */
+#define IA2C_PBT_LR_ACTOR 1
+#define IA2C_PBT_LR_CRITIC 2
+#define IA2C_PBT_BETA 4
+typedef struct ia2c_pbt_desc {
+    int32_t window;                   /* episodes summed into the fitness, 1 <= window <= capacity - 1 */
+    int32_t slot;                     /* ring slot of the newest record */
+    int32_t q;                        /* recipients (and donor candidates), 0 <= 2q <= R */
+    uint32_t perturb;                 /* IA2C_PBT_* bits */
+    double factor_lo, factor_hi;      /* multipliers for a clear / set top bit, finite and > 0 */
+    uint64_t seed;                    /* Philox key (stream 5) */
+    uint32_t generation;              /* Philox counter word 3 */
+    int32_t reserved;
+    double* lr_actor;                 /* in/out device double[R] */
+    double* lr_critic;                /* in/out device double[R] */
+    float* gamma;                     /* in/out device float[R] */
+    float* beta;                      /* in/out device float[R] */
+    double* log_fitness;              /* out f64[R] */
+    int32_t* log_rank;                /* out i32[R] */
+    int32_t* log_donor;               /* out i32[R], -1 for a run that kept its own state */
+    double* log_lr_actor;             /* out f64[R], after the step */
+    double* log_lr_critic;            /* out f64[R] */
+    float* log_gamma;                 /* out f32[R] */
+    float* log_beta;                  /* out f32[R] */
+    void* workspace; size_t workspace_bytes;
+} ia2c_pbt_desc;
+size_t ia2c_pbt_workspace_bytes(int32_t runs);
+int ia2c_pbt_step(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_history_desc* h, const ia2c_pbt_desc* p,
+                  void* stream);
+
 #ifdef __cplusplus
 }
 #endif
