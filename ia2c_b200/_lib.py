@@ -32,6 +32,7 @@ A2C_MAX_STEPS = 65534         # IA2C_A2C_MAX_STEPS
 EVAL_MAX_RUNS = 65535         # IA2C_EVAL_MAX_RUNS
 EVAL_MAX_AGENTS = 1023        # IA2C_EVAL_MAX_AGENTS
 EVAL_MAX_STEPS = 65535        # IA2C_EVAL_MAX_STEPS
+EVAL_MAX_LINEUPS = 1 << 20    # IA2C_EVAL_MAX_LINEUPS
 
 
 class EpisodeDesc(C.Structure):
@@ -90,6 +91,17 @@ class EvalDesc(C.Structure):
         ("episodes", i32), ("T", i32), ("max_episode_steps", i32), ("greedy", i32),
         ("seed", u64), ("episode0", u32), ("inj_u_action", vp),
         ("policy", vp), ("policy_floats", C.c_size_t), ("returns", vp), ("action_counts", vp),
+    ]
+
+
+class LineupDesc(C.Structure):
+    """Mirror of ``ia2c_lineup_desc``: a cross-play evaluation of P lineups seated from a pool of actors (ia2c_evaluate_lineups)."""
+    _fields_ = [
+        ("actor_params", vp), ("nets", i32), ("N", i32), ("P", i32), ("reserved", i32), ("lineups", vp), ("E", i64),
+        ("episodes", i32), ("T", i32), ("max_episode_steps", i32), ("greedy", i32),
+        ("seed", u64), ("episode0", u32), ("inj_u_action", vp),
+        ("policy", vp), ("policy_floats", C.c_size_t), ("returns", vp), ("action_counts", vp),
+        ("return_sum", vp), ("return_m2", vp),
     ]
 
 
@@ -165,6 +177,7 @@ SIGNATURES = {
     "ia2c_a2c_train_update": (C.c_int, [C.POINTER(A2CDesc), vp]),
     "ia2c_eval_policy_floats": (C.c_size_t, [C.POINTER(EvalDesc)]),
     "ia2c_evaluate": (C.c_int, [C.POINTER(EvalDesc), vp]),
+    "ia2c_evaluate_lineups": (C.c_int, [C.POINTER(LineupDesc), vp]),
     "ia2c_record_episode": (C.c_int, [_DP, i32, C.POINTER(HistoryDesc), i32, vp]),
     "ia2c_pbt_workspace_bytes": (C.c_size_t, [i32]),
     "ia2c_pbt_step": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(HistoryDesc), C.POINTER(PbtDesc), vp]),

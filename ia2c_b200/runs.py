@@ -260,6 +260,14 @@ class IA2CRuns(RecordsHistory):
         return evaluate_actors(self.actor_params, self.R, self.N, E, episodes, self.T, self.desc.max_episode_steps, greedy,
                                seed, first_episode, self.device)
 
+    def cross_play(self, episodes=1, num_envs=None, greedy=False, seed=0, first_episode=0, split=None):
+        """``evaluate.cross_play(self, ...)``: the R x R matrix of this batch's runs played against each other (cell (a, b)
+        seats agents 0 .. split-1 of run a and the rest of run b); the diagonal is each run's ``evaluate``."""
+        from .evaluate import cross_play
+
+        return cross_play(self, episodes=episodes, num_envs=num_envs, greedy=greedy, seed=seed, first_episode=first_episode,
+                          split=split)
+
     def agent_steps_per_episode(self):
         return self.R * self.E * self.N * self.T
 

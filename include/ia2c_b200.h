@@ -522,6 +522,65 @@ typedef struct ia2c_eval_desc {
 size_t ia2c_eval_policy_floats(const ia2c_eval_desc* d);
 int ia2c_evaluate(const ia2c_eval_desc* d, void* stream);
 
+/* ------------------------------------------------------------------ cross-play: lineups of actors from a pool -- */
+/* Evaluates P lineups whose seats are filled from a pool of actors (the rows of one batch, or of several sources
+ * concatenated), so that separately trained runs can be played against each other: the cross-play matrix of a sweep.
+ *
+ * Definitions: the pool is actor_params f32[nets, 105]; lineup p seats pool row lineups[p * N + i] in seat i (rows may
+ * repeat within a lineup, and a row may sit in a seat other than the one it was trained in).  Lineup p plays `episodes`
+ * (K) episodes of T steps in each of E envs exactly as ia2c_evaluate plays one run: same reset state, same-step autoreset at
+ * max_episode_steps, fp64 step-order return, Philox stream 4 with the same counters (e = the env within the lineup), or
+ * the argmax with greedy != 0 (E = K = 1).
+ * Contract: lineup p computes, byte for byte, the returns and action counts that an R = 1 ia2c_evaluate call computes when
+ * its actor rows are pool[lineups[p, 0..N-1]], with the same seed, episode0, E, K, T, max_episode_steps and greedy.  So the
+ * lineup of run r's own agents reproduces run r's evaluation, and all lineups see the same random numbers: the cells of a
+ * cross-play matrix are paired samples.
+ *
+ * Layout:
+ *   lineups       i32[P, N], pool rows;
+ *   policy        out and workspace f32[nets, 9, 3]: the pool's table, as ia2c_evaluate tabulates it (>= nets * 27 floats);
+ *   returns       out f64[P, episodes, E];
+ *   action_counts out u64[P * N, 3], overwritten: per lineup and seat;
+ *   return_sum    out f64[P]: lineup p's n = K * E returns, items x[j] = returns[p] in row-major order, summed in a fixed order:
+ *                 lane j of 256 adds x[j], x[j + 256], x[j + 512], ... in increasing order from +0.0, then a halving tree
+ *                 combines the lanes (s[j] += s[j + w] for j < w, w = 128, 64, ..., 1) and the sum is s[0] (the order of
+ *                 ia2c_record_episode's return_sum); every addition is one IEEE fp64 add, round to nearest;
+ *   return_m2     out f64[P]: with mean = return_sum / n (one IEEE divide), the sum of (x[j] - mean)^2 (one subtract and one
+ *                 multiply each, never fused) in the same order.  Both are the same bytes from run to run;
+ *   inj_u_action  f32[episodes, T, P*E, N] or NULL: the uniforms instead of Philox (the evaluation tape with P in place of R).
+ * Guarded entries: lineups live on the device and are not checked before the launches.  A lineup with an entry outside
+ * [0, nets) reads nothing of the table; its returns, return_sum and return_m2 are NaN and its counts 0.  Other lineups are
+ * unaffected.
+ *
+ * Three launches, all with programmatic dependent launch (table, lineups and returns read after the wait through L2):
+ *   lineup_policy_kernel           the pool's table (ia2c_evaluate's per-row forward and softmax), and action_counts zeroed;
+ *   lineup_episodes_kernel<WIDE>   ia2c_evaluate's episode kernel with the block's table gathered from the lineup's pool rows;
+ *                                  grid (item blocks, y, z) with lineup p = blockIdx.z * gridDim.y + blockIdx.y, so that P
+ *                                  may exceed 65535;
+ *   lineup_stats_kernel            one warp per lineup: return_sum and return_m2.
+ * Nothing outside policy, returns, action_counts, return_sum and return_m2 is written.
+ * Every check runs before the first CUDA call: a NULL descriptor or pointer, N outside 2..1023, nets < 1, P outside
+ * 1..IA2C_EVAL_MAX_LINEUPS, E, episodes, T, max_episode_steps, episode0 and greedy as ia2c_evaluate checks them, and a
+ * policy workspace smaller than nets * 27 floats. */
+#define IA2C_EVAL_MAX_LINEUPS 1048576   /* P: the full matrix of 1024 runs */
+typedef struct ia2c_lineup_desc {
+    const float* actor_params;       /* f32[nets, 105]: the pool */
+    int32_t nets, N;                 /* pool rows >= 1; seats 2 <= N <= 1023 */
+    int32_t P, reserved;             /* lineups, 1 <= P <= IA2C_EVAL_MAX_LINEUPS */
+    const int32_t* lineups;          /* i32[P, N] */
+    int64_t E;                       /* envs per lineup */
+    int32_t episodes, T, max_episode_steps, greedy;
+    uint64_t seed;                   /* Philox key (stream 4) */
+    uint32_t episode0;               /* Philox episode of item k is episode0 + k; episode0 + episodes <= 2^32 */
+    const float* inj_u_action;       /* f32[episodes, T, P*E, N] or NULL */
+    float* policy; size_t policy_floats;   /* out and workspace: f32[nets, 9, 3] */
+    double* returns;                 /* out: f64[P, episodes, E] */
+    unsigned long long* action_counts;     /* out: u64[P*N, 3] */
+    double* return_sum;              /* out: f64[P] */
+    double* return_m2;               /* out: f64[P] */
+} ia2c_lineup_desc;
+int ia2c_evaluate_lineups(const ia2c_lineup_desc* d, void* stream);
+
 /* ------------------------------------------------------------------ learning curves: per-episode statistics on the device -- */
 /* Reduces the trajectory an episode just left into slot `slot` of a caller-owned ring, in ONE launch, so that learning curves
  * are read back in bulk instead of with a stream synchronisation per episode.  `d` is the descriptor the episode ran with: a
