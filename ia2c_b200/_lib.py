@@ -33,6 +33,7 @@ EVAL_MAX_RUNS = 65535         # IA2C_EVAL_MAX_RUNS
 EVAL_MAX_AGENTS = 1023        # IA2C_EVAL_MAX_AGENTS
 EVAL_MAX_STEPS = 65535        # IA2C_EVAL_MAX_STEPS
 EVAL_MAX_LINEUPS = 1 << 20    # IA2C_EVAL_MAX_LINEUPS
+PARTNER_MAX_TEAMS = 1 << 20   # IA2C_PARTNER_MAX_TEAMS
 
 
 class EpisodeDesc(C.Structure):
@@ -121,6 +122,12 @@ class PbtDesc(C.Structure):
 
 PBT_LR_ACTOR, PBT_LR_CRITIC, PBT_BETA = 1, 2, 4   # IA2C_PBT_* bits of PbtDesc.perturb
 
+
+class PartnerDesc(C.Structure):
+    """Mirror of ``ia2c_partner_desc``: a pool of frozen partners seated before an episode (ia2c_seat_partners)."""
+    _fields_ = [("rows", vp), ("P", i32), ("seats", vp), ("S", i32), ("teams", vp), ("Q", i32), ("episode", u32),
+                ("log_team", vp)]
+
 _DP = C.POINTER(EpisodeDesc)
 
 # name -> (restype, argtypes); every symbol declared in include/ia2c_b200.h
@@ -181,6 +188,7 @@ SIGNATURES = {
     "ia2c_record_episode": (C.c_int, [_DP, i32, C.POINTER(HistoryDesc), i32, vp]),
     "ia2c_pbt_workspace_bytes": (C.c_size_t, [i32]),
     "ia2c_pbt_step": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(HistoryDesc), C.POINTER(PbtDesc), vp]),
+    "ia2c_seat_partners": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(PartnerDesc), vp]),
 }
 
 _lib = None

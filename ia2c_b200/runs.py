@@ -14,6 +14,10 @@ per-env buffers have an env axis of length R*E, run r at [r*E, (r+1)*E).  ``run_
 ``exploit_explore`` runs one generation of population-based training on the device between episodes (``ia2c_pbt_step``):
 the worst runs by recent recorded returns take copies of the best runs' state and perturbed copies of their
 hyper-parameters; ``pbt_history`` reads back what each generation did.
+
+``set_partners`` (ia2c_b200/partners.py) seats frozen partners from a pool in every run's partner seats before each episode
+(``ia2c_seat_partners``): each run draws a team from its own training seed, so run r still equals a standalone trainer with
+the same seed and pool.
 """
 from __future__ import annotations
 
@@ -25,6 +29,7 @@ import torch
 
 from . import _lib
 from .history import DeviceRing, RecordsHistory
+from .partners import SeatsPartners
 from .trainer import N_ACTIONS, N_FEATURES, IA2CTrainer, reference_init
 
 # buffers with one row per (run, agent), and buffers with an env axis (its position) of length R * E
@@ -53,7 +58,7 @@ def _per_run(name, value, R, dtype):
     return arr.astype(dtype), float(arr[0])
 
 
-class IA2CRuns(RecordsHistory):
+class IA2CRuns(SeatsPartners, RecordsHistory):
     # the C entry point of one batched episode and the descriptor flags it takes
     _ENTRY = "ia2c_train_episode_runs"
     _FLAGS = _lib.FLAG_FUSED_ROLLOUT | _lib.FLAG_FUSED_CRITIC | _lib.FLAG_ACTOR_COLUMNS
@@ -149,9 +154,9 @@ class IA2CRuns(RecordsHistory):
         ``read_stats`` windows."""
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):
-            _lib.check(getattr(self.lib, self._ENTRY)(C.byref(self.desc), C.byref(self.runs_desc),
-                                                      torch.cuda.current_stream(self.device).cuda_stream),
-                       self._ENTRY)
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            self._seat_partners(stream)
+            _lib.check(getattr(self.lib, self._ENTRY)(C.byref(self.desc), C.byref(self.runs_desc), stream), self._ENTRY)
         self.episode += 1
         if sync_stats:
             return self.read_stats()
@@ -159,7 +164,11 @@ class IA2CRuns(RecordsHistory):
     def _history_dims(self):
         return self.R, self.N, self.E, self.T, False
 
+    def _partner_runs(self):
+        return self.R, C.byref(self.runs_desc)
+
     def _enqueue_episode(self, desc_ref, stream):
+        self._seat_partners(stream)
         _lib.check(getattr(self.lib, self._ENTRY)(desc_ref, C.byref(self.runs_desc), stream), self._ENTRY)
 
     def read_stats(self):
@@ -199,7 +208,7 @@ class IA2CRuns(RecordsHistory):
         sd.update(episode=self.episode, seed=self.seeds[r], dims=(self.E, self.E, self.N, self.M, self.T), rank=0, world=1,
                   critic_losses=[x[r].copy() for x in self.critic_losses], actor_losses=[x[r].copy() for x in self.actor_losses],
                   reward_lst=[x[r].copy() for x in self.reward_lst])
-        return sd
+        return self._partner_state(sd)
 
     # ------------------------------------------------------------------ checkpoint / resume of the whole batch
     def state_dict(self):
@@ -210,7 +219,7 @@ class IA2CRuns(RecordsHistory):
                   reward_lst=[x.copy() for x in self.reward_lst])
         if self._pbt_generation > 0:   # PBT changed the hyper-parameters: they are part of the runs' state now
             sd.update(hyper={k: self._hyper[k].detach().cpu().clone() for k, _ in _HYPER}, pbt_generation=self._pbt_generation)
-        return sd
+        return self._partner_state(sd)
 
     def load_state_dict(self, sd):
         """Restores parameters, optimiser, env and belief state, the episode counter, the runs' seeds and the windows.  A
@@ -242,6 +251,7 @@ class IA2CRuns(RecordsHistory):
                     self._hyper[k].copy_(torch.from_numpy(built))
             self._pbt_generation = 0
         self._pbt_mark = self._history.head if self._history is not None else 0   # the ring's records predate the load
+        self._load_partner_state(sd)   # the checkpoint's pool, or none
 
     def save(self, path):
         torch.save(self.state_dict(), path)

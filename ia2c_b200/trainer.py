@@ -20,6 +20,7 @@ import torch.nn as nn
 from . import _lib
 from .history import RecordsHistory
 from .nets import hidden_size
+from .partners import SeatsPartners
 from .sharding import shard_envs
 
 N_FEATURES, N_ACTIONS, N_JOINT = 6, 3, 9
@@ -47,7 +48,7 @@ def reference_init(n_agents, n_models, seed=None):
     return actor, critic, np.stack(fa)
 
 
-class IA2CTrainer(RecordsHistory):
+class IA2CTrainer(SeatsPartners, RecordsHistory):
     def __init__(self, num_envs, n_agents=2, n_models=5, steps_per_episode=30, max_episode_steps=30,
                  lr_critic=0.0002, lr_actor=0.0001, beta=0.001, gamma=0.9, seed=0, device=None,
                  rank=0, world_size=1, process_group=None, dumps=False, fused_rollout=None, fused_critic=None,
@@ -236,6 +237,7 @@ class IA2CTrainer(RecordsHistory):
     def rollout(self):
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):
+            self._seat_partners(self._stream())
             _lib.check(self.lib.ia2c_rollout(C.byref(self.desc), self._stream()), "ia2c_rollout")
 
     def update(self):
@@ -271,6 +273,7 @@ class IA2CTrainer(RecordsHistory):
         if self.world == 1:   # one C call for the whole episode
             self.desc.episode = self.episode
             with torch.cuda.device(self.device):
+                self._seat_partners(self._stream())
                 _lib.check(self.lib.ia2c_train_episode(C.byref(self.desc), self._stream()), "ia2c_train_episode")
         elif self.p2p:        # one C call per rank: the gradient exchanges are kernels of the same stream
             self.desc.episode = self.episode
@@ -294,13 +297,23 @@ class IA2CTrainer(RecordsHistory):
         return 1, self.N, self.E, self.T, True
 
     def _enqueue_episode(self, desc_ref, stream):
+        self._seat_partners(stream)
         _lib.check(self.lib.ia2c_train_episode(desc_ref, stream), "ia2c_train_episode")
+
+    # ---- frozen partners (ia2c_b200/partners.py: set_partners, partner_history) -------------------------------------
+    def _check_partners(self):
+        if self.world > 1:
+            raise _lib.IA2CError("set_partners seats partners on one GPU (a rank sees only its env shard)")
+
+    def _partner_runs(self):
+        return 1, None
 
     def train_episode_host(self, host_u_action, host_u_belief):
         """End-to-end form with HOST inputs/outputs: pinned uniforms in, losses + episode returns out;
         the copies and a stream sync are inside the call (single rank)."""
         if self.world > 1:
             raise _lib.IA2CError("train_episode_host is the single-rank entry point")
+        self._refuse_partners("train_episode_host")
         if self.inj_u_action is None or self.inj_u_belief is None:
             T, E, N, K = self.T, self.E, self.N, self.K
             self.inject(u_action=torch.zeros(T + 1, E, N), u_belief=torch.zeros(T + 1, E, N, K, dtype=torch.float64))
@@ -350,6 +363,7 @@ class IA2CTrainer(RecordsHistory):
         """Pipelined end-to-end form: a list of per-episode pinned host tapes (``pack_host_tape``) in, per-episode
         losses and returns out (the loss / return windows are updated; ``window_stats()`` computes their means on demand).  One H2D copy per episode, overlapping the previous episode's compute, and one D2H
         copy of the result region (``ia2c_train_episodes_host``; multi-rank: the same pipeline with torch streams)."""
+        self._refuse_partners("train_episodes_host")
         n = len(host_tapes)
         N, E = self.N, self.E
         self._ensure_stage()
@@ -442,6 +456,7 @@ class IA2CTrainer(RecordsHistory):
         ms = (C.c_float * 5)()
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):
+            self._seat_partners(self._stream())   # before the first event: the timings cover the episode's kernels only
             _lib.check(self.lib.ia2c_train_episode_timed(C.byref(self.desc), ms, self._stream()), "ia2c_train_episode_timed")
         self.episode += 1
         return dict(zip(("rollout", "critic_grad", "critic_reduce_adam", "actor_grad", "actor_reduce_adam"), list(ms)))
@@ -505,7 +520,7 @@ class IA2CTrainer(RecordsHistory):
         sd.update(episode=self.episode, seed=self.seed, dims=(self.E_total, self.E, self.N, self.M, self.T),
                   rank=self.rank, world=self.world, critic_losses=list(self.critic_losses),
                   actor_losses=list(self.actor_losses), reward_lst=list(self.reward_lst))
-        return sd
+        return self._partner_state(sd)
 
     def load_state_dict(self, sd):
         if tuple(sd["dims"]) != (self.E_total, self.E, self.N, self.M, self.T) or sd["world"] != self.world:
@@ -517,6 +532,7 @@ class IA2CTrainer(RecordsHistory):
         self.desc.seed = self.seed
         self.critic_losses, self.actor_losses = list(sd["critic_losses"]), list(sd["actor_losses"])
         self.reward_lst = list(sd["reward_lst"])
+        self._load_partner_state(sd)   # the checkpoint's pool, or none
 
     def save(self, path):
         torch.save(self.state_dict(), path)

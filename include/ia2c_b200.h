@@ -688,6 +688,51 @@ size_t ia2c_pbt_workspace_bytes(int32_t runs);
 int ia2c_pbt_step(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_history_desc* h, const ia2c_pbt_desc* p,
                   void* stream);
 
+/* ------------------------------------------------------------------ frozen partners: train against a pool of actors -- */
+/* Seats frozen actors from a pool in each run's partner seats before an episode, so that the learning seats train against
+ * partners drawn from a population (fictitious co-play, population play) instead of against one co-learning partner.  Called
+ * before the episode's entry point (ia2c_train_episode, ia2c_rollout, ia2c_train_episode_runs, ia2c_train_episode_runs_many),
+ * which then runs unchanged.  Nothing is read back to the host.
+ *
+ * Definitions (R runs of N agents: `r` NULL is one standalone run, R = 1, keyed by d->seed; else the batch's stacked layout):
+ *   pool    rows f32[P, 105], actor rows (any row may sit in any seat: the IA2C actor reads only the shared observation);
+ *           seats i32[S], the partner seats, distinct, in [0, N), 1 <= S <= N - 1 (at least one seat keeps learning);
+ *           teams i32[Q, S]: team t seats pool row teams[t, j] in seat seats[j].
+ *   draw    before episode k run r draws ONE Philox block, stream 6: key = the run's training seed (r->seed[run], or d->seed),
+ *           counter = (0, 0, 0 | 6 << 16, k) (the layout of the other streams: index 0, t = 0, episode = k = p->episode)
+ *           -> words (x, y, z, w); team = (x * Q) >> 32 in unsigned 64-bit arithmetic.  A run of a batch and a standalone
+ *           trainer with the same seed draw the same teams.
+ *   seat    for each j < S, the 420 bytes of actor_params row r*N + seats[j] become pool row teams[team, j].  Nothing else of
+ *           `d` is written: the partner seats' critic, Adam moments and steps, actor_grad_accum, belief records and models stay
+ *           as they are, and the episode then runs and updates every seat as it always does.  The partner seats' updates are
+ *           discarded by the next call; the row a partner seat holds after an episode is its partner plus one update.
+ * Contract: a run trained with ia2c_seat_partners before each episode computes, byte for byte, what the same entry point
+ * computes when the caller writes the drawn team's rows into the seat rows itself before each episode.
+ * Guarded entries: seats and teams live on the device and are not checked before the launch.  A run whose drawn team has an
+ * entry outside [0, P), or whose seats have one outside [0, N), writes none of its seats and logs -1; other runs are unaffected.
+ * Log: log_team[run] = the drawn team, or -1 (out i32[R]).
+ *
+ * One launch with programmatic dependent launch: partner_seat_kernel, grid (R, ceil(S / seats per block)); every block redraws
+ * its run's Philox block and checks the run's S entries, one thread copies each 4-byte word of a row.  It waits before its
+ * first store (the previous episode's reduce + Adam and ia2c_pbt_step write the rows it overwrites), reads seats, teams and the
+ * seeds after the wait through L2, and releases its successor first thing: every first kernel of an episode reads actor_params
+ * only after its own wait.
+ * Every check runs before the first CUDA call: a NULL descriptor or pointer (d->actor_params, rows, seats, teams, log_team,
+ * r->seed), runs < 1, runs * N above IA2C_MAX_RUN_NETS, S outside 1..N-1, P < 1, Q outside 1..IA2C_PARTNER_MAX_TEAMS
+ * (IA2C_ERR_INVALID); env_offset != 0 or E_total != E (a multi-GPU shard; IA2C_ERR_UNSUPPORTED). */
+#define IA2C_PARTNER_MAX_TEAMS 1048576   /* Q */
+typedef struct ia2c_partner_desc {
+    const float* rows;                /* f32[P, 105]: the pool */
+    int32_t P;                        /* pool rows >= 1 */
+    const int32_t* seats;             /* i32[S] */
+    int32_t S;                        /* 1 <= S <= N - 1 */
+    const int32_t* teams;             /* i32[Q, S] */
+    int32_t Q;                        /* 1 <= Q <= IA2C_PARTNER_MAX_TEAMS */
+    uint32_t episode;                 /* Philox counter word 3: the episode about to run */
+    int32_t* log_team;                /* out i32[R] */
+} ia2c_partner_desc;
+int ia2c_seat_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_partner_desc* p, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
