@@ -128,6 +128,13 @@ class PartnerDesc(C.Structure):
     _fields_ = [("rows", vp), ("P", i32), ("seats", vp), ("S", i32), ("teams", vp), ("Q", i32), ("episode", u32),
                 ("log_team", vp)]
 
+
+class EnvPartnerDesc(C.Structure):
+    """Mirror of ``ia2c_env_partner_desc``: a pool of frozen partners drawn per env inside the rollout kernels
+    (ia2c_train_episode_env_partners)."""
+    _fields_ = [("rows", vp), ("P", i32), ("policy", vp), ("seats", vp), ("S", i32), ("teams", vp), ("Q", i32),
+                ("log_env_team", vp)]
+
 _DP = C.POINTER(EpisodeDesc)
 
 # name -> (restype, argtypes); every symbol declared in include/ia2c_b200.h
@@ -189,6 +196,9 @@ SIGNATURES = {
     "ia2c_pbt_workspace_bytes": (C.c_size_t, [i32]),
     "ia2c_pbt_step": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(HistoryDesc), C.POINTER(PbtDesc), vp]),
     "ia2c_seat_partners": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(PartnerDesc), vp]),
+    "ia2c_partner_policy": (C.c_int, [vp, i32, vp, vp]),
+    "ia2c_rollout_env_partners": (C.c_int, [_DP, C.POINTER(EnvPartnerDesc), vp]),
+    "ia2c_train_episode_env_partners": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(EnvPartnerDesc), vp]),
 }
 
 _lib = None

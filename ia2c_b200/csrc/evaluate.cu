@@ -32,7 +32,7 @@ namespace ia2c {
 namespace {
 
 constexpr int F = IA2C_OBS_FEATURES, A = IA2C_AGENT_ACTIONS;
-constexpr int kClasses = 9;                       // 3 previous x 3 current observation classes
+constexpr int kClasses = kObsClasses;             // 3 previous x 3 current observation classes
 constexpr int kRow = kClasses * A;                // table floats per net
 constexpr uint32_t kStreamEval = 4;               // Philox stream of the evaluation sampler (DESIGN.md §4)
 constexpr int kPolicyThreads = 128;
@@ -80,27 +80,6 @@ __device__ __forceinline__ void eval_env_step(uint32_t packed, int N, int max_st
     }
     s = s2;
     hist = r;
-}
-
-// Table row of thread idx = net * 9 + c: net's softmax at observation class c, into policy[idx * 3 ..].
-__device__ __forceinline__ void policy_row(const float* actor_params, float* policy, int64_t idx) {
-    const int64_t net = idx / kClasses;
-    const int c = (int)(idx - net * kClasses);
-    float flat[kActorP];
-#pragma unroll
-    for (int k = 0; k < kActorP; ++k) flat[k] = __ldcg(actor_params + net * kActorP + k);
-    RegNet<A> w;
-    load_regnet<A>(w, flat);
-    float x[F], y[A];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-        x[k] = (k == c / 3) ? 1.f : 0.f;
-        x[3 + k] = (k == c % 3) ? 1.f : 0.f;
-    }
-    forward_regnet<A>(w, x, y);
-    softmax_inplace<A>(y);
-#pragma unroll
-    for (int o = 0; o < A; ++o) policy[idx * A + o] = y[o];
 }
 
 __global__ void __launch_bounds__(kPolicyThreads) eval_policy_kernel(const __grid_constant__ ia2c_eval_desc d) {

@@ -356,4 +356,30 @@ __device__ __forceinline__ float select_out(const float (&q)[O], int idx) {
     return v;
 }
 
+// Policy table (evaluation, frozen partners per env): row idx = net * 9 + c holds net's softmax at observation class
+// c = 3 * prev_cls + cur_cls, computed with the training samplers' forward and softmax, so it holds the very probabilities they
+// sample from.  Loads through L2 (the rows may come from the kernels just before).
+constexpr int kObsClasses = 9;
+__device__ __forceinline__ void policy_row(const float* actor_params, float* policy, int64_t idx) {
+    constexpr int A = IA2C_AGENT_ACTIONS;
+    const int64_t net = idx / kObsClasses;
+    const int c = (int)(idx - net * kObsClasses);
+    float flat[kActorP];
+#pragma unroll
+    for (int k = 0; k < kActorP; ++k) flat[k] = __ldcg(actor_params + net * kActorP + k);
+    RegNet<A> w;
+    load_regnet<A>(w, flat);
+    float x[kIn], y[A];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        x[k] = (k == c / 3) ? 1.f : 0.f;
+        x[3 + k] = (k == c % 3) ? 1.f : 0.f;
+    }
+    forward_regnet<A>(w, x, y);
+    softmax_inplace<A>(y);
+#pragma unroll
+    for (int o = 0; o < A; ++o) policy[idx * A + o] = y[o];
+}
+
 }  // namespace ia2c
+

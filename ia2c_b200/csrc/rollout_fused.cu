@@ -70,8 +70,10 @@ __device__ __forceinline__ void obs_from_cls(int packed, float (&x)[F]) {
 }
 
 // RUNS: a batch of independent runs (ia2c_train_episode_runs), blockIdx.y = run; see `run` below.
-template <int N, int M, bool CRITIC, bool RUNS>
-__global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc d, float* __restrict__ partials, RunsArg<RUNS> ra) {
+// PARTNERS: frozen partners per env (ia2c_train_episode_env_partners): a partner lane loads its env's pool row instead of its own.
+template <int N, int M, bool CRITIC, bool RUNS, bool PARTNERS = false>
+__global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc d, float* __restrict__ partials, RunsArg<RUNS> ra,
+                                                               PartnerArg<PARTNERS> pa) {
     constexpr int K = N - 1;
     constexpr int G = N <= 2 ? 2 : (N <= 4 ? 4 : 8);     // lanes per env
     constexpr int EPW = 32 / G;
@@ -171,7 +173,15 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
     if (role == 1) {
         // ================================================================ A: env + actor, step t = it - 1
         RegNet<A> net;
-        load_regnet<A>(net, d.actor_params + (net0 + i) * kActorP);
+        if constexpr (PARTNERS) {   // the env's team, drawn once by every lane of its group; the leader logs it
+            const int team = env_team(pa, run_seed<RUNS>(d, ra, run), d.episode, e, N);
+            const int slot = team >= 0 && sub < N ? env_partner_slot(pa, i) : -1;
+            if (live && sub == 0) pa.log[ge] = team;
+            load_regnet<A>(net, slot >= 0 ? pa.rows + (int64_t)__ldcg(pa.teams + (int64_t)team * pa.S + slot) * kActorP
+                                          : d.actor_params + (net0 + i) * kActorP);
+        } else {
+            load_regnet<A>(net, d.actor_params + (net0 + i) * kActorP);
+        }
         int s = 2, prev_cls = 1, cur_cls = 1, elapsed = 0;   // env state, replicated in the group's lanes
         double hist = 0.0, ep_ret = 0.0;
         const double rcp10 = drcp_seq(10.0);
@@ -503,17 +513,27 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
 }
 
 template <int N, int M>
-int launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s) {
+int launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, const EnvPartners* p, cudaStream_t s) {
     constexpr int G = N <= 2 ? 2 : (N <= 4 ? 4 : 8);
     const int64_t blocks = (d->E + (32 / G) - 1) / (32 / G);   // one block = 4 stage warps over 32/G envs
+    if (p) {
+        if (runs)
+            return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, true, true, true>,
+                              dim3((unsigned)blocks, (unsigned)runs->runs), dim3(kBlock), 0, s, *d, d->partials, *runs, *p);
+        if (d->flags & IA2C_FLAG_FUSED_CRITIC)
+            return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, true, false, true>, dim3((unsigned)blocks), dim3(kBlock),
+                              0, s, *d, d->partials, NoRuns{}, *p);
+        return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, false, false, true>, dim3((unsigned)blocks), dim3(kBlock), 0,
+                          s, *d, nullptr, NoRuns{}, *p);
+    }
     if (runs)   // every run with its own row of blocks, partitioned as a standalone run of E envs
         return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, true, true>, dim3((unsigned)blocks, (unsigned)runs->runs),
-                          dim3(kBlock), 0, s, *d, d->partials, *runs);
+                          dim3(kBlock), 0, s, *d, d->partials, *runs, NoPartners{});
     if (d->flags & IA2C_FLAG_FUSED_CRITIC)
         return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, true, false>, dim3((unsigned)blocks), dim3(kBlock), 0, s, *d,
-                          d->partials, NoRuns{});
+                          d->partials, NoRuns{}, NoPartners{});
     return launch_pdl("rollout_fused_kernel", rollout_fused_kernel<N, M, false, false>, dim3((unsigned)blocks), dim3(kBlock), 0, s, *d,
-                      nullptr, NoRuns{});
+                      nullptr, NoRuns{}, NoPartners{});
 }
 
 }  // namespace
@@ -528,16 +548,17 @@ int64_t rollout_fused_blocks(int64_t E, int N) {
 }
 
 // runs != nullptr: all runs of a batch (ia2c_train_episode_runs), always with the critic-gradient stage.
-int rollout_fused_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s) {
-    if (d->M == 3 && d->N == 2) return launch<2, 3>(d, runs, s);
+// p != nullptr: the PARTNERS instantiation (frozen partners per env).
+int rollout_fused_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, const EnvPartners* p, cudaStream_t s) {
+    if (d->M == 3 && d->N == 2) return launch<2, 3>(d, runs, p, s);
     switch (d->N) {
-        case 2: return launch<2, 5>(d, runs, s);
-        case 3: return launch<3, 5>(d, runs, s);
-        case 4: return launch<4, 5>(d, runs, s);
-        case 5: return launch<5, 5>(d, runs, s);
-        case 6: return launch<6, 5>(d, runs, s);
-        case 7: return launch<7, 5>(d, runs, s);
-        case 8: return launch<8, 5>(d, runs, s);
+        case 2: return launch<2, 5>(d, runs, p, s);
+        case 3: return launch<3, 5>(d, runs, p, s);
+        case 4: return launch<4, 5>(d, runs, p, s);
+        case 5: return launch<5, 5>(d, runs, p, s);
+        case 6: return launch<6, 5>(d, runs, p, s);
+        case 7: return launch<7, 5>(d, runs, p, s);
+        case 8: return launch<8, 5>(d, runs, p, s);
     }
     set_error("rollout_fused: no instantiation for N=%d M=%d", d->N, d->M);
     return IA2C_ERR_UNSUPPORTED;

@@ -33,12 +33,14 @@
 
 namespace ia2c {
 int rollout_fused_supported(int N, int M);                                  // rollout_fused.cu
-int rollout_fused_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s);
+int rollout_fused_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, const EnvPartners* p, cudaStream_t s);
 int64_t rollout_fused_blocks(int64_t E, int N);
 int actor_pipe_launch(const ia2c_episode_desc* d, cudaStream_t s);
 int reduce_adam_runs_launch(const ReduceArgs& A, const double* lr_per_net, int nets, cudaStream_t s);   // used by a2c.cu
 int64_t actor_pipe_blocks(int64_t E, int N);
 int belief_pairs_episode_runs_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s);   // belief.cu
+int validate_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p, const char* who);   // partners.cu
+EnvPartners env_partners_arg(const ia2c_env_partner_desc* p);
 
 namespace {
 
@@ -190,9 +192,13 @@ __global__ void __launch_bounds__(kActorThreads) actor_step_kernel(StepArgs S) {
 // RUNS: a batch of independent runs (ia2c_train_episode_runs_many), blockIdx.y = run.  A block's chunk lies inside one run (its
 // threads hold that run's actors, rows run * N + i); the run's envs are columns [run * E, (run + 1) * E) of an env axis of
 // length R * E (stride ES), and `e` stays the env's index within its run, which keys its Philox counters.
+// PARTNERS: frozen partners per env (ia2c_train_episode_env_partners).  The chunk's owner threads draw their envs' teams into
+// shared memory and log them; a partner-seat thread samples from its env's pool row of the policy table (Org has 9 observation
+// classes; the table holds what forward_regnet + softmax_inplace compute, so the samples are those of the row's actor).
 constexpr int kManyMaxEnvs = 32;     // envs per block
-template <bool RUNS>
-__global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant__ ia2c_episode_desc d, int envs_per_block, RunsArg<RUNS> ra) {
+template <bool RUNS, bool PARTNERS = false>
+__global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant__ ia2c_episode_desc d, int envs_per_block, RunsArg<RUNS> ra,
+                                                           const __grid_constant__ PartnerArg<PARTNERS> pa) {
     extern __shared__ __align__(16) unsigned char many_smem[];
     const int N = d.N, T = d.T, i = threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
     const int64_t E = d.E, e0 = (int64_t)blockIdx.x * envs_per_block;
@@ -211,6 +217,20 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
     int s = 2, prev_cls = 1, cur_cls = 1, elapsed = 0;
     double hist = 0.0, ep_ret = 0.0;
     const bool owner = i < EC;
+    __shared__ int team_s[PARTNERS ? kManyMaxEnvs : 1];
+    int slot = -1;   // this agent's partner-seat slot
+    const int32_t* partner_teams = nullptr;
+    const float* partner_policy = nullptr;
+    int partner_S = 0;
+    auto team_of = [&](int el) { return PARTNERS ? team_s[el] : -1; };
+    if constexpr (PARTNERS) {
+        partner_teams = pa.teams, partner_policy = pa.policy, partner_S = pa.S;
+        if (owner) {
+            team_s[i] = env_team(pa, run_seed<RUNS>(d, ra, run), d.episode, e0 + i, N);
+            pa.log[g0 + i] = team_s[i];
+        }
+        if (agent) slot = env_partner_slot(pa, i);
+    }
     if (owner) {
         cls_s[i] = 1 | (1 << 2);
         float* o = d.obs + (g0 + i) * F;
@@ -229,14 +249,22 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
                     a = d.inj_actions[row];
                 } else {
                     const int packed = cls_s[el];
-                    float x[F], y[A];
+                    float y[A];
+                    if (PARTNERS && slot >= 0 && team_of(el) >= 0) {
+                        const int64_t row = __ldcg(partner_teams + (int64_t)team_of(el) * partner_S + slot);
+                        const float* pr = partner_policy + (row * 9 + 3 * (packed & 3) + (packed >> 2)) * A;
 #pragma unroll
-                    for (int k = 0; k < 3; ++k) {
-                        x[k] = (k == (packed & 3)) ? 1.f : 0.f;
-                        x[3 + k] = (k == (packed >> 2)) ? 1.f : 0.f;
+                        for (int k = 0; k < A; ++k) y[k] = __ldcg(pr + k);
+                    } else {
+                        float x[F];
+#pragma unroll
+                        for (int k = 0; k < 3; ++k) {
+                            x[k] = (k == (packed & 3)) ? 1.f : 0.f;
+                            x[3 + k] = (k == (packed >> 2)) ? 1.f : 0.f;
+                        }
+                        forward_regnet<A>(net, x, y);
+                        softmax_inplace<A>(y);
                     }
-                    forward_regnet<A>(net, x, y);
-                    softmax_inplace<A>(y);
                     const float u = d.inj_u_action ? d.inj_u_action[row]
                                                    : philox_uniform_f32(run_seed<RUNS>(d, ra, run), kStreamAction, d.episode, (uint32_t)t,
                                                                         (uint64_t)((d.env_offset + e) * N + i));
@@ -596,14 +624,14 @@ int grad_blocks(const ia2c_episode_desc* d) {
 // blocks (1024 x 256: 7 envs = one wave of 147 blocks instead of two waves of 4).  Envs are independent (no sum crosses an env),
 // so the choice changes no result.
 struct ManyPlan { int threads, envs_per_block; size_t smem; int64_t blocks; };   // blocks: per run (grid x)
-template <bool RUNS>
+template <bool RUNS, bool PARTNERS = false>
 ManyPlan many_plan(const ia2c_episode_desc* d, int runs) {
     ManyPlan p;
     p.threads = ((d->N + 31) / 32) * 32;
     p.smem = (size_t)kManyMaxEnvs * (8 + 1 + 1) * 4 + (size_t)kManyMaxEnvs * p.threads;
     static int resident_per_sm[9] = {0};     // per instantiation, by threads / 32; the same on every B200 of the box
     int& per_sm = resident_per_sm[p.threads / 32];
-    if (per_sm == 0 && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_many_kernel<RUNS>, p.threads, p.smem) != cudaSuccess) per_sm = 1;
+    if (per_sm == 0 && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_many_kernel<RUNS, PARTNERS>, p.threads, p.smem) != cudaSuccess) per_sm = 1;
     const int64_t resident = (int64_t)kSMs * std::max(1, per_sm);
     p.envs_per_block = 1;
     int64_t best = INT64_MAX;
@@ -659,26 +687,33 @@ extern "C" size_t ia2c_episode_partials_floats(const ia2c_episode_desc* d) {
 
 extern "C" int ia2c_rollout_fused_supported(int32_t N, int32_t M) { return rollout_fused_supported(N, M); }
 
-extern "C" int ia2c_rollout(const ia2c_episode_desc* d, void* stream) {
-    if (int rc = validate(d, "ia2c_rollout")) return rc;
+static int check_rollout(const ia2c_episode_desc* d, const char* who) {
+    if (int rc = validate(d, who)) return rc;
     IA2C_REQUIRE(d->env_state && d->env_hist && d->env_cls && d->env_elapsed && d->ep_return && d->belief_records &&
-                     d->filter_action, "ia2c_rollout: null env/belief pointer");
-    cudaStream_t s = as_stream(stream);
+                     d->filter_action, "%s: null env/belief pointer", who);
     if (d->flags & IA2C_FLAG_FUSED_ROLLOUT) {
-        IA2C_REQUIRE(rollout_fused_supported(d->N, d->M), "ia2c_rollout: IA2C_FLAG_FUSED_ROLLOUT needs N<=8 with M=5 (or N=2, M=3); got N=%d M=%d", d->N, d->M);
+        IA2C_REQUIRE(rollout_fused_supported(d->N, d->M), "%s: IA2C_FLAG_FUSED_ROLLOUT needs N<=8 with M=5 (or N=2, M=3); got N=%d M=%d", who, d->N, d->M);
         if (d->flags & IA2C_FLAG_FUSED_CRITIC) {
             IA2C_REQUIRE(d->partials && d->partials_floats >= ia2c_episode_partials_floats(d) && d->critic_step,
-                         "ia2c_rollout: IA2C_FLAG_FUSED_CRITIC needs the partials workspace and critic_step");
+                         "%s: IA2C_FLAG_FUSED_CRITIC needs the partials workspace and critic_step", who);
         }
-        return rollout_fused_launch(d, nullptr, s);
     }
+    return 0;
+}
+
+// The rollout of ia2c_rollout; p != nullptr: the PARTNERS instantiations (the path was checked by validate_env_partners).
+static int rollout_launch(const ia2c_episode_desc* d, const EnvPartners* p, void* stream) {
+    cudaStream_t s = as_stream(stream);
+    if (d->flags & IA2C_FLAG_FUSED_ROLLOUT) return rollout_fused_launch(d, nullptr, p, s);
     const bool episode_beliefs = !(d->flags & IA2C_FLAG_BELIEF_PER_STEP) && ia2c_belief_supports_episode(d->N, d->M);
-    if (episode_beliefs && !(d->flags & IA2C_FLAG_ROLLOUT_PER_STEP) && d->N <= 256) {
+    if (p || (episode_beliefs && !(d->flags & IA2C_FLAG_ROLLOUT_PER_STEP) && d->N <= 256)) {
         // ONE persistent kernel for the T+1 env / actor steps, then ONE kernel for the episode's belief updates
-        const ManyPlan mp = many_plan<false>(d, 1);
-        if (int rc = launch_pdl("rollout_many_kernel", rollout_many_kernel<false>, dim3((unsigned)mp.blocks), dim3(mp.threads), mp.smem, s,
-                                *d, mp.envs_per_block, NoRuns{}))
-            return rc;
+        const ManyPlan mp = p ? many_plan<false, true>(d, 1) : many_plan<false>(d, 1);
+        const int rc = p ? launch_pdl("rollout_many_kernel", rollout_many_kernel<false, true>, dim3((unsigned)mp.blocks), dim3(mp.threads),
+                                      mp.smem, s, *d, mp.envs_per_block, NoRuns{}, *p)
+                         : launch_pdl("rollout_many_kernel", rollout_many_kernel<false>, dim3((unsigned)mp.blocks), dim3(mp.threads),
+                                      mp.smem, s, *d, mp.envs_per_block, NoRuns{}, NoPartners{});
+        if (rc) return rc;
         return ia2c_belief_update_pairs_episode(d->belief_records, d->filter_action, d->act, d->inj_u_belief, d->pred_dump, d->belief_dump,
                                                 d->partner_pred, d->E, d->N, d->M, d->T + 1, d->seed, d->episode, d->env_offset, stream);
     }
@@ -716,6 +751,11 @@ extern "C" int ia2c_rollout(const ia2c_episode_desc* d, void* stream) {
         return ia2c_belief_update_pairs_episode(d->belief_records, d->filter_action, d->act, d->inj_u_belief, d->pred_dump, d->belief_dump,
                                                 d->partner_pred, d->E, d->N, d->M, d->T + 1, d->seed, d->episode, d->env_offset, stream);
     return 0;
+}
+
+extern "C" int ia2c_rollout(const ia2c_episode_desc* d, void* stream) {
+    if (int rc = check_rollout(d, "ia2c_rollout")) return rc;
+    return rollout_launch(d, nullptr, stream);
 }
 
 static int run_reduce(const ia2c_episode_desc* d, int which, int from_partials, int apply, cudaStream_t s) {
@@ -919,11 +959,14 @@ extern "C" int ia2c_apply_adam(const ia2c_episode_desc* d, int32_t which, void* 
     return run_reduce(d, which, 0, 1, as_stream(stream));
 }
 
-extern "C" int ia2c_train_episode(const ia2c_episode_desc* d, void* stream) {
-    if (int rc = ia2c_rollout(d, stream)) return rc;
+// One standalone episode; p != nullptr: with frozen partners per env (the caller checked everything before the first CUDA call).
+static int train_episode_impl(const ia2c_episode_desc* d, const EnvPartners* p, void* stream) {
+    if (int rc = p ? rollout_launch(d, p, stream) : ia2c_rollout(d, stream)) return rc;
     if (int rc = ia2c_critic_phase(d, stream)) return rc;
     return ia2c_actor_phase(d, stream);
 }
+
+extern "C" int ia2c_train_episode(const ia2c_episode_desc* d, void* stream) { return train_episode_impl(d, nullptr, stream); }
 
 // One episode of a multi-GPU run in ONE call per rank: rollout, critic gradient, fused NVLink all-reduce + Adam
 // (epoch0 + 1), actor gradient, fused all-reduce + Adam (epoch0 + 2).  desc.flags = SKIP_ADAM | GRAD_ONLY.
@@ -1292,17 +1335,22 @@ static int reduce_runs(const ia2c_episode_desc& e, const ia2c_runs_desc* r, int 
     return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr);
 }
 
-extern "C" int ia2c_train_episode_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream) {
-    if (int rc = validate_runs(d, r)) return rc;
+// One episode of a batch (N <= 8); p != nullptr: with frozen partners per env.
+static int train_runs_impl(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const EnvPartners* p, void* stream) {
     cudaStream_t s = as_stream(stream);
     const int R = r->runs, nets = R * d->N;
     ia2c_episode_desc e = *d;
     e.flags = IA2C_FLAG_FUSED_ROLLOUT | IA2C_FLAG_FUSED_CRITIC | IA2C_FLAG_ACTOR_COLUMNS;
-    if (int rc = rollout_fused_launch(&e, r, s)) return rc;
+    if (int rc = rollout_fused_launch(&e, r, p, s)) return rc;
     if (int rc = reduce_runs(e, r, 0, s)) return rc;
     dim3 grid(grad_blocks(&e), nets);
     if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
     return reduce_runs(e, r, 1, s);
+}
+
+extern "C" int ia2c_train_episode_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream) {
+    if (int rc = validate_runs(d, r)) return rc;
+    return train_runs_impl(d, r, nullptr, stream);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1345,15 +1393,18 @@ static int validate_runs_many(const ia2c_episode_desc* d, const ia2c_runs_desc* 
     return 0;
 }
 
-extern "C" int ia2c_train_episode_runs_many(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream) {
-    if (int rc = validate_runs_many(d, r)) return rc;
+// One episode of a batch (9 <= N <= 256); p != nullptr: with frozen partners per env.
+static int train_runs_many_impl(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const EnvPartners* p, void* stream) {
     cudaStream_t s = as_stream(stream);
     const int R = r->runs, nets = R * d->N;
     ia2c_episode_desc e = *d;
     e.flags = IA2C_FLAG_ACTOR_COLUMNS;   // both reductions sum grad_blocks(E) partial rows per net
-    const ManyPlan mp = many_plan<true>(&e, R);
-    if (int rc = launch_pdl("rollout_many_kernel", rollout_many_kernel<true>, dim3((unsigned)mp.blocks, (unsigned)R), dim3(mp.threads), mp.smem,
-                            s, e, mp.envs_per_block, *r))
+    const ManyPlan mp = p ? many_plan<true, true>(&e, R) : many_plan<true>(&e, R);
+    const dim3 many_grid((unsigned)mp.blocks, (unsigned)R);
+    if (int rc = p ? launch_pdl("rollout_many_kernel", rollout_many_kernel<true, true>, many_grid, dim3(mp.threads), mp.smem, s, e,
+                                mp.envs_per_block, *r, *p)
+                   : launch_pdl("rollout_many_kernel", rollout_many_kernel<true>, many_grid, dim3(mp.threads), mp.smem, s, e,
+                                mp.envs_per_block, *r, NoPartners{}))
         return rc;
     if (int rc = belief_pairs_episode_runs_launch(&e, r, s)) return rc;
     const dim3 grid(grad_blocks(&e), nets);
@@ -1361,6 +1412,40 @@ extern "C" int ia2c_train_episode_runs_many(const ia2c_episode_desc* d, const ia
     if (int rc = reduce_runs(e, r, 0, s)) return rc;
     if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
     return reduce_runs(e, r, 1, s);
+}
+
+extern "C" int ia2c_train_episode_runs_many(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream) {
+    if (int rc = validate_runs_many(d, r)) return rc;
+    return train_runs_many_impl(d, r, nullptr, stream);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Frozen partners per env (include/ia2c_b200.h: ia2c_train_episode_env_partners): the episode entry points above with the
+// PARTNERS instantiations of the rollout kernels; validate_env_partners (partners.cu) refuses every path that has none.
+extern "C" int ia2c_rollout_env_partners(const ia2c_episode_desc* d, const ia2c_env_partner_desc* p, void* stream) {
+    const char* who = "ia2c_rollout_env_partners";
+    if (int rc = validate_env_partners(d, nullptr, p, who)) return rc;
+    if (int rc = check_rollout(d, who)) return rc;
+    const EnvPartners ep = env_partners_arg(p);
+    return rollout_launch(d, &ep, stream);
+}
+
+extern "C" int ia2c_train_episode_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
+                                               void* stream) {
+    const char* who = "ia2c_train_episode_env_partners";
+    if (int rc = validate_env_partners(d, r, p, who)) return rc;
+    const EnvPartners ep = env_partners_arg(p);
+    if (!r) {
+        if (int rc = check_rollout(d, who)) return rc;
+        if (int rc = check_update_ptrs(d, who)) return rc;
+        return train_episode_impl(d, &ep, stream);
+    }
+    if (d->N <= 8) {
+        if (int rc = validate_runs(d, r)) return rc;
+        return train_runs_impl(d, r, &ep, stream);
+    }
+    if (int rc = validate_runs_many(d, r)) return rc;
+    return train_runs_many_impl(d, r, &ep, stream);
 }
 
 // reduce_adam_kernel<true> for `nets` nets of P entries with one learning rate per net (lr_per_net, or A.lr where NULL): the

@@ -17,7 +17,8 @@ hyper-parameters; ``pbt_history`` reads back what each generation did.
 
 ``set_partners`` (ia2c_b200/partners.py) seats frozen partners from a pool in every run's partner seats before each episode
 (``ia2c_seat_partners``): each run draws a team from its own training seed, so run r still equals a standalone trainer with
-the same seed and pool.
+the same seed and pool.  ``set_partners(pool, per_env=True)`` draws a team per env inside the rollout kernels instead
+(``ia2c_train_episode_env_partners``), with the same rule.
 """
 from __future__ import annotations
 
@@ -154,9 +155,7 @@ class IA2CRuns(SeatsPartners, RecordsHistory):
         ``read_stats`` windows."""
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-            self._seat_partners(stream)
-            _lib.check(getattr(self.lib, self._ENTRY)(C.byref(self.desc), C.byref(self.runs_desc), stream), self._ENTRY)
+            self._enqueue_episode(C.byref(self.desc), torch.cuda.current_stream(self.device).cuda_stream)
         self.episode += 1
         if sync_stats:
             return self.read_stats()
@@ -168,6 +167,10 @@ class IA2CRuns(SeatsPartners, RecordsHistory):
         return self.R, C.byref(self.runs_desc)
 
     def _enqueue_episode(self, desc_ref, stream):
+        if self._env_partners:
+            self._play_env_partners(lambda p: self.lib.ia2c_train_episode_env_partners(desc_ref, C.byref(self.runs_desc), p, stream),
+                                    "ia2c_train_episode_env_partners")
+            return
         self._seat_partners(stream)
         _lib.check(getattr(self.lib, self._ENTRY)(desc_ref, C.byref(self.runs_desc), stream), self._ENTRY)
 

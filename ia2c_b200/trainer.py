@@ -237,8 +237,12 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
     def rollout(self):
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):
-            self._seat_partners(self._stream())
-            _lib.check(self.lib.ia2c_rollout(C.byref(self.desc), self._stream()), "ia2c_rollout")
+            s = self._stream()
+            if self._env_partners:
+                self._play_env_partners(lambda p: self.lib.ia2c_rollout_env_partners(C.byref(self.desc), p, s), "ia2c_rollout_env_partners")
+                return
+            self._seat_partners(s)
+            _lib.check(self.lib.ia2c_rollout(C.byref(self.desc), s), "ia2c_rollout")
 
     def update(self):
         d, s = C.byref(self.desc), self._stream()
@@ -273,8 +277,7 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         if self.world == 1:   # one C call for the whole episode
             self.desc.episode = self.episode
             with torch.cuda.device(self.device):
-                self._seat_partners(self._stream())
-                _lib.check(self.lib.ia2c_train_episode(C.byref(self.desc), self._stream()), "ia2c_train_episode")
+                self._enqueue_episode(C.byref(self.desc), self._stream())
         elif self.p2p:        # one C call per rank: the gradient exchanges are kernels of the same stream
             self.desc.episode = self.episode
             with torch.cuda.device(self.device):
@@ -297,6 +300,10 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         return 1, self.N, self.E, self.T, True
 
     def _enqueue_episode(self, desc_ref, stream):
+        if self._env_partners:
+            self._play_env_partners(lambda p: self.lib.ia2c_train_episode_env_partners(desc_ref, None, p, stream),
+                                    "ia2c_train_episode_env_partners")
+            return
         self._seat_partners(stream)
         _lib.check(self.lib.ia2c_train_episode(desc_ref, stream), "ia2c_train_episode")
 
@@ -304,6 +311,18 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
     def _check_partners(self):
         if self.world > 1:
             raise _lib.IA2CError("set_partners seats partners on one GPU (a rank sees only its env shard)")
+
+    def _check_env_partners(self):
+        """The rollouts with per-env kernels: the fused one (N <= 8) and the whole-episode one (9 <= N <= 256)."""
+        N, M, flags = self.N, self.M, self.desc.flags
+        if N > 256:
+            raise _lib.IA2CError(f"set_partners(per_env=True): n_agents={N} above 256 runs the per-step rollout, which has no per-env kernels")
+        if N <= 8 and not flags & _lib.FLAG_FUSED_ROLLOUT:
+            raise _lib.IA2CError(f"set_partners(per_env=True): n_agents={N}, n_models={M} runs the per-step rollout "
+                                 "(fused_rollout=False or no fused instantiation), which has no per-env kernels")
+        if N > 8 and (flags & (_lib.FLAG_ROLLOUT_PER_STEP | _lib.FLAG_BELIEF_PER_STEP) or not self.lib.ia2c_belief_supports_episode(N, M)):
+            raise _lib.IA2CError("set_partners(per_env=True): the per-step rollout (rollout_kernel='step', belief_kernel='step' "
+                                 "or no whole-episode belief kernel) has no per-env kernels")
 
     def _partner_runs(self):
         return 1, None
@@ -453,6 +472,7 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         {rollout, critic_grad, critic_reduce_adam, actor_grad, actor_reduce_adam}.  Single rank."""
         if self.world > 1:
             raise _lib.IA2CError("train_episode_timed is the single-rank profiling entry point")
+        self._refuse_env_partners("train_episode_timed")
         ms = (C.c_float * 5)()
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):

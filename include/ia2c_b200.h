@@ -733,6 +733,62 @@ typedef struct ia2c_partner_desc {
 } ia2c_partner_desc;
 int ia2c_seat_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_partner_desc* p, void* stream);
 
+/* ------------------------------------------------------------------ frozen partners per env -- */
+/* A second partner mode: instead of one team per run and episode (ia2c_seat_partners), every ENV draws its own team before
+ * every episode, and the rollout kernels play it in that env.  A learner of E envs then meets up to E partners per episode,
+ * so each actor update averages over the pool instead of following one partner's convention (population play).
+ *
+ * Definitions (R runs of N agents, E envs per run; `r` NULL is one standalone run, R = 1, keyed by d->seed):
+ *   pool    rows, P, seats, S, teams, Q as in ia2c_partner_desc; policy f32[P, 9, 3], row p's softmax at observation class
+ *           c = 3 * prev + cur, as ia2c_partner_policy writes it (it is what the training samplers compute from row p).
+ *   draw    before episode k = d->episode, env e of run r (e counted within its run) draws ONE Philox block, stream 7:
+ *           key = the run's training seed (r->seed[run], or d->seed), counter = (e, 0, 0 | 7 << 16, k) -> words (x, y, z, w);
+ *           team = (x * Q) >> 32 in unsigned 64-bit arithmetic.  A run of a batch and a standalone trainer with the same seed
+ *           draw the same teams.
+ *   play    in env e the agent in seat seats[j] acts with pool row teams[team, j]: the same observation, action uniform and
+ *           inverse-CDF sampler as with its own row (if a seat repeats, the lowest j wins).  Nothing of the run's own state is
+ *           read or written for this: the partner seats' own actor rows are never used to act while the mode is on, yet they
+ *           receive the episode's updates as every seat does (their critics, beliefs and Adam state are trained on the
+ *           partners' actions).  A run that leaves the mode continues self-play from those rows.
+ *   guard   an env whose drawn team has a row outside [0, P), or whose seats have one outside [0, N), plays the run's own rows
+ *           in every seat and logs -1; other envs are unaffected.
+ *   log     log_env_team[r * E + e] = the drawn team, or -1 (out i32[R, E], written by the rollout kernel).
+ * Contract: the trajectory is byte-equal to what the same kernel path produces if env e's partner seats held team t_e's rows;
+ * with Q = 1 the mode equals ia2c_seat_partners before each episode, byte for byte, in everything the partner seats' actor rows
+ * do not feed.  Everything after the rollout (critic, belief filter, actor gradient of every seat) is unchanged.
+ *
+ * Kernels: the PARTNERS instantiations of rollout_fused_kernel (N <= 8, every (N, M) it has, standalone and batched: every
+ * env's lane group draws its team once before the step loop, a partner lane loads its pool row into registers, the group's
+ * leader logs) and rollout_many_kernel (9 <= N <= 256: the block's owner threads draw the chunk's teams into shared memory and
+ * log them, a partner-seat thread samples from policy[teams[team, j]] at the env's class).  Pool, seats, teams and table are
+ * read after griddepcontrol.wait.  An episode makes exactly the launches of the unpartnered entry point.
+ *
+ * ia2c_partner_policy: one launch (programmatic dependent launch) writing policy f32[P, 9, 3] from rows f32[P, 105] with the
+ * forward and softmax of ia2c_evaluate's table; build it once per pool (needed for N > 8; the N <= 8 kernels read the rows).
+ * ia2c_rollout_env_partners: what ia2c_rollout does, standalone.  ia2c_train_episode_env_partners: r NULL is
+ * ia2c_train_episode; otherwise ia2c_train_episode_runs (N <= 8) or ia2c_train_episode_runs_many (9 <= N <= 256), with the
+ * same descriptors and checks.
+ * Refusals, all before the first CUDA call.  IA2C_ERR_INVALID: a NULL descriptor or pointer (rows, seats, teams, log_env_team,
+ * r->seed; policy when N > 8), runs < 1, N < 2, runs * N above IA2C_MAX_RUN_NETS, S outside 1..N-1, P < 1, Q outside
+ * 1..IA2C_PARTNER_MAX_TEAMS, and whatever the unpartnered entry point refuses as invalid.  IA2C_ERR_UNSUPPORTED: every path
+ * without a PARTNERS instantiation (standalone N <= 8 without IA2C_FLAG_FUSED_ROLLOUT, an (N, M) without a fused
+ * instantiation, N > 256, IA2C_FLAG_ROLLOUT_PER_STEP or IA2C_FLAG_BELIEF_PER_STEP, no whole-episode belief kernel), injected
+ * actions (inj_actions), and a multi-GPU shard (env_offset != 0 or E_total != E). */
+typedef struct ia2c_env_partner_desc {
+    const float* rows;                /* f32[P, 105]: the pool */
+    int32_t P;                        /* pool rows >= 1 */
+    const float* policy;              /* f32[P, 9, 3] from ia2c_partner_policy; may be NULL for N <= 8 */
+    const int32_t* seats;             /* i32[S] */
+    int32_t S;                        /* 1 <= S <= N - 1 */
+    const int32_t* teams;             /* i32[Q, S] */
+    int32_t Q;                        /* 1 <= Q <= IA2C_PARTNER_MAX_TEAMS */
+    int32_t* log_env_team;            /* out i32[R, E] */
+} ia2c_env_partner_desc;
+int ia2c_partner_policy(const float* rows, int32_t P, float* policy, void* stream);
+int ia2c_rollout_env_partners(const ia2c_episode_desc* d, const ia2c_env_partner_desc* p, void* stream);
+int ia2c_train_episode_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
+                                    void* stream);
+
 #ifdef __cplusplus
 }
 #endif
