@@ -34,6 +34,7 @@ EVAL_MAX_AGENTS = 1023        # IA2C_EVAL_MAX_AGENTS
 EVAL_MAX_STEPS = 65535        # IA2C_EVAL_MAX_STEPS
 EVAL_MAX_LINEUPS = 1 << 20    # IA2C_EVAL_MAX_LINEUPS
 PARTNER_MAX_TEAMS = 1 << 20   # IA2C_PARTNER_MAX_TEAMS
+PARTNER_PRIORITY_MAX_CELLS = 1 << 24   # IA2C_PARTNER_PRIORITY_MAX_CELLS: runs * teams of the prioritized statistics
 
 
 class EpisodeDesc(C.Structure):
@@ -135,6 +136,12 @@ class EnvPartnerDesc(C.Structure):
     _fields_ = [("rows", vp), ("P", i32), ("policy", vp), ("seats", vp), ("S", i32), ("teams", vp), ("Q", i32),
                 ("log_env_team", vp)]
 
+
+class PartnerPriorityDesc(C.Structure):
+    """Mirror of ``ia2c_partner_priority_desc``: per-(run, team) return statistics and the runs' weight tables of prioritized
+    per-env partners (ia2c_record_partner_returns, ia2c_prioritize_partners)."""
+    _fields_ = [("count", vp), ("sum", vp), ("table", vp), ("R", i32), ("Q", i32)]
+
 _DP = C.POINTER(EpisodeDesc)
 
 # name -> (restype, argtypes); every symbol declared in include/ia2c_b200.h
@@ -199,6 +206,11 @@ SIGNATURES = {
     "ia2c_partner_policy": (C.c_int, [vp, i32, vp, vp]),
     "ia2c_rollout_env_partners": (C.c_int, [_DP, C.POINTER(EnvPartnerDesc), vp]),
     "ia2c_train_episode_env_partners": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(EnvPartnerDesc), vp]),
+    "ia2c_rollout_env_partners_prioritized": (C.c_int, [_DP, C.POINTER(EnvPartnerDesc), C.POINTER(PartnerPriorityDesc), vp]),
+    "ia2c_train_episode_env_partners_prioritized": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(EnvPartnerDesc),
+                                                              C.POINTER(PartnerPriorityDesc), vp]),
+    "ia2c_record_partner_returns": (C.c_int, [_DP, vp, C.POINTER(PartnerPriorityDesc), vp]),
+    "ia2c_prioritize_partners": (C.c_int, [C.POINTER(PartnerPriorityDesc), i32, f64, i32, vp]),
 }
 
 _lib = None

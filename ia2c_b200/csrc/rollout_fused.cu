@@ -174,7 +174,7 @@ __global__ void __launch_bounds__(kBlock) rollout_fused_kernel(ia2c_episode_desc
         // ================================================================ A: env + actor, step t = it - 1
         RegNet<A> net;
         if constexpr (PARTNERS) {   // the env's team, drawn once by every lane of its group; the leader logs it
-            const int team = env_team(pa, run_seed<RUNS>(d, ra, run), d.episode, e, N);
+            const int team = env_team(pa, run_seed<RUNS>(d, ra, run), d.episode, e, N, run);
             const int slot = team >= 0 && sub < N ? env_partner_slot(pa, i) : -1;
             if (live && sub == 0) pa.log[ge] = team;
             load_regnet<A>(net, slot >= 0 ? pa.rows + (int64_t)__ldcg(pa.teams + (int64_t)team * pa.S + slot) * kActorP

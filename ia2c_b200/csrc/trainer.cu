@@ -41,6 +41,7 @@ int64_t actor_pipe_blocks(int64_t E, int N);
 int belief_pairs_episode_runs_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s);   // belief.cu
 int validate_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p, const char* who);   // partners.cu
 EnvPartners env_partners_arg(const ia2c_env_partner_desc* p);
+int validate_partner_priority(const ia2c_partner_priority_desc* w, const char* who);
 
 namespace {
 
@@ -226,7 +227,7 @@ __global__ void __launch_bounds__(256) rollout_many_kernel(const __grid_constant
     if constexpr (PARTNERS) {
         partner_teams = pa.teams, partner_policy = pa.policy, partner_S = pa.S;
         if (owner) {
-            team_s[i] = env_team(pa, run_seed<RUNS>(d, ra, run), d.episode, e0 + i, N);
+            team_s[i] = env_team(pa, run_seed<RUNS>(d, ra, run), d.episode, e0 + i, N, run);
             pa.log[g0 + i] = team_s[i];
         }
         if (agent) slot = env_partner_slot(pa, i);
@@ -1422,6 +1423,16 @@ extern "C" int ia2c_train_episode_runs_many(const ia2c_episode_desc* d, const ia
 // ------------------------------------------------------------------------------------------------
 // Frozen partners per env (include/ia2c_b200.h: ia2c_train_episode_env_partners): the episode entry points above with the
 // PARTNERS instantiations of the rollout kernels; validate_env_partners (partners.cu) refuses every path that has none.
+// The prioritized twins' own checks (the priority descriptor matches the runs and the pool), after validate_env_partners.
+static int check_priority(const ia2c_runs_desc* r, const ia2c_env_partner_desc* p, const ia2c_partner_priority_desc* w,
+                          const char* who) {
+    if (int rc = validate_partner_priority(w, who)) return rc;
+    const int32_t R = r ? r->runs : 1;
+    IA2C_REQUIRE(w->R == R, "%s: priority R=%d, but %d runs", who, w->R, R);
+    IA2C_REQUIRE(w->Q == p->Q, "%s: priority Q=%d, but the pool has Q=%d", who, w->Q, p->Q);
+    return 0;
+}
+
 extern "C" int ia2c_rollout_env_partners(const ia2c_episode_desc* d, const ia2c_env_partner_desc* p, void* stream) {
     const char* who = "ia2c_rollout_env_partners";
     if (int rc = validate_env_partners(d, nullptr, p, who)) return rc;
@@ -1430,11 +1441,27 @@ extern "C" int ia2c_rollout_env_partners(const ia2c_episode_desc* d, const ia2c_
     return rollout_launch(d, &ep, stream);
 }
 
-extern "C" int ia2c_train_episode_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
-                                               void* stream) {
-    const char* who = "ia2c_train_episode_env_partners";
+extern "C" int ia2c_rollout_env_partners_prioritized(const ia2c_episode_desc* d, const ia2c_env_partner_desc* p,
+                                                     const ia2c_partner_priority_desc* w, void* stream) {
+    const char* who = "ia2c_rollout_env_partners_prioritized";
+    IA2C_REQUIRE(w, "%s: null priority descriptor", who);
+    if (int rc = validate_env_partners(d, nullptr, p, who)) return rc;
+    if (int rc = check_priority(nullptr, p, w, who)) return rc;
+    if (int rc = check_rollout(d, who)) return rc;
+    EnvPartners ep = env_partners_arg(p);
+    ep.table = w->table;
+    return rollout_launch(d, &ep, stream);
+}
+
+// The uniform per-env episode, or (w != nullptr) the prioritized one drawing from w->table.
+static int train_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
+                              const ia2c_partner_priority_desc* w, const char* who, void* stream) {
     if (int rc = validate_env_partners(d, r, p, who)) return rc;
-    const EnvPartners ep = env_partners_arg(p);
+    EnvPartners ep = env_partners_arg(p);
+    if (w) {
+        if (int rc = check_priority(r, p, w, who)) return rc;
+        ep.table = w->table;
+    }
     if (!r) {
         if (int rc = check_rollout(d, who)) return rc;
         if (int rc = check_update_ptrs(d, who)) return rc;
@@ -1446,6 +1473,19 @@ extern "C" int ia2c_train_episode_env_partners(const ia2c_episode_desc* d, const
     }
     if (int rc = validate_runs_many(d, r)) return rc;
     return train_runs_many_impl(d, r, &ep, stream);
+}
+
+extern "C" int ia2c_train_episode_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
+                                               void* stream) {
+    return train_env_partners(d, r, p, nullptr, "ia2c_train_episode_env_partners", stream);
+}
+
+extern "C" int ia2c_train_episode_env_partners_prioritized(const ia2c_episode_desc* d, const ia2c_runs_desc* r,
+                                                           const ia2c_env_partner_desc* p, const ia2c_partner_priority_desc* w,
+                                                           void* stream) {
+    const char* who = "ia2c_train_episode_env_partners_prioritized";
+    IA2C_REQUIRE(w, "%s: null priority descriptor", who);
+    return train_env_partners(d, r, p, w, who, stream);
 }
 
 // reduce_adam_kernel<true> for `nets` nets of P entries with one learning rate per net (lr_per_net, or A.lr where NULL): the

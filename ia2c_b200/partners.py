@@ -15,6 +15,11 @@ episode number and the env's index within its run), and the rollout kernels play
 (``ia2c_train_episode_env_partners``): a learner of E envs meets up to E partners per episode instead of one.  The partner
 seats' own actor rows are not used to act while the mode is on; they still receive every episode's update, and after
 ``set_partners(None)`` self-play continues from them.  ``env_partner_history`` reads back the team of every env.
+
+``set_partners(pool, per_env=True, prioritized=True)`` weights those draws (prioritized fictitious self-play): after every
+episode one more launch adds each env's return to its run's statistics for the team it played (``ia2c_record_partner_returns``),
+and ``prioritize_partners`` rebuilds every run's weight table from them in one launch (``ia2c_prioritize_partners``), giving
+the teams a run does worst with the largest weights.  ``partner_returns`` and ``partner_weights`` read both back.
 """
 from __future__ import annotations
 
@@ -133,6 +138,7 @@ class SeatsPartners:
     _partner_log = None
     _env_partners = False       # per-env mode
     _env_partner_log = None
+    _priority = None            # prioritized per-env mode: {"count", "sum", "table"} device tensors and "desc"
 
     def _check_partners(self):
         """Raise, before any device work, where partners cannot be seated."""
@@ -140,7 +146,7 @@ class SeatsPartners:
     def _check_env_partners(self):
         """Raise, before any device work, where partners cannot be played per env."""
 
-    def set_partners(self, pool, per_env=False):
+    def set_partners(self, pool, per_env=False, prioritized=False):
         """Seat partners from ``pool`` (a ``PartnerPool`` of this trainer's n_agents and device) before every episode that
         ``train_episode``, ``train_episodes`` (and ``IA2CTrainer.rollout``) start, or stop with ``None``.  Each run draws one
         team per episode (Philox stream 6: key = its training seed, counter word 3 = the episode number) and the team's rows
@@ -156,9 +162,17 @@ class SeatsPartners:
         episode's updates, so after ``set_partners(None)`` self-play continues from rows trained on the partners'
         trajectories.  Refused (before any device work) where the rollout has no per-env kernels: the per-step rollout
         (``fused_rollout=False`` or an (N, M) without a fused instantiation up to 8 agents; ``rollout_kernel="step"`` or
-        ``belief_kernel="step"`` above), N > 256 and more than one GPU; injected actions are refused when an episode starts."""
+        ``belief_kernel="step"`` above), N > 256 and more than one GPU; injected actions are refused when an episode starts.
+
+        ``prioritized=True`` (with ``per_env=True`` only): each run draws its envs' teams with the weights of its own table
+        (include/ia2c_b200.h, ia2c_partner_priority_desc, states the definitions), equal until the first
+        ``prioritize_partners``, so until then the episodes are byte for byte those of the uniform mode.  Every episode adds one
+        launch that records each env's return for the team it played; nothing synchronises.  Every ``set_partners`` call
+        starts from zeroed statistics and equal weights, and ``set_partners(None)`` drops them."""
+        if prioritized and not per_env:
+            raise ValueError("set_partners: prioritized=True draws per env: pass per_env=True")
         if pool is None:
-            self._partners, self._env_partners = None, False
+            self._partners, self._env_partners, self._priority = None, False, None
             return
         self._check_partners()
         if not isinstance(pool, PartnerPool):
@@ -169,16 +183,32 @@ class SeatsPartners:
             raise ValueError(f"set_partners: the pool lives on {pool.device}, this trainer on {self.device}")
         if per_env:
             self._check_env_partners()
+            R, _ = self._partner_runs()
+            if prioritized and R * pool.Q > _lib.PARTNER_PRIORITY_MAX_CELLS:
+                raise ValueError(f"set_partners: runs * teams = {R * pool.Q} above PARTNER_PRIORITY_MAX_CELLS "
+                                 f"({_lib.PARTNER_PRIORITY_MAX_CELLS})")
             e = _lib.EnvPartnerDesc()
             e.rows, e.P, e.seats, e.S = pool.rows.data_ptr(), pool.P, pool.seats.data_ptr(), pool.S
             e.teams, e.Q = pool.teams.data_ptr(), pool.Q
             e.policy = pool.policy_table(self.lib).data_ptr() if self.N > 8 else None
             self._partners, self._env_partners, self._env_partner_desc = pool, True, e
+            self._priority = self._new_priority(R, pool.Q) if prioritized else None
             return
         p = _lib.PartnerDesc()
         p.rows, p.P, p.seats, p.S = pool.rows.data_ptr(), pool.P, pool.seats.data_ptr(), pool.S
         p.teams, p.Q = pool.teams.data_ptr(), pool.Q
-        self._partners, self._env_partners, self._partner_desc = pool, False, p
+        self._partners, self._env_partners, self._partner_desc, self._priority = pool, False, p, None
+
+    def _new_priority(self, R, Q):
+        """Zeroed statistics and equal weights (C_q = q * 2^24) for R runs of Q teams, on the device."""
+        with torch.cuda.device(self.device):
+            pr = dict(count=torch.zeros((R, Q), dtype=torch.int64, device=self.device),
+                      sum=torch.zeros((R, Q), dtype=torch.int64, device=self.device),
+                      table=(torch.arange(Q + 1, dtype=torch.int64, device=self.device) << 24).repeat(R, 1))
+        w = _lib.PartnerPriorityDesc()
+        w.count, w.sum, w.table, w.R, w.Q = pr["count"].data_ptr(), pr["sum"].data_ptr(), pr["table"].data_ptr(), R, Q
+        pr["desc"] = w
+        return pr
 
     @property
     def partners(self):
@@ -194,9 +224,15 @@ class SeatsPartners:
         if self._env_partners:
             raise _lib.IA2CError(f"{what} does not play partners per env: call set_partners(None) first")
 
-    def _play_env_partners(self, call, name):
+    @property
+    def partners_prioritized(self):
+        """True while the per-env draws are weighted (``set_partners(pool, per_env=True, prioritized=True)``)."""
+        return self._priority is not None
+
+    def _play_env_partners(self, call, name, call_prioritized=None, desc_ref=None, stream=None):
         """Enqueue one per-env episode: ``call(partner descriptor reference)`` returns the C status; its log slot is taken
-        here."""
+        here.  In the prioritized mode ``call_prioritized(partner descriptor reference, priority descriptor reference)`` runs
+        the episode instead, followed by the record of its returns (``desc_ref``: the episode descriptor, on ``stream``)."""
         if getattr(self, "inj_actions", None) is not None:
             raise _lib.IA2CError(f"{name}: injected actions replace the partners' samples (inject(actions=None) first)")
         R, _ = self._partner_runs()
@@ -206,8 +242,54 @@ class SeatsPartners:
         log, p = self._env_partner_log, self._env_partner_desc
         slot = log.free_slot()
         p.log_env_team = log.ptr["env_team"] + slot * log.row_bytes["env_team"]
-        _lib.check(call(C.byref(p)), name)
+        if self._priority is None:
+            _lib.check(call(C.byref(p)), name)
+        else:
+            w = C.byref(self._priority["desc"])
+            _lib.check(call_prioritized(C.byref(p), w), name + "_prioritized")
+            _lib.check(self.lib.ia2c_record_partner_returns(desc_ref, p.log_env_team, w, stream), "ia2c_record_partner_returns")
         log.commit(episode=self.episode)
+
+    def _require_priority(self, what):
+        if self._priority is None:
+            raise _lib.IA2CError(f"{what}: partners are not drawn with priorities (set_partners(pool, per_env=True, prioritized=True))")
+
+    def prioritize_partners(self, power=2, floor=0.1, reset=True):
+        """Rebuild every run's weight table from its statistics, in one launch and without synchronising: the team with the
+        lowest mean return gets weight 1, the one with the highest gets ``floor``, and in between w = floor + (1 - floor) *
+        x ** power, x = (best mean - mean) / (best mean - worst mean); a team never played gets 1, so it is tried.  ``reset``
+        zeroes the statistics in the same launch, so that the next call weighs only the episodes after this one."""
+        self._require_priority("prioritize_partners")
+        if isinstance(power, bool) or not isinstance(power, (int, np.integer)) or not 0 <= power <= 16:
+            raise ValueError(f"prioritize_partners: power={power!r} must be an integer in [0, 16]")
+        floor = float(floor)
+        if not 0.0 <= floor <= 1.0:
+            raise ValueError(f"prioritize_partners: floor={floor} outside [0, 1]")
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ia2c_prioritize_partners(C.byref(self._priority["desc"]), int(power), floor, int(bool(reset)),
+                                                         torch.cuda.current_stream(self.device).cuda_stream),
+                       "ia2c_prioritize_partners")
+
+    def _run_axis(self, a):
+        return a[0] if self._partner_runs()[1] is None else a
+
+    def partner_returns(self):
+        """Synchronise and return the statistics since the last reset: ``count`` [R, Q] i64 (episodes' envs that played team
+        q) and ``mean`` [R, Q] f64 (their mean return, as the fixed-point sums give it; NaN where count is 0).
+        ``IA2CTrainer``: [Q]."""
+        self._require_priority("partner_returns")
+        with torch.cuda.device(self.device):
+            count, total = self._priority["count"].cpu().numpy(), self._priority["sum"].cpu().numpy()
+        with np.errstate(invalid="ignore", divide="ignore"):
+            mean = np.where(count > 0, total.astype(np.float64) * 2.0 ** -20 / count, np.nan)
+        return dict(count=self._run_axis(count), mean=self._run_axis(mean))
+
+    def partner_weights(self):
+        """Synchronise and return every run's team weights W [R, Q] i64 (2^24 is weight 1; ``IA2CTrainer``: [Q])."""
+        self._require_priority("partner_weights")
+        with torch.cuda.device(self.device):
+            table = self._priority["table"].cpu().numpy()
+        return self._run_axis(np.diff(table, axis=1))
 
     def env_partner_history(self):
         """Synchronise and return every per-env episode since the previous call: ``episode`` [n] and ``env_team`` [n, R, E]
@@ -246,15 +328,29 @@ class SeatsPartners:
         team = np.concatenate([c["team"] for c in chunks]) if chunks else np.zeros((0, R), dtype=np.int32)
         return dict(episode=ep, team=team[:, 0] if runs_ref is None else team)
 
-    def _partner_state(self, sd):
+    def _partner_state(self, sd, run=None):
+        """Add the pool, the mode and the prioritized statistics and table (all runs', or run ``run``'s alone) to ``sd``."""
         if self._partners is not None:
             sd["partners"] = self._partners.state()
             sd["partners_per_env"] = self._env_partners
+            if self._priority is not None:
+                rows = slice(None) if run is None else slice(run, run + 1)
+                sd["partner_priority"] = {k: self._priority[k][rows].detach().cpu().clone() for k in ("count", "sum", "table")}
         return sd
 
     def _load_partner_state(self, sd):
-        """Restore the pool and mode a checkpoint carries (a checkpoint without the mode is per-episode), or clear the pool
-        for one without."""
+        """Restore the pool, mode and prioritized statistics a checkpoint carries (a checkpoint without the mode is
+        per-episode, one without statistics is uniform), or clear the pool for one without."""
         part = sd.get("partners")
+        prio = sd.get("partner_priority") if part is not None else None
+        if prio is not None:
+            R, Q = self._partner_runs()[0], int(part["teams"].shape[0])
+            for k, shape in (("count", (R, Q)), ("sum", (R, Q)), ("table", (R, Q + 1))):
+                if tuple(prio[k].shape) != shape:
+                    raise ValueError(f"checkpoint partner_priority[{k!r}] has shape {tuple(prio[k].shape)}, expected {shape}")
         self.set_partners(PartnerPool(part["rows"], part["teams"], part["seats"], self.N, device=self.device)
-                          if part is not None else None, per_env=bool(sd.get("partners_per_env", False)))
+                          if part is not None else None, per_env=bool(sd.get("partners_per_env", False)),
+                          **({"prioritized": True} if prio is not None else {}))
+        if prio is not None:
+            for k in ("count", "sum", "table"):
+                self._priority[k].copy_(prio[k])

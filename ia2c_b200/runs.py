@@ -168,8 +168,11 @@ class IA2CRuns(SeatsPartners, RecordsHistory):
 
     def _enqueue_episode(self, desc_ref, stream):
         if self._env_partners:
-            self._play_env_partners(lambda p: self.lib.ia2c_train_episode_env_partners(desc_ref, C.byref(self.runs_desc), p, stream),
-                                    "ia2c_train_episode_env_partners")
+            runs = C.byref(self.runs_desc)
+            self._play_env_partners(lambda p: self.lib.ia2c_train_episode_env_partners(desc_ref, runs, p, stream),
+                                    "ia2c_train_episode_env_partners",
+                                    lambda p, w: self.lib.ia2c_train_episode_env_partners_prioritized(desc_ref, runs, p, w, stream),
+                                    desc_ref, stream)
             return
         self._seat_partners(stream)
         _lib.check(getattr(self.lib, self._ENTRY)(desc_ref, C.byref(self.runs_desc), stream), self._ENTRY)
@@ -211,7 +214,7 @@ class IA2CRuns(SeatsPartners, RecordsHistory):
         sd.update(episode=self.episode, seed=self.seeds[r], dims=(self.E, self.E, self.N, self.M, self.T), rank=0, world=1,
                   critic_losses=[x[r].copy() for x in self.critic_losses], actor_losses=[x[r].copy() for x in self.actor_losses],
                   reward_lst=[x[r].copy() for x in self.reward_lst])
-        return self._partner_state(sd)
+        return self._partner_state(sd, run=r)
 
     # ------------------------------------------------------------------ checkpoint / resume of the whole batch
     def state_dict(self):
@@ -336,7 +339,8 @@ class IA2CRuns(SeatsPartners, RecordsHistory):
         index.  Each of the bottom q = floor(fraction * R) runs takes a donor from the top q (Philox stream 5 keyed by
         ``seed``, counter word 3 the generation): its parameters, Adam moments and steps, actor gradient sum and belief
         models become a byte copy of the donor's, and it inherits the donor's hyper-parameters, each name in ``perturb``
-        multiplied by factors[0] or factors[1].  A recipient keeps its seed, env state and statistics windows.  Afterwards
+        multiplied by factors[0] or factors[1].  A recipient keeps its seed, env state and statistics windows, and with
+        prioritized partners its own partner statistics and weight table: they describe the episodes it played.  Afterwards
         run r equals ``IA2CTrainer(E, n_agents=N, n_models=M, seed=seeds[r], **run_hyper(r))`` (``actor_kernel="columns"``
         for N > 8) loaded with ``run_state_dict(r)``.  Two launches; the log (``pbt_history``) drains, synchronising, once
         every ``PBT_LOG_CAPACITY - 1`` generations that ``pbt_history`` has not read."""

@@ -239,7 +239,9 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         with torch.cuda.device(self.device):
             s = self._stream()
             if self._env_partners:
-                self._play_env_partners(lambda p: self.lib.ia2c_rollout_env_partners(C.byref(self.desc), p, s), "ia2c_rollout_env_partners")
+                d = C.byref(self.desc)
+                self._play_env_partners(lambda p: self.lib.ia2c_rollout_env_partners(d, p, s), "ia2c_rollout_env_partners",
+                                        lambda p, w: self.lib.ia2c_rollout_env_partners_prioritized(d, p, w, s), d, s)
                 return
             self._seat_partners(s)
             _lib.check(self.lib.ia2c_rollout(C.byref(self.desc), s), "ia2c_rollout")
@@ -302,7 +304,9 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
     def _enqueue_episode(self, desc_ref, stream):
         if self._env_partners:
             self._play_env_partners(lambda p: self.lib.ia2c_train_episode_env_partners(desc_ref, None, p, stream),
-                                    "ia2c_train_episode_env_partners")
+                                    "ia2c_train_episode_env_partners",
+                                    lambda p, w: self.lib.ia2c_train_episode_env_partners_prioritized(desc_ref, None, p, w, stream),
+                                    desc_ref, stream)
             return
         self._seat_partners(stream)
         _lib.check(self.lib.ia2c_train_episode(desc_ref, stream), "ia2c_train_episode")

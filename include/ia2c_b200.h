@@ -789,6 +789,58 @@ int ia2c_rollout_env_partners(const ia2c_episode_desc* d, const ia2c_env_partner
 int ia2c_train_episode_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
                                     void* stream);
 
+/* ------------------------------------------------------------------ prioritized partners per env -- */
+/* The per-env mode above draws every team with probability 1/Q, so a learner spends most of its samples on partners it
+ * already plays well with.  Prioritized draws (prioritized fictitious self-play) weight each team by how badly the run does
+ * with it, from statistics the device records after every episode: no host round trip.  Only the per-env mode has them.
+ *
+ * Definitions (R runs, E envs per run, Q teams; a standalone run is R = 1):
+ *   statistics  count i64[R, Q] and sum i64[R, Q].  ia2c_record_partner_returns, after a prioritized episode, adds for every
+ *               env e of run r with logged team t = env_team[r * E + e]:  count[r, t] += 1,
+ *               sum[r, t] += llrint(ep_return[r * E + e] * 2^20) (round half to even: fixed point with 20 fraction bits).
+ *               An env is skipped where t lies outside [0, Q) (a logged -1), where its return is not finite, or where
+ *               |return| * 2^20 >= 2^62.  Integer adds give the same bytes in any order (64-bit atomics); sums wrap.
+ *   weights     ia2c_prioritize_partners(power p in 0..16, floor f in [0, 1]), per run, in fp64 with correctly rounded
+ *               operations and no contraction:  for every played team (count > 0) m_q = ((double)sum_q * 2^-20) / (double)count_q;
+ *               hi, lo = the largest and smallest m_q.  No team played, or hi == lo: W_q = 2^24 for every q.  Otherwise
+ *               x_q = (hi - m_q) / (hi - lo) and w_q = f + (1 - f) * x_q^p for a played team (x^p multiplied left to right from
+ *               x^0 = 1), w_q = 1 (the worst played team's weight: untried partners are tried) for an unplayed one, and
+ *               W_q = min(2^24, floor(w_q * 2^24)).
+ *   table       u64[R, Q + 1]: C_0 = 0, C_{q+1} = C_q + W_q.  Equal weights (C_q = q * 2^24) until the first
+ *               ia2c_prioritize_partners; the caller initialises it so.  `reset` zeroes the run's statistics in the same launch.
+ *   draw        env e of run r takes the stream-7 word x of ia2c_env_partner_desc's draw; y = floor(x * C_Q / 2^32) (a 128-bit
+ *               product) and the team is the q with C_q <= y < C_{q+1}: teams of weight 0 are never drawn.  With equal
+ *               weights this is (x * Q) >> 32 exactly, so a prioritized run equals a uniform per-env run byte for byte until
+ *               its first ia2c_prioritize_partners.  C_Q = 0 logs -1 (the env plays its own rows); the guard of the per-env
+ *               mode is unchanged.
+ *
+ * ia2c_rollout_env_partners_prioritized / ia2c_train_episode_env_partners_prioritized: ia2c_rollout_env_partners /
+ * ia2c_train_episode_env_partners drawing from w->table (the PARTNERS instantiations of the rollout kernels: same launches).
+ * ia2c_record_partner_returns: one launch (partner_returns_kernel, one thread per (run, env)) after the episode's kernels,
+ * reading d->ep_return (R * E entries) and the episode's env-team log.  ia2c_prioritize_partners: one launch
+ * (partner_priority_kernel, one block per run: min / max, weights, prefix scan, optional reset).  All programmatic dependent
+ * launches that read nothing before griddepcontrol.wait.
+ * Refusals, all before the first CUDA call.  IA2C_ERR_INVALID: a NULL descriptor or pointer (count, sum, table; env_team,
+ * d->ep_return), R < 1, Q outside 1..IA2C_PARTNER_MAX_TEAMS, R * Q above IA2C_PARTNER_PRIORITY_MAX_CELLS, E < 1, p outside
+ * 0..16, f outside [0, 1], and for the twins R != runs or Q != the pool's Q, with everything the uniform entry points refuse
+ * (with their status).  IA2C_ERR_UNSUPPORTED: ia2c_record_partner_returns on a multi-GPU shard (env_offset != 0 or
+ * E_total != E). */
+#define IA2C_PARTNER_PRIORITY_MAX_CELLS 16777216   /* R * Q: 16 B of statistics per cell */
+typedef struct ia2c_partner_priority_desc {
+    int64_t* count;                   /* i64[R, Q] */
+    int64_t* sum;                     /* i64[R, Q]: returns in fixed point, 2^-20 */
+    uint64_t* table;                  /* u64[R, Q + 1]: prefix sums of the weights */
+    int32_t R;                        /* runs >= 1 */
+    int32_t Q;                        /* teams, the pool's Q */
+} ia2c_partner_priority_desc;
+int ia2c_rollout_env_partners_prioritized(const ia2c_episode_desc* d, const ia2c_env_partner_desc* p,
+                                          const ia2c_partner_priority_desc* w, void* stream);
+int ia2c_train_episode_env_partners_prioritized(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
+                                                const ia2c_partner_priority_desc* w, void* stream);
+int ia2c_record_partner_returns(const ia2c_episode_desc* d, const int32_t* env_team, const ia2c_partner_priority_desc* w,
+                                void* stream);
+int ia2c_prioritize_partners(const ia2c_partner_priority_desc* w, int32_t power, double floor_weight, int32_t reset, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
