@@ -250,7 +250,7 @@ __global__ void debug_divide_kernel(const double* __restrict__ a, const double* 
 //  (2) the stored posterior is rint(100 * bp[m]/S) and the predicted action is a comparison of u with the cumulative
 //      mixture — both are DECISIONS, so they are first taken in fp32 (table lookups, one MUFU.RCP, FFMA) together with
 //      a rigorous distance-to-the-boundary test: the fp32 quotient 100*bp/S is within 6e-5 of the fp64 value
-//      (9 roundings of 2^-24 relative on a value <= 100), so a rounding is accepted only when it is more than 1e-4
+//      (10 roundings of 2^-24 relative on a value <= 100), so a rounding is accepted only when it is more than 1e-4
 //      away from a half-integer; the inverse-CDF comparison u*S < sum_m bp[m]*Fcum[m][a] is accepted only when the
 //      two sides differ by more than 1e-5*S (their fp32 errors are below 1e-6*S each);
 //  (3) a record that fails either test (~0.1 % of them) is recomputed with the exact fp64 sequence of belief_core on
@@ -263,8 +263,8 @@ __global__ void debug_divide_kernel(const double* __restrict__ a, const double* 
 // FAST = the steady-state call of the rollout (device Philox, no dumps, priors from the records): the optional
 // pointers are compiled out instead of costing a predicated-off instruction each per record.
 constexpr float kRoundMagic = 12582912.f;       // 1.5 * 2^23: x + magic has rint(x) in its low mantissa bits
-// Rounding screen: x32 = bp32 * (rcp.approx(S32) * 100) differs from the real 100*bp/S by at most 9 * 2^-24 relative (table entry
-// 1, four fp32 adds + their inputs 5, rcp.approx 2, the *100 1 — units of 2^-24), i.e. 5.4e-5 at x = 100; the window is 1.9 x that.
+// Rounding screen: x32 = bp32 * (rcp.approx(S32) * 100) differs from the real 100*bp/S by at most 10 * 2^-24 relative (table entry
+// 1, M - 1 <= five fp32 adds + their inputs 6, rcp.approx 2, the *100 1 — units of 2^-24), i.e. 6.0e-5 at x = 100; the window is 1.7 x that.
 constexpr float kHalfWindow = 0.5f - 1.0e-4f;    // |100*b - rint(100*b)| above this -> exact path
 constexpr float kCdfWindow = 1e-5f;              // |u*S - cumulative| below this * S -> exact path
 
@@ -319,8 +319,8 @@ __device__ __forceinline__ float lds_f32(uint32_t addr) {
 }
 
 // Second-level rounding screen of ONE record, run by the rare lanes whose first-level test (constant window kHalfWindow)
-// fired: the same fp32 quantities, but every value is tested against its OWN error bound — x32 is within 9 * 2^-24 * x of the
-// real quotient, so a rounding is safe when |x32 - rint(x32)| < 0.5 - 1e-6 * (rint(x32) + 1) (1.9 x the bound).  Cuts the
+// fired: the same fp32 quantities, but every value is tested against its OWN error bound — x32 is within 10 * 2^-24 * x of the
+// real quotient, so a rounding is safe when |x32 - rint(x32)| < 0.5 - 1e-6 * (rint(x32) + 1) (1.7 x the bound).  Cuts the
 // records that reach the fp64 sequence by ~5x.  -> true when the record still needs the exact path.
 template <int M>
 __device__ __noinline__ bool belief_refine_rounding(uint32_t row_s, uint2 raw) {
