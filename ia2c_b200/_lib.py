@@ -142,6 +142,11 @@ class PartnerPriorityDesc(C.Structure):
     per-env partners (ia2c_record_partner_returns, ia2c_prioritize_partners)."""
     _fields_ = [("count", vp), ("sum", vp), ("table", vp), ("R", i32), ("Q", i32)]
 
+
+class FrozenSeats(C.Structure):
+    """Mirror of ``ia2c_frozen_seats``: bit n of mask[n >> 6] set, seat n frozen (ia2c_train_episode_frozen)."""
+    _fields_ = [("mask", u64 * 4)]
+
 _DP = C.POINTER(EpisodeDesc)
 
 # name -> (restype, argtypes); every symbol declared in include/ia2c_b200.h
@@ -211,6 +216,8 @@ SIGNATURES = {
                                                               C.POINTER(PartnerPriorityDesc), vp]),
     "ia2c_record_partner_returns": (C.c_int, [_DP, vp, C.POINTER(PartnerPriorityDesc), vp]),
     "ia2c_prioritize_partners": (C.c_int, [C.POINTER(PartnerPriorityDesc), i32, f64, i32, vp]),
+    "ia2c_train_episode_frozen": (C.c_int, [_DP, C.POINTER(RunsDesc), C.POINTER(EnvPartnerDesc), C.POINTER(PartnerPriorityDesc),
+                                            C.POINTER(FrozenSeats), vp]),
 }
 
 _lib = None

@@ -150,6 +150,10 @@ class A2COrgTrainer:
         self.inj_actions = torch.as_tensor(a.reshape(self.T + 1, self.R * self.E).astype(np.uint8)).to(self.device)
         self.desc.inj_actions = self.inj_actions.data_ptr()
 
+    def freeze_seats(self, seats):
+        """Refused: the native A2C trainer trains one joint agent, which has no seats to freeze."""
+        raise _lib.IA2CError("A2COrgTrainer trains one joint agent: it has no seats to freeze")
+
     def train_update(self, sync_stats=False):
         """One update of every run in one C call; asynchronous unless ``sync_stats``."""
         self.desc.update = self.update

@@ -21,6 +21,7 @@
 
 namespace ia2c {
 int belief_pairs_episode_runs_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s);   // trainer.cu
+int belief_pairs_episode_seats_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, const TrainedSeats& f, cudaStream_t s);
 namespace {
 
 constexpr int kThreads = 256;
@@ -90,6 +91,7 @@ belief_dense_kernel(const double* __restrict__ filter_action, const double* __re
     }
 }
 
+#ifndef IA2C_BELIEF_SEATS   // the non-template kernels: in belief.cu only
 // Runtime-dimension fallback (M, A <= 8), same operation order.
 __global__ void __launch_bounds__(kThreads)
 belief_dense_generic_kernel(const double* __restrict__ filter_action, const double* __restrict__ lik_in,
@@ -130,6 +132,7 @@ belief_dense_generic_kernel(const double* __restrict__ filter_action, const doub
     }
     ap_out[r] = ap;
 }
+#endif
 
 // ------------------------------------------------------------------------------------------------
 // Packed pairwise update.  A block owns `n_envs` whole envs (small N*K) or one env's agent chunk
@@ -230,6 +233,7 @@ __global__ void __launch_bounds__(kThreads) belief_pairs_kernel(PairsArgs P) {
     }
 }
 
+#ifndef IA2C_BELIEF_SEATS
 __global__ void debug_divide_kernel(const double* __restrict__ a, const double* __restrict__ b, double* __restrict__ q_seq,
                                     double* __restrict__ q_ieee, int64_t n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -237,6 +241,7 @@ __global__ void debug_divide_kernel(const double* __restrict__ a, const double* 
     q_seq[i] = ddiv_seq(a[i], b[i]);
     q_ieee[i] = __ddiv_rn(a[i], b[i]);
 }
+#endif
 
 // ------------------------------------------------------------------------------------------------
 // Table-driven pairwise update for many modelled others (K >= 32).
@@ -752,8 +757,14 @@ constexpr int kEpWarpQuads = 32 * kEpQuads;    // quad slots of a warp: an env's
 // RUNS (FAST only): a batch of independent runs (ia2c_train_episode_runs_many), blockIdx.y = run * N + agent is the filter row; the
 // run's envs are columns [run * E, (run + 1) * E) of an env axis of length R * E, `e0` stays the env's index within the run
 // (Philox counters), and the Philox key is the run's seed, read after the wait.
-template <int M, bool FAST, bool RUNS>
-__global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const __grid_constant__ EpisodePairsArgs P, RunsArg<RUNS> ra) {
+// SEATS: frozen seats (ia2c_train_episode_frozen), grid y still R * N: y < R * L runs trained seat sa.seat[y % L] of run y / L;
+// the blocks beyond it belong to the frozen rows, whose records stay untouched, and only write 0xFF ("no prediction") into
+// their rows of partner_pred.
+// (SEATS_Y: blockIdx.y, or in a SEATS instantiation the row of the full grid a trained row's block works as; trainer.cu has the same)
+#define SEATS_Y (SEATS ? seats_y<RUNS>(N, sa) : blockIdx.y)
+template <int M, bool FAST, bool RUNS, bool SEATS = false>
+__global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const __grid_constant__ EpisodePairsArgs P, RunsArg<RUNS> ra,
+                                                                           const __grid_constant__ SeatsArg<SEATS> sa) {
     static_assert(FAST || !RUNS, "batches have no dumps or tapes");
     constexpr int A = IA2C_AGENT_ACTIONS;
     const double* const u_injected = FAST ? nullptr : P.u_injected;
@@ -761,8 +772,21 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
     uint8_t* const pred_dump = FAST ? nullptr : P.pred_dump;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int queue_n_w[kEpWarps];   // flagged records of the warp's current step
-    const int N = P.N, K = P.K, i = RUNS ? (int)blockIdx.y % N : blockIdx.y;   // i: the agent
-    const int run = RUNS ? (int)blockIdx.y / N : 0;
+    const int N = P.N, K = P.K, i = RUNS ? (int)SEATS_Y % N : SEATS_Y;   // i: the agent
+    const int run = RUNS ? (int)SEATS_Y / N : 0;
+    if constexpr (SEATS) {
+        const int n_runs = RUNS ? (int)gridDim.y / N : 1, L = sa.L;
+        if ((int)blockIdx.y >= n_runs * L) {   // a frozen row: this block's envs, every step
+            pdl_release();
+            pdl_wait();
+            const int y = (int)blockIdx.y - n_runs * L, nf = N - L, seat = sa.seat[L + y % nf];
+            const int64_t col = (int64_t)(y / nf) * P.E, eb = (int64_t)blockIdx.x * kEpWarps * P.envs_per_warp;
+            const int64_t ne = min((int64_t)kEpWarps * P.envs_per_warp, P.E - eb);
+            for (int64_t k = threadIdx.x; k < (int64_t)P.T1 * ne; k += blockDim.x)
+                P.partner_pred[((k / ne) * P.E * n_runs + col + eb + k % ne) * N + seat] = 0xFF;
+            return;
+        }
+    }
     const int KQ = (K + 3) >> 2;
     const int EW = P.envs_per_warp, EWp = (EW + 3) & ~3;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -783,7 +807,7 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
     uint32_t* seen4 = reinterpret_cast<uint32_t*>(queue - warp * (4 * kEpWarpQuads) + 4 * kEpQuads * kThreads);    // [kEpQuads][kThreads] the others' actions
     pdl_release();
     for (int k = threadIdx.x; k <= 100; k += blockDim.x) tab[k] = __ddiv_rn((double)k, 100.0);
-    for (int k = threadIdx.x; k < M * A; k += blockDim.x) fa[k] = P.filter_action[(int64_t)(RUNS ? blockIdx.y : i) * M * A + k];
+    for (int k = threadIdx.x; k < M * A; k += blockDim.x) fa[k] = P.filter_action[(int64_t)(RUNS ? SEATS_Y : i) * M * A + k];
     if (threadIdx.x < kEpWarps) queue_n_w[threadIdx.x] = 0;
     for (int k = threadIdx.x; k < kEpWarps * EWp; k += blockDim.x) (counts - warp * EWp)[k] = 0u;
     __syncthreads();
@@ -1084,6 +1108,8 @@ __global__ void __launch_bounds__(kThreads, 2) belief_pairs_episode_kernel(const
     }
 }
 
+#undef SEATS_Y
+
 // Launch shape of belief_pairs_episode_kernel for P.E envs (of one run): sets P.envs_per_warp, returns the env blocks (grid x)
 // and the dynamic shared memory.  The standalone and the batched launcher share it, so the batch's shared memory always
 // matches what the kernel carves out of it.
@@ -1110,10 +1136,10 @@ int launch_pairs_episode(EpisodePairsArgs& P, cudaStream_t stream) {
     const bool fast = !P.u_injected && !P.belief_dump && !P.pred_dump;
     if (fast) {
         if (smem > 48 * 1024) cudaFuncSetAttribute(belief_pairs_episode_kernel<M, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, true, false>, grid, dim3(kThreads), smem, stream, P, NoRuns{});
+        return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, true, false>, grid, dim3(kThreads), smem, stream, P, NoRuns{}, NoSeats{});
     }
     if (smem > 48 * 1024) cudaFuncSetAttribute(belief_pairs_episode_kernel<M, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, false, false>, grid, dim3(kThreads), smem, stream, P, NoRuns{});
+    return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, false, false>, grid, dim3(kThreads), smem, stream, P, NoRuns{}, NoSeats{});
 }
 
 // The batched form (ia2c_train_episode_runs_many): one run's shape, grid (env blocks of one run, R * N).
@@ -1123,7 +1149,23 @@ int launch_pairs_episode_runs(EpisodePairsArgs& P, const ia2c_runs_desc& runs, c
     dim3 grid((unsigned)sh.env_blocks, (unsigned)(runs.runs * P.N));
     if (sh.smem > 48 * 1024)
         cudaFuncSetAttribute(belief_pairs_episode_kernel<M, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh.smem);
-    return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, true, true>, grid, dim3(kThreads), sh.smem, stream, P, runs);
+    return launch_pdl("belief_pairs_episode_kernel", belief_pairs_episode_kernel<M, true, true>, grid, dim3(kThreads), sh.smem, stream, P, runs, NoSeats{});
+}
+
+// The SEATS forms (ia2c_train_episode_frozen): grid y covers every filter row, trained rows first (belief_pairs_episode_kernel).
+template <int M, bool FAST, bool RUNS>
+int launch_episode_seats(EpisodePairsArgs& P, const RunsArg<RUNS>& ra, int rows, const TrainedSeats& f, cudaStream_t stream) {
+    const EpisodeShape sh = episode_shape<M>(P);
+    auto kernel = belief_pairs_episode_kernel<M, FAST, RUNS, true>;
+    if (sh.smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh.smem);
+    return launch_pdl("belief_pairs_episode_kernel", kernel, dim3((unsigned)sh.env_blocks, (unsigned)rows), dim3(kThreads), sh.smem, stream,
+                      P, ra, f);
+}
+template <int M>
+int launch_pairs_episode_seats(EpisodePairsArgs& P, const ia2c_runs_desc* runs, const TrainedSeats& f, cudaStream_t stream) {
+    if (runs) return launch_episode_seats<M, true, true>(P, *runs, runs->runs * P.N, f, stream);
+    if (!P.u_injected && !P.belief_dump && !P.pred_dump) return launch_episode_seats<M, true, false>(P, NoRuns{}, P.N, f, stream);
+    return launch_episode_seats<M, false, false>(P, NoRuns{}, P.N, f, stream);
 }
 
 template <int M>
@@ -1156,6 +1198,7 @@ int launch_pairs(PairsArgs& P, cudaStream_t stream) {
 }  // namespace
 }  // namespace ia2c
 
+#ifndef IA2C_BELIEF_SEATS   // the entry points: in belief.cu; belief_seats.cu has the frozen-seat launch alone
 using namespace ia2c;
 
 extern "C" int ia2c_belief_update_dense(const double* filter_action, const double* lik, const double* prev,
@@ -1241,3 +1284,26 @@ int ia2c::belief_pairs_episode_runs_launch(const ia2c_episode_desc* d, const ia2
         default: return launch_pairs_episode_runs<6>(P, *runs, s);
     }
 }
+
+#else
+// The whole-episode belief update of a frozen-seat episode (ia2c_train_episode_frozen, which has validated everything): the
+// standalone form of ia2c_belief_update_pairs_episode (runs NULL) or the batched form above, over the trained seats' rows.
+int ia2c::belief_pairs_episode_seats_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, const TrainedSeats& f, cudaStream_t s) {
+    EpisodePairsArgs P{d->belief_records, d->filter_action, d->act, nullptr, nullptr, nullptr, d->partner_pred, d->E, 0, d->N, d->N - 1,
+                       d->T + 1, 0, d->episode, {}};
+    if (!runs) {
+        P.u_injected = d->inj_u_belief, P.pred_dump = d->pred_dump, P.belief_dump = d->belief_dump, P.env_offset = d->env_offset;
+        for (int r = 0; r < 10; ++r) {
+            P.rk[2 * r] = (uint32_t)d->seed + (uint32_t)r * 0x9E3779B9u;
+            P.rk[2 * r + 1] = (uint32_t)(d->seed >> 32) + (uint32_t)r * 0xBB67AE85u;
+        }
+    }
+    switch (d->M) {
+        case 2: return launch_pairs_episode_seats<2>(P, runs, f, s);
+        case 3: return launch_pairs_episode_seats<3>(P, runs, f, s);
+        case 4: return launch_pairs_episode_seats<4>(P, runs, f, s);
+        case 5: return launch_pairs_episode_seats<5>(P, runs, f, s);
+        default: return launch_pairs_episode_seats<6>(P, runs, f, s);
+    }
+}
+#endif

@@ -39,6 +39,7 @@ int actor_pipe_launch(const ia2c_episode_desc* d, cudaStream_t s);
 int reduce_adam_runs_launch(const ReduceArgs& A, const double* lr_per_net, int nets, cudaStream_t s);   // used by a2c.cu
 int64_t actor_pipe_blocks(int64_t E, int N);
 int belief_pairs_episode_runs_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, cudaStream_t s);   // belief.cu
+int belief_pairs_episode_seats_launch(const ia2c_episode_desc* d, const ia2c_runs_desc* runs, const TrainedSeats& f, cudaStream_t s);
 int validate_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p, const char* who);   // partners.cu
 EnvPartners env_partners_arg(const ia2c_env_partner_desc* p);
 int validate_partner_priority(const ia2c_partner_priority_desc* w, const char* who);
@@ -351,22 +352,30 @@ __host__ __device__ inline ChunkPlan chunk_plan(int T, int64_t E, int N) {
     return p;
 }
 
+// blockIdx.y and gridDim.y, or in a SEATS instantiation the row and the rows of the full grid its block works as (seats_y): the
+// kernels without SEATS compile to what they compiled to before frozen seats existed.
+#define SEATS_Y (SEATS ? seats_y<RUNS>(N, sa) : blockIdx.y)
+#define SEATS_GY (SEATS ? seats_gy(N, sa) : gridDim.y)
+
 // partial row layout: P gradient entries then the loss partial.
 // RUNS: a batch of independent runs (ia2c_train_episode_runs_many), laid out as actor_grad_kernel<true> lays them out:
 // blockIdx.y = run * N + agent is the net row, the run's envs are columns [run * E, (run + 1) * E) of an env axis of length R * E.
-template <bool RUNS>
-__global__ void __launch_bounds__(kGradThreads) critic_grad_kernel(ia2c_episode_desc d, float* __restrict__ partials, RunsArg<RUNS> ra) {
+// SEATS: frozen seats (ia2c_train_episode_frozen): blockIdx.y = run * L + k runs trained seat sa.seat[k] of the run, net row
+// run * N + seat, with the net's partition and partial rows of the unfrozen episode.
+template <bool RUNS, bool SEATS = false>
+__global__ void __launch_bounds__(kGradThreads) critic_grad_kernel(ia2c_episode_desc d, float* __restrict__ partials, RunsArg<RUNS> ra,
+                                                                   const __grid_constant__ SeatsArg<SEATS> sa) {
     constexpr int P = kCriticP, GN = F2<J>::G2;   // 148 floats = 74 float2
     __shared__ __align__(16) float w[SmemNet<J>::size];
     __shared__ float red[(kGradThreads / 32) * (P + 1)];
     pdl_prologue();
-    const int N = d.N, n = RUNS ? (int)blockIdx.y % N : blockIdx.y;   // n: the agent
-    const int run = RUNS ? (int)blockIdx.y / N : 0;
-    stage_smemnet<J>(w, d.critic_params + (int64_t)(RUNS ? blockIdx.y : n) * P);
-    if (blockIdx.x == 0 && threadIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.critic_step[RUNS ? blockIdx.y : n] += 1;
+    const int N = d.N, n = RUNS ? (int)SEATS_Y % N : SEATS_Y;   // n: the agent
+    const int run = RUNS ? (int)SEATS_Y / N : 0;
+    stage_smemnet<J>(w, d.critic_params + (int64_t)(RUNS ? SEATS_Y : n) * P);
+    if (blockIdx.x == 0 && threadIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.critic_step[RUNS ? SEATS_Y : n] += 1;
     __syncthreads();
     const int64_t E = d.E, rows = (int64_t)d.T * E;
-    const int64_t ES = RUNS ? E * (gridDim.y / N) : E;
+    const int64_t ES = RUNS ? E * (SEATS_GY / N) : E;
     const ChunkPlan cp = chunk_plan(d.T, E, N);
     const int64_t items = E * cp.n_chunks;
     const float inv_b = 1.f / (float)((int64_t)d.T * d.E_total);
@@ -419,13 +428,14 @@ __global__ void __launch_bounds__(kGradThreads) critic_grad_kernel(ia2c_episode_
     float g[2 * GN];
     unpack_g2(g2, g);
     g[P] = loss;
-    block_reduce_store<P + 1>(reinterpret_cast<float(&)[P + 1]>(g), red, partials + ((int64_t)(RUNS ? blockIdx.y : n) * gridDim.x + blockIdx.x) * (P + 1));
+    block_reduce_store<P + 1>(reinterpret_cast<float(&)[P + 1]>(g), red, partials + ((int64_t)(RUNS ? SEATS_Y : n) * gridDim.x + blockIdx.x) * (P + 1));
 }
 
 // RUNS: a batch of independent runs (ia2c_train_episode_runs): blockIdx.y = run * N + agent is the net row, the run's envs are
-// columns [run * E, (run + 1) * E) of an env axis of length R * E (stride ES).
-template <bool RUNS>
-__global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_desc d, float* __restrict__ partials, RunsArg<RUNS> ra) {
+// columns [run * E, (run + 1) * E) of an env axis of length R * E (stride ES).  SEATS: the trained seats only, as critic_grad_kernel.
+template <bool RUNS, bool SEATS = false>
+__global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_desc d, float* __restrict__ partials, RunsArg<RUNS> ra,
+                                                                  const __grid_constant__ SeatsArg<SEATS> sa) {
     constexpr int P = kActorP, PC = kCriticP, GN = F2<A>::G2;   // 106 floats = 53 float2
     __shared__ __align__(16) float wc[SmemNet<J>::size];
     __shared__ __align__(16) float w[SmemNet<A>::size];
@@ -435,15 +445,15 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
     pdl_prologue();
     KCLOCK(k_waited);
     KSTAMP(g_kclock, 5);
-    const int N = d.N, n = RUNS ? (int)blockIdx.y % N : blockIdx.y;   // n: the agent
-    const int run = RUNS ? (int)blockIdx.y / N : 0;
-    stage_smemnet<J>(wc, d.critic_params + (int64_t)(RUNS ? blockIdx.y : n) * PC);
-    stage_smemnet<A>(w, d.actor_params + (int64_t)(RUNS ? blockIdx.y : n) * P);
-    if (blockIdx.x == 0 && threadIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.actor_step[RUNS ? blockIdx.y : n] += 1;
+    const int N = d.N, n = RUNS ? (int)SEATS_Y % N : SEATS_Y;   // n: the agent
+    const int run = RUNS ? (int)SEATS_Y / N : 0;
+    stage_smemnet<J>(wc, d.critic_params + (int64_t)(RUNS ? SEATS_Y : n) * PC);
+    stage_smemnet<A>(w, d.actor_params + (int64_t)(RUNS ? SEATS_Y : n) * P);
+    if (blockIdx.x == 0 && threadIdx.x == 0 && !(d.flags & IA2C_FLAG_SKIP_ADAM)) d.actor_step[RUNS ? SEATS_Y : n] += 1;
     __syncthreads();
     KCLOCK(k_staged);
     const int64_t E = d.E, rows = (int64_t)d.T * E;
-    const int64_t ES = RUNS ? E * (gridDim.y / N) : E;
+    const int64_t ES = RUNS ? E * (SEATS_GY / N) : E;
     const ChunkPlan cp = chunk_plan(d.T, E, N);
     const int64_t items = E * cp.n_chunks;
     const float inv_b = 1.f / (float)((int64_t)d.T * d.E_total);
@@ -550,12 +560,15 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
     float g[2 * GN];
     unpack_g2(g2, g);
     g[P] = loss;
-    block_reduce_store<P + 1>(reinterpret_cast<float(&)[P + 1]>(g), red, partials + ((int64_t)(RUNS ? blockIdx.y : n) * gridDim.x + blockIdx.x) * (P + 1));
+    block_reduce_store<P + 1>(reinterpret_cast<float(&)[P + 1]>(g), red, partials + ((int64_t)(RUNS ? SEATS_Y : n) * gridDim.x + blockIdx.x) * (P + 1));
     KSTAMP(g_kclock, 7);
     KCLOCK_PRINT(d.episode == 5 && (blockIdx.x == 0 || blockIdx.x == gridDim.x - 1) && blockIdx.y == 0 && threadIdx.x == 0,
                  "actor_grad block %3d entry %llu: waited +%llu, staged +%llu, rows done +%llu, exit +%llu ns\n", (int)blockIdx.x,
                  k_entry % 1000000000ull, k_waited - k_entry, k_staged - k_entry, k_loop_end - k_entry, stage_ns() - k_entry);
 }
+
+#undef SEATS_Y
+#undef SEATS_GY
 
 // Sum partials over blocks (fixed order) -> grad[n][0..P] (slot P = loss); optionally Adam.  (reduce.cuh holds
 // ReduceArgs and the per-entry epilogue with the Adam step.)
@@ -565,13 +578,23 @@ __global__ void __launch_bounds__(kGradThreads) actor_grad_kernel(ia2c_episode_d
 // Everything the update reads is requested right after the wait — the partial rows (every slice), the Adam operands (slice 0)
 // and the step counter (the bias thread) — so the kernel costs one memory round trip before its barrier and none after it.
 // RUNS: the R * N nets of a batch of runs (ia2c_train_episode_runs); net n belongs to run n / N and steps with that run's lr.
-template <bool RUNS>
-__global__ void __launch_bounds__(32 * kReduceSlices) reduce_adam_kernel(ReduceArgs R, ReduceRunsArg<RUNS> rr) {
+// SEATS: frozen seats (ia2c_train_episode_frozen): the grid still covers every net; a frozen net's blocks only write NaN into its
+// loss_out entry (and, after the fused critic stage, which bumps every seat's counter, take that bump back) and return.
+template <bool RUNS, bool SEATS = false>
+__global__ void __launch_bounds__(32 * kReduceSlices) reduce_adam_kernel(ReduceArgs R, ReduceRunsArg<RUNS> rr,
+                                                                         const __grid_constant__ SeatsArg<SEATS> sa) {
     pdl_prologue();
     KSTAMP(g_kclock, R.P == kCriticP ? 0 : 10);
     const int n = blockIdx.x, P = R.P;
     const int col = threadIdx.x & 31, slice = threadIdx.x >> 5;
     const int i = blockIdx.y * 32 + col;
+    if constexpr (SEATS) {
+        if (seat_frozen(sa, n % sa.N)) {
+            if (slice == 0 && i == P) R.loss_out[n] = __int_as_float(0x7fc00000);
+            if (sa.undo_step && blockIdx.y == 0 && threadIdx.x == 0) R.step[n] -= 1;
+            return;
+        }
+    }
     __shared__ float part[kReduceSlices][33];
     __shared__ AdamBias bias;
     const bool bias_thread = threadIdx.x == blockDim.x - 1 && R.apply_adam;
@@ -673,10 +696,15 @@ static bool actor_columns(const ia2c_episode_desc* d) { return d->flags & IA2C_F
 static int actor_partial_blocks(const ia2c_episode_desc* d) {
     return actor_columns(d) ? grad_blocks(d) : (int)actor_pipe_blocks(d->E, d->N);
 }
-static int launch_actor_grad(const ia2c_episode_desc* d, cudaStream_t s) {
+// f != nullptr: frozen seats, the trained seats' rows only (ia2c_train_episode_frozen has checked for the column kernel)
+static int launch_actor_grad(const ia2c_episode_desc* d, cudaStream_t s, const TrainedSeats* f = nullptr) {
+    if (f) {
+        return launch_pdl("actor_grad_kernel", actor_grad_kernel<false, true>, dim3(grad_blocks(d), f->L), dim3(kGradThreads), 0, s, *d,
+                          d->partials, NoRuns{}, *f);
+    }
     if (!actor_columns(d)) return actor_pipe_launch(d, s);
     dim3 grid(grad_blocks(d), d->N);
-    return launch_pdl("actor_grad_kernel", actor_grad_kernel<false>, grid, dim3(kGradThreads), 0, s, *d, d->partials, NoRuns{});
+    return launch_pdl("actor_grad_kernel", actor_grad_kernel<false>, grid, dim3(kGradThreads), 0, s, *d, d->partials, NoRuns{}, NoSeats{});
 }
 
 extern "C" size_t ia2c_episode_partials_floats(const ia2c_episode_desc* d) {
@@ -703,7 +731,8 @@ static int check_rollout(const ia2c_episode_desc* d, const char* who) {
 }
 
 // The rollout of ia2c_rollout; p != nullptr: the PARTNERS instantiations (the path was checked by validate_env_partners).
-static int rollout_launch(const ia2c_episode_desc* d, const EnvPartners* p, void* stream) {
+// f != nullptr: frozen seats, whose rows the whole-episode belief kernel skips (N <= 8: the fused rollout is unchanged).
+static int rollout_launch(const ia2c_episode_desc* d, const EnvPartners* p, void* stream, const TrainedSeats* f = nullptr) {
     cudaStream_t s = as_stream(stream);
     if (d->flags & IA2C_FLAG_FUSED_ROLLOUT) return rollout_fused_launch(d, nullptr, p, s);
     const bool episode_beliefs = !(d->flags & IA2C_FLAG_BELIEF_PER_STEP) && ia2c_belief_supports_episode(d->N, d->M);
@@ -715,6 +744,7 @@ static int rollout_launch(const ia2c_episode_desc* d, const EnvPartners* p, void
                          : launch_pdl("rollout_many_kernel", rollout_many_kernel<false>, dim3((unsigned)mp.blocks), dim3(mp.threads),
                                       mp.smem, s, *d, mp.envs_per_block, NoRuns{}, NoPartners{});
         if (rc) return rc;
+        if (f) return belief_pairs_episode_seats_launch(d, nullptr, *f, s);
         return ia2c_belief_update_pairs_episode(d->belief_records, d->filter_action, d->act, d->inj_u_belief, d->pred_dump, d->belief_dump,
                                                 d->partner_pred, d->E, d->N, d->M, d->T + 1, d->seed, d->episode, d->env_offset, stream);
     }
@@ -759,7 +789,8 @@ extern "C" int ia2c_rollout(const ia2c_episode_desc* d, void* stream) {
     return rollout_launch(d, nullptr, stream);
 }
 
-static int run_reduce(const ia2c_episode_desc* d, int which, int from_partials, int apply, cudaStream_t s) {
+// f != nullptr: frozen seats (ia2c_train_episode_frozen), the SEATS instantiation over all N rows.
+static int run_reduce(const ia2c_episode_desc* d, int which, int from_partials, int apply, cudaStream_t s, const TrainedSeats* f = nullptr) {
     ReduceArgs R = make_reduce_args(*d, which, which == 0 ? critic_partial_blocks(d) : actor_partial_blocks(d));
     R.apply_adam = apply;
     R.from_partials = from_partials;
@@ -768,7 +799,12 @@ static int run_reduce(const ia2c_episode_desc* d, int which, int from_partials, 
         if (int rc = check_launch("bump_steps_kernel")) return rc;
     }
     dim3 grid(d->N, ceil_div(R.P + 1, 32));
-    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<false>, grid, dim3(32 * kReduceSlices), 0, s, R, NoRuns{});
+    if (f) {
+        TrainedSeats g = *f;
+        g.undo_step = which == 0 && fused_critic(d);
+        return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<false, true>, grid, dim3(32 * kReduceSlices), 0, s, R, NoRuns{}, g);
+    }
+    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<false>, grid, dim3(32 * kReduceSlices), 0, s, R, NoRuns{}, NoSeats{});
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -932,25 +968,37 @@ static int check_update_ptrs(const ia2c_episode_desc* d, const char* who) {
     return 0;
 }
 
+// The launches of the critic / actor phase; f != nullptr: frozen seats (the caller has checked everything).
+static int critic_phase_launch(const ia2c_episode_desc* d, cudaStream_t s, const TrainedSeats* f = nullptr) {
+    if (!fused_critic(d)) {   // otherwise the rollout kernel's critic stage already wrote the partials
+        if (f) {
+            if (int rc = launch_pdl("critic_grad_kernel", critic_grad_kernel<false, true>, dim3(grad_blocks(d), f->L), dim3(kGradThreads), 0, s,
+                                    *d, d->partials, NoRuns{}, *f)) return rc;
+        } else {
+            dim3 grid(grad_blocks(d), d->N);
+            if (int rc = launch_pdl("critic_grad_kernel", critic_grad_kernel<false>, grid, dim3(kGradThreads), 0, s, *d, d->partials, NoRuns{}, NoSeats{})) return rc;
+        }
+    }
+    if (d->flags & IA2C_FLAG_GRAD_ONLY) return 0;
+    return run_reduce(d, 0, 1, !(d->flags & IA2C_FLAG_SKIP_ADAM), s, f);
+}
+
+static int actor_phase_launch(const ia2c_episode_desc* d, cudaStream_t s, const TrainedSeats* f = nullptr) {
+    if (int rc = launch_actor_grad(d, s, f)) return rc;
+    if (d->flags & IA2C_FLAG_GRAD_ONLY) return 0;
+    return run_reduce(d, 1, 1, !(d->flags & IA2C_FLAG_SKIP_ADAM), s, f);
+}
+
 extern "C" int ia2c_critic_phase(const ia2c_episode_desc* d, void* stream) {
     if (int rc = validate(d, "ia2c_critic_phase")) return rc;
     if (int rc = check_update_ptrs(d, "ia2c_critic_phase")) return rc;
-    cudaStream_t s = as_stream(stream);
-    if (!fused_critic(d)) {   // otherwise the rollout kernel's critic stage already wrote the partials
-        dim3 grid(grad_blocks(d), d->N);
-        if (int rc = launch_pdl("critic_grad_kernel", critic_grad_kernel<false>, grid, dim3(kGradThreads), 0, s, *d, d->partials, NoRuns{})) return rc;
-    }
-    if (d->flags & IA2C_FLAG_GRAD_ONLY) return 0;
-    return run_reduce(d, 0, 1, !(d->flags & IA2C_FLAG_SKIP_ADAM), s);
+    return critic_phase_launch(d, as_stream(stream));
 }
 
 extern "C" int ia2c_actor_phase(const ia2c_episode_desc* d, void* stream) {
     if (int rc = validate(d, "ia2c_actor_phase")) return rc;
     if (int rc = check_update_ptrs(d, "ia2c_actor_phase")) return rc;
-    cudaStream_t s = as_stream(stream);
-    if (int rc = launch_actor_grad(d, s)) return rc;
-    if (d->flags & IA2C_FLAG_GRAD_ONLY) return 0;
-    return run_reduce(d, 1, 1, !(d->flags & IA2C_FLAG_SKIP_ADAM), s);
+    return actor_phase_launch(d, as_stream(stream));
 }
 
 extern "C" int ia2c_apply_adam(const ia2c_episode_desc* d, int32_t which, void* stream) {
@@ -960,11 +1008,12 @@ extern "C" int ia2c_apply_adam(const ia2c_episode_desc* d, int32_t which, void* 
     return run_reduce(d, which, 0, 1, as_stream(stream));
 }
 
-// One standalone episode; p != nullptr: with frozen partners per env (the caller checked everything before the first CUDA call).
-static int train_episode_impl(const ia2c_episode_desc* d, const EnvPartners* p, void* stream) {
-    if (int rc = p ? rollout_launch(d, p, stream) : ia2c_rollout(d, stream)) return rc;
-    if (int rc = ia2c_critic_phase(d, stream)) return rc;
-    return ia2c_actor_phase(d, stream);
+// One standalone episode; p != nullptr: with frozen partners per env, f != nullptr: with frozen seats (for both the caller
+// checked everything before the first CUDA call).
+static int train_episode_impl(const ia2c_episode_desc* d, const EnvPartners* p, void* stream, const TrainedSeats* f = nullptr) {
+    if (int rc = (p || f) ? rollout_launch(d, p, stream, f) : ia2c_rollout(d, stream)) return rc;
+    if (int rc = f ? critic_phase_launch(d, as_stream(stream), f) : ia2c_critic_phase(d, stream)) return rc;
+    return f ? actor_phase_launch(d, as_stream(stream), f) : ia2c_actor_phase(d, stream);
 }
 
 extern "C" int ia2c_train_episode(const ia2c_episode_desc* d, void* stream) { return train_episode_impl(d, nullptr, stream); }
@@ -1233,7 +1282,7 @@ extern "C" int ia2c_train_episode_timed(const ia2c_episode_desc* d, float* host_
     cudaEventRecord(ev[0], s);
     rc = ia2c_rollout(d, stream);
     cudaEventRecord(ev[1], s);
-    if (!rc && !fused_critic(d)) { critic_grad_kernel<false><<<grid, kGradThreads, 0, s>>>(*d, d->partials, NoRuns{}); rc = check_launch("critic_grad_kernel"); }
+    if (!rc && !fused_critic(d)) { critic_grad_kernel<false><<<grid, kGradThreads, 0, s>>>(*d, d->partials, NoRuns{}, NoSeats{}); rc = check_launch("critic_grad_kernel"); }
     cudaEventRecord(ev[2], s);
     if (!rc) rc = run_reduce(d, 0, 1, apply, s);
     cudaEventRecord(ev[3], s);
@@ -1326,27 +1375,38 @@ static int validate_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r) {
 }
 
 // reduce + Adam of a batch's R * N critics (which = 0) or actors (1), each net with its run's learning rate; `e` carries the
-// internal flags, which select the partial-row count of the producing kernel
-static int reduce_runs(const ia2c_episode_desc& e, const ia2c_runs_desc* r, int which, cudaStream_t s) {
+// internal flags, which select the partial-row count of the producing kernel; f != nullptr: frozen seats
+static int reduce_runs(const ia2c_episode_desc& e, const ia2c_runs_desc* r, int which, cudaStream_t s, const TrainedSeats* f) {
     const int nets = r->runs * e.N;
     ReduceArgs A = make_reduce_args(e, which, which == 0 ? critic_partial_blocks(&e) : actor_partial_blocks(&e));
     A.loss_out = e.loss_out + (which == 0 ? 0 : nets);
     const ReduceRuns rr = {which == 0 ? r->lr_critic : r->lr_actor, e.N};
     dim3 grid(nets, ceil_div(A.P + 1, 32));
-    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr);
+    if (f) {
+        TrainedSeats g = *f;
+        g.undo_step = which == 0 && fused_critic(&e);
+        return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true, true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr, g);
+    }
+    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr, NoSeats{});
 }
 
-// One episode of a batch (N <= 8); p != nullptr: with frozen partners per env.
-static int train_runs_impl(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const EnvPartners* p, void* stream) {
+// One episode of a batch (N <= 8); p != nullptr: with frozen partners per env, f != nullptr: with frozen seats.
+static int train_runs_impl(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const EnvPartners* p, void* stream,
+                           const TrainedSeats* f = nullptr) {
     cudaStream_t s = as_stream(stream);
     const int R = r->runs, nets = R * d->N;
     ia2c_episode_desc e = *d;
     e.flags = IA2C_FLAG_FUSED_ROLLOUT | IA2C_FLAG_FUSED_CRITIC | IA2C_FLAG_ACTOR_COLUMNS;
     if (int rc = rollout_fused_launch(&e, r, p, s)) return rc;
-    if (int rc = reduce_runs(e, r, 0, s)) return rc;
-    dim3 grid(grad_blocks(&e), nets);
-    if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
-    return reduce_runs(e, r, 1, s);
+    if (int rc = reduce_runs(e, r, 0, s, f)) return rc;
+    if (f) {
+        if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true, true>, dim3(grad_blocks(&e), R * f->L), dim3(kGradThreads), 0, s,
+                                e, e.partials, *r, *f)) return rc;
+    } else {
+        dim3 grid(grad_blocks(&e), nets);
+        if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r, NoSeats{})) return rc;
+    }
+    return reduce_runs(e, r, 1, s, f);
 }
 
 extern "C" int ia2c_train_episode_runs(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream) {
@@ -1394,8 +1454,9 @@ static int validate_runs_many(const ia2c_episode_desc* d, const ia2c_runs_desc* 
     return 0;
 }
 
-// One episode of a batch (9 <= N <= 256); p != nullptr: with frozen partners per env.
-static int train_runs_many_impl(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const EnvPartners* p, void* stream) {
+// One episode of a batch (9 <= N <= 256); p != nullptr: with frozen partners per env, f != nullptr: with frozen seats.
+static int train_runs_many_impl(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const EnvPartners* p, void* stream,
+                                const TrainedSeats* f = nullptr) {
     cudaStream_t s = as_stream(stream);
     const int R = r->runs, nets = R * d->N;
     ia2c_episode_desc e = *d;
@@ -1407,12 +1468,20 @@ static int train_runs_many_impl(const ia2c_episode_desc* d, const ia2c_runs_desc
                    : launch_pdl("rollout_many_kernel", rollout_many_kernel<true>, many_grid, dim3(mp.threads), mp.smem, s, e,
                                 mp.envs_per_block, *r, NoPartners{}))
         return rc;
+    if (f) {
+        const dim3 grid(grad_blocks(&e), R * f->L);
+        if (int rc = belief_pairs_episode_seats_launch(&e, r, *f, s)) return rc;
+        if (int rc = launch_pdl("critic_grad_kernel", critic_grad_kernel<true, true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r, *f)) return rc;
+        if (int rc = reduce_runs(e, r, 0, s, f)) return rc;
+        if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true, true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r, *f)) return rc;
+        return reduce_runs(e, r, 1, s, f);
+    }
     if (int rc = belief_pairs_episode_runs_launch(&e, r, s)) return rc;
     const dim3 grid(grad_blocks(&e), nets);
-    if (int rc = launch_pdl("critic_grad_kernel", critic_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
-    if (int rc = reduce_runs(e, r, 0, s)) return rc;
-    if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r)) return rc;
-    return reduce_runs(e, r, 1, s);
+    if (int rc = launch_pdl("critic_grad_kernel", critic_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r, NoSeats{})) return rc;
+    if (int rc = reduce_runs(e, r, 0, s, nullptr)) return rc;
+    if (int rc = launch_pdl("actor_grad_kernel", actor_grad_kernel<true>, grid, dim3(kGradThreads), 0, s, e, e.partials, *r, NoSeats{})) return rc;
+    return reduce_runs(e, r, 1, s, nullptr);
 }
 
 extern "C" int ia2c_train_episode_runs_many(const ia2c_episode_desc* d, const ia2c_runs_desc* r, void* stream) {
@@ -1453,9 +1522,9 @@ extern "C" int ia2c_rollout_env_partners_prioritized(const ia2c_episode_desc* d,
     return rollout_launch(d, &ep, stream);
 }
 
-// The uniform per-env episode, or (w != nullptr) the prioritized one drawing from w->table.
+// The uniform per-env episode, or (w != nullptr) the prioritized one drawing from w->table; f != nullptr: with frozen seats.
 static int train_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
-                              const ia2c_partner_priority_desc* w, const char* who, void* stream) {
+                              const ia2c_partner_priority_desc* w, const char* who, void* stream, const TrainedSeats* f = nullptr) {
     if (int rc = validate_env_partners(d, r, p, who)) return rc;
     EnvPartners ep = env_partners_arg(p);
     if (w) {
@@ -1465,14 +1534,14 @@ static int train_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* 
     if (!r) {
         if (int rc = check_rollout(d, who)) return rc;
         if (int rc = check_update_ptrs(d, who)) return rc;
-        return train_episode_impl(d, &ep, stream);
+        return train_episode_impl(d, &ep, stream, f);
     }
     if (d->N <= 8) {
         if (int rc = validate_runs(d, r)) return rc;
-        return train_runs_impl(d, r, &ep, stream);
+        return train_runs_impl(d, r, &ep, stream, f);
     }
     if (int rc = validate_runs_many(d, r)) return rc;
-    return train_runs_many_impl(d, r, &ep, stream);
+    return train_runs_many_impl(d, r, &ep, stream, f);
 }
 
 extern "C" int ia2c_train_episode_env_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
@@ -1488,12 +1557,66 @@ extern "C" int ia2c_train_episode_env_partners_prioritized(const ia2c_episode_de
     return train_env_partners(d, r, p, w, who, stream);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Frozen seats (include/ia2c_b200.h: ia2c_train_episode_frozen): the entry points above with the SEATS instantiations of the
+// gradient, reduce and whole-episode belief kernels.  Everything is checked here, before the first CUDA call; the trained seats'
+// list goes to the kernels by value.
+extern "C" int ia2c_train_episode_frozen(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
+                                         const ia2c_partner_priority_desc* w, const ia2c_frozen_seats* f, void* stream) {
+    const char* who = "ia2c_train_episode_frozen";
+    if (int rc = validate(d, who)) return rc;
+    IA2C_REQUIRE(f != nullptr, "%s: null frozen-seat mask", who);
+    IA2C_REQUIRE(!w || p, "%s: prioritized draws (w) need the per-env pool (p)", who);
+    auto unsupported = [](const char* what, const char* who) {
+        set_error("%s: %s", who, what);
+        return IA2C_ERR_UNSUPPORTED;
+    };
+    const int N = d->N;
+    if (N > 256) return unsupported("N above 256 runs the per-step rollout, which has no frozen-seat kernels", who);
+    TrainedSeats ts = {};
+    ts.N = N;
+    int frozen = 0;
+    for (int k = 0; k < 4; ++k) {
+        ts.mask[k] = f->mask[k];
+        const uint64_t beyond = k * 64 >= N ? ~0ull : (N - k * 64 >= 64 ? 0ull : ~0ull << (N - k * 64));
+        IA2C_REQUIRE(!(f->mask[k] & beyond), "%s: mask[%d] = 0x%llx has a seat at or above N = %d", who, k, (unsigned long long)f->mask[k], N);
+        frozen += __builtin_popcountll(f->mask[k]);
+    }
+    IA2C_REQUIRE(frozen >= 1 && frozen <= N - 1, "%s: %d of %d seats frozen: at least one seat must be frozen and one trained", who,
+                 frozen, N);
+    ts.L = N - frozen;
+    for (int n = 0, a = 0, b = ts.L; n < N; ++n) ts.seat[seat_frozen(ts, n) ? b++ : a++] = (uint16_t)n;
+    if (d->flags & (IA2C_FLAG_SKIP_ADAM | IA2C_FLAG_GRAD_ONLY))
+        return unsupported("SKIP_ADAM / GRAD_ONLY: frozen seats train on one GPU, with the Adam step of every episode", who);
+    if (d->env_offset != 0 || d->E_total != d->E)
+        return unsupported("frozen seats train on one GPU: desc.env_offset must be 0 and desc.E_total == desc.E", who);
+    if (d->flags & (IA2C_FLAG_ROLLOUT_PER_STEP | IA2C_FLAG_BELIEF_PER_STEP))
+        return unsupported("the per-step rollout and belief kernels (ROLLOUT_PER_STEP, BELIEF_PER_STEP) have no frozen-seat form", who);
+    if (N <= 8 && (!rollout_fused_supported(N, d->M) || (!r && !(d->flags & IA2C_FLAG_FUSED_ROLLOUT))))
+        return unsupported("N <= 8 needs the fused rollout (IA2C_FLAG_FUSED_ROLLOUT and N <= 8 with M = 5, or N = 2 with M = 3)", who);
+    if (N > 8 && !ia2c_belief_supports_episode(N, d->M)) return unsupported("no whole-episode belief kernel for this (N, M)", who);
+    if (!(d->flags & IA2C_FLAG_ACTOR_COLUMNS))
+        return unsupported("the pipelined actor kernel has no frozen-seat form: set IA2C_FLAG_ACTOR_COLUMNS (actor_kernel=\"columns\")", who);
+    if (p) return train_env_partners(d, r, p, w, who, stream, &ts);
+    if (!r) {
+        if (int rc = check_rollout(d, who)) return rc;
+        if (int rc = check_update_ptrs(d, who)) return rc;
+        return train_episode_impl(d, nullptr, stream, &ts);
+    }
+    if (N <= 8) {
+        if (int rc = validate_runs(d, r)) return rc;
+        return train_runs_impl(d, r, nullptr, stream, &ts);
+    }
+    if (int rc = validate_runs_many(d, r)) return rc;
+    return train_runs_many_impl(d, r, nullptr, stream, &ts);
+}
+
 // reduce_adam_kernel<true> for `nets` nets of P entries with one learning rate per net (lr_per_net, or A.lr where NULL): the
 // native A2C trainer (a2c.cu) reduces and steps its R actor and R critic rows with it.
 int ia2c::reduce_adam_runs_launch(const ReduceArgs& A, const double* lr_per_net, int nets, cudaStream_t s) {
     const ReduceRuns rr = {lr_per_net, 1};
     const dim3 grid(nets, ceil_div(A.P + 1, 32));
-    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr);
+    return launch_pdl("reduce_adam_kernel", reduce_adam_kernel<true>, grid, dim3(32 * kReduceSlices), 0, s, A, rr, NoSeats{});
 }
 
 #ifdef IA2C_STAGE_CLOCKS

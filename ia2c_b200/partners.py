@@ -20,6 +20,11 @@ seats' own actor rows are not used to act while the mode is on; they still recei
 episode one more launch adds each env's return to its run's statistics for the team it played (``ia2c_record_partner_returns``),
 and ``prioritize_partners`` rebuilds every run's weight table from them in one launch (``ia2c_prioritize_partners``), giving
 the teams a run does worst with the largest weights.  ``partner_returns`` and ``partner_weights`` read both back.
+
+``freeze_seats(seats)`` freezes seats of every run (``ia2c_train_episode_frozen``): a frozen seat still acts, with its own
+actor row, a seated pool row or its env's pool row, but nothing of it is updated and the update kernels skip it.
+``freeze_seats(pool.seats)`` trains against truly frozen partners in every partner mode; without a pool it trains a best
+response to fixed co-players.
 """
 from __future__ import annotations
 
@@ -139,12 +144,78 @@ class SeatsPartners:
     _env_partners = False       # per-env mode
     _env_partner_log = None
     _priority = None            # prioritized per-env mode: {"count", "sum", "table"} device tensors and "desc"
+    _frozen = frozenset()       # frozen seats
+    _frozen_desc = None
 
     def _check_partners(self):
         """Raise, before any device work, where partners cannot be seated."""
 
     def _check_env_partners(self):
         """Raise, before any device work, where partners cannot be played per env."""
+
+    def _check_frozen(self):
+        """Raise, before any device work, where seats cannot be frozen."""
+
+    def freeze_seats(self, seats):
+        """Freeze ``seats`` (seat indices in [0, n_agents), the same for every run; at least one frozen and one trained) in
+        every episode that ``train_episode`` and ``train_episodes`` start, or train every seat again with ``None``.  A frozen
+        seat acts as before (its own actor row, the row a pool seats in it, or its env's pool row in the per-env mode), but
+        its parameters, gradients, Adam moments and steps and actor gradient sum stay byte for byte as they are, its
+        ``loss_out`` entries are NaN, and the gradient and reduce kernels do not run its rows.  Up to 8 agents the fused
+        rollout still runs every seat's belief filter; from 9 agents the belief kernel skips frozen seats, whose belief
+        records stay as they are and whose partner predictions read 0xFF ("no prediction", so ``history()`` counts no hit).
+        A trained seat's every byte is what the episode computes with nothing frozen, and run r of a batch equals a
+        standalone trainer with its seed, pool, partner mode and frozen set.  Launches per episode are unchanged.  Refused,
+        before any device work, off the whole-episode kernel paths (see ``_check_frozen``); ``rollout`` / ``update``, the
+        host-tape pipelines and ``train_episode_timed`` refuse to run while seats are frozen."""
+        if seats is None:
+            self._frozen, self._frozen_desc = frozenset(), None
+            return
+        fs = self._frozen_set(seats)
+        f = _lib.FrozenSeats()
+        for x in fs:
+            f.mask[x >> 6] |= 1 << (x & 63)
+        self._frozen, self._frozen_desc = fs, f
+
+    def _frozen_set(self, seats):
+        """``seats`` (a set, sequence, array or tensor of seat indices, e.g. ``pool.seats``) as a frozenset, after every check
+        of ``freeze_seats``; raises before any device work."""
+        if isinstance(seats, (int, np.integer)):
+            raise ValueError("freeze_seats: pass a set of seats, e.g. freeze_seats({1})")
+        if not isinstance(seats, (torch.Tensor, np.ndarray)):
+            seats = np.asarray(list(seats), dtype=np.int64)
+        fs = frozenset(int(x) for x in _host_ints(seats, "seats").reshape(-1))
+        if any(not 0 <= x < self.N for x in fs):
+            raise ValueError(f"freeze_seats: seats {sorted(fs)} outside [0, {self.N})")
+        if not 1 <= len(fs) <= self.N - 1:
+            raise ValueError(f"freeze_seats: {len(fs)} of {self.N} seats: at least one seat must be frozen and one trained")
+        self._check_frozen()
+        return fs
+
+    def _check_frozen_state(self, sd):
+        """Raise, before a checkpoint's tensors are copied, if its frozen seats cannot be frozen here."""
+        if sd.get("frozen_seats"):
+            self._frozen_set(sd["frozen_seats"])
+
+    @property
+    def frozen_seats(self):
+        """The frozen seats (a frozenset, empty while every seat trains)."""
+        return self._frozen
+
+    def _refuse_frozen(self, what):
+        if self._frozen:
+            raise _lib.IA2CError(f"{what} does not freeze seats: call freeze_seats(None) first")
+
+    def _enqueue_frozen(self, desc_ref, runs_ref, stream):
+        """Enqueue one training episode with the frozen seats, in the partner mode that is set."""
+        f, name = C.byref(self._frozen_desc), "ia2c_train_episode_frozen"
+        if self._env_partners:
+            self._play_env_partners(lambda p: self.lib.ia2c_train_episode_frozen(desc_ref, runs_ref, p, None, f, stream), name,
+                                    lambda p, w: self.lib.ia2c_train_episode_frozen(desc_ref, runs_ref, p, w, f, stream),
+                                    desc_ref, stream)
+            return
+        self._seat_partners(stream)
+        _lib.check(self.lib.ia2c_train_episode_frozen(desc_ref, runs_ref, None, None, f, stream), name)
 
     def set_partners(self, pool, per_env=False, prioritized=False):
         """Seat partners from ``pool`` (a ``PartnerPool`` of this trainer's n_agents and device) before every episode that
@@ -329,7 +400,10 @@ class SeatsPartners:
         return dict(episode=ep, team=team[:, 0] if runs_ref is None else team)
 
     def _partner_state(self, sd, run=None):
-        """Add the pool, the mode and the prioritized statistics and table (all runs', or run ``run``'s alone) to ``sd``."""
+        """Add the pool, the mode and the prioritized statistics and table (all runs', or run ``run``'s alone) and the frozen
+        seats to ``sd``."""
+        if self._frozen:
+            sd["frozen_seats"] = sorted(self._frozen)
         if self._partners is not None:
             sd["partners"] = self._partners.state()
             sd["partners_per_env"] = self._env_partners
@@ -340,7 +414,8 @@ class SeatsPartners:
 
     def _load_partner_state(self, sd):
         """Restore the pool, mode and prioritized statistics a checkpoint carries (a checkpoint without the mode is
-        per-episode, one without statistics is uniform), or clear the pool for one without."""
+        per-episode, one without statistics is uniform), or clear the pool for one without; then the frozen seats (none
+        for a checkpoint without them)."""
         part = sd.get("partners")
         prio = sd.get("partner_priority") if part is not None else None
         if prio is not None:
@@ -354,3 +429,4 @@ class SeatsPartners:
         if prio is not None:
             for k in ("count", "sum", "table"):
                 self._priority[k].copy_(prio[k])
+        self.freeze_seats(sd.get("frozen_seats"))

@@ -18,7 +18,8 @@ hyper-parameters; ``pbt_history`` reads back what each generation did.
 ``set_partners`` (ia2c_b200/partners.py) seats frozen partners from a pool in every run's partner seats before each episode
 (``ia2c_seat_partners``): each run draws a team from its own training seed, so run r still equals a standalone trainer with
 the same seed and pool.  ``set_partners(pool, per_env=True)`` draws a team per env inside the rollout kernels instead
-(``ia2c_train_episode_env_partners``), with the same rule.
+(``ia2c_train_episode_env_partners``), with the same rule.  ``freeze_seats`` freezes the same seats in every run
+(``ia2c_train_episode_frozen``).
 """
 from __future__ import annotations
 
@@ -167,6 +168,9 @@ class IA2CRuns(SeatsPartners, RecordsHistory):
         return self.R, C.byref(self.runs_desc)
 
     def _enqueue_episode(self, desc_ref, stream):
+        if self._frozen:
+            self._enqueue_frozen(desc_ref, C.byref(self.runs_desc), stream)
+            return
         if self._env_partners:
             runs = C.byref(self.runs_desc)
             self._play_env_partners(lambda p: self.lib.ia2c_train_episode_env_partners(desc_ref, runs, p, stream),
@@ -235,6 +239,7 @@ class IA2CRuns(SeatsPartners, RecordsHistory):
         counts only episodes recorded after the load."""
         if tuple(sd["dims"]) != (self.R, self.E, self.N, self.M, self.T):
             raise ValueError(f"checkpoint is for (runs, E, N, M, T) = {tuple(sd['dims'])}, batch has {(self.R, self.E, self.N, self.M, self.T)}")
+        self._check_frozen_state(sd)   # a set this object cannot freeze is refused before anything is copied
         for k in IA2CTrainer._CKPT_TENSORS:
             getattr(self, k).copy_(sd[k])
         self.episode = int(sd["episode"])

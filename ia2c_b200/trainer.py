@@ -235,6 +235,7 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         return torch.cuda.current_stream(self.device).cuda_stream
 
     def rollout(self):
+        self._refuse_frozen("rollout")
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):
             s = self._stream()
@@ -247,6 +248,7 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
             _lib.check(self.lib.ia2c_rollout(C.byref(self.desc), s), "ia2c_rollout")
 
     def update(self):
+        self._refuse_frozen("update")
         d, s = C.byref(self.desc), self._stream()
         with torch.cuda.device(self.device):
             if self.p2p:
@@ -302,6 +304,9 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         return 1, self.N, self.E, self.T, True
 
     def _enqueue_episode(self, desc_ref, stream):
+        if self._frozen:
+            self._enqueue_frozen(desc_ref, None, stream)
+            return
         if self._env_partners:
             self._play_env_partners(lambda p: self.lib.ia2c_train_episode_env_partners(desc_ref, None, p, stream),
                                     "ia2c_train_episode_env_partners",
@@ -328,6 +333,23 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
             raise _lib.IA2CError("set_partners(per_env=True): the per-step rollout (rollout_kernel='step', belief_kernel='step' "
                                  "or no whole-episode belief kernel) has no per-env kernels")
 
+    def _check_frozen(self):
+        """The paths with whole-episode kernels and the column actor kernel, on one GPU."""
+        N, M, flags = self.N, self.M, self.desc.flags
+        if self.world > 1:
+            raise _lib.IA2CError("freeze_seats trains on one GPU (a rank sees only its env shard)")
+        if N > 256:
+            raise _lib.IA2CError(f"freeze_seats: n_agents={N} above 256 runs the per-step rollout, which has no frozen-seat kernels")
+        if N <= 8 and not flags & _lib.FLAG_FUSED_ROLLOUT:
+            raise _lib.IA2CError(f"freeze_seats: n_agents={N}, n_models={M} runs the per-step rollout "
+                                 "(fused_rollout=False or no fused instantiation), which has no frozen-seat kernels")
+        if N > 8 and (flags & (_lib.FLAG_ROLLOUT_PER_STEP | _lib.FLAG_BELIEF_PER_STEP) or not self.lib.ia2c_belief_supports_episode(N, M)):
+            raise _lib.IA2CError("freeze_seats: the per-step rollout (rollout_kernel='step', belief_kernel='step' or no "
+                                 "whole-episode belief kernel) has no frozen-seat kernels")
+        if not flags & _lib.FLAG_ACTOR_COLUMNS:
+            raise _lib.IA2CError('freeze_seats: the pipelined actor kernel has no frozen-seat form: build the trainer with '
+                                 'actor_kernel="columns"')
+
     def _partner_runs(self):
         return 1, None
 
@@ -337,6 +359,7 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         if self.world > 1:
             raise _lib.IA2CError("train_episode_host is the single-rank entry point")
         self._refuse_partners("train_episode_host")
+        self._refuse_frozen("train_episode_host")
         if self.inj_u_action is None or self.inj_u_belief is None:
             T, E, N, K = self.T, self.E, self.N, self.K
             self.inject(u_action=torch.zeros(T + 1, E, N), u_belief=torch.zeros(T + 1, E, N, K, dtype=torch.float64))
@@ -387,6 +410,7 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         losses and returns out (the loss / return windows are updated; ``window_stats()`` computes their means on demand).  One H2D copy per episode, overlapping the previous episode's compute, and one D2H
         copy of the result region (``ia2c_train_episodes_host``; multi-rank: the same pipeline with torch streams)."""
         self._refuse_partners("train_episodes_host")
+        self._refuse_frozen("train_episodes_host")
         n = len(host_tapes)
         N, E = self.N, self.E
         self._ensure_stage()
@@ -477,6 +501,7 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         if self.world > 1:
             raise _lib.IA2CError("train_episode_timed is the single-rank profiling entry point")
         self._refuse_env_partners("train_episode_timed")
+        self._refuse_frozen("train_episode_timed")
         ms = (C.c_float * 5)()
         self.desc.episode = self.episode
         with torch.cuda.device(self.device):
@@ -550,6 +575,7 @@ class IA2CTrainer(SeatsPartners, RecordsHistory):
         if tuple(sd["dims"]) != (self.E_total, self.E, self.N, self.M, self.T) or sd["world"] != self.world:
             raise ValueError(f"checkpoint is for dims/world {sd['dims']}/{sd['world']}, "
                              f"trainer has {(self.E_total, self.E, self.N, self.M, self.T)}/{self.world}")
+        self._check_frozen_state(sd)   # a set this object cannot freeze is refused before anything is copied
         for k in self._CKPT_TENSORS:
             getattr(self, k).copy_(sd[k])
         self.episode, self.seed = int(sd["episode"]), int(sd["seed"])

@@ -749,7 +749,8 @@ int ia2c_seat_partners(const ia2c_episode_desc* d, const ia2c_runs_desc* r, cons
  *           inverse-CDF sampler as with its own row (if a seat repeats, the lowest j wins).  Nothing of the run's own state is
  *           read or written for this: the partner seats' own actor rows are never used to act while the mode is on, yet they
  *           receive the episode's updates as every seat does (their critics, beliefs and Adam state are trained on the
- *           partners' actions).  A run that leaves the mode continues self-play from those rows.
+ *           partners' actions).  A run that leaves the mode continues self-play from those rows.  To keep them as they are,
+ *           train with the partner seats frozen (ia2c_train_episode_frozen, below).
  *   guard   an env whose drawn team has a row outside [0, P), or whose seats have one outside [0, N), plays the run's own rows
  *           in every seat and logs -1; other envs are unaffected.
  *   log     log_env_team[r * E + e] = the drawn team, or -1 (out i32[R, E], written by the rollout kernel).
@@ -840,6 +841,43 @@ int ia2c_train_episode_env_partners_prioritized(const ia2c_episode_desc* d, cons
 int ia2c_record_partner_returns(const ia2c_episode_desc* d, const int32_t* env_team, const ia2c_partner_priority_desc* w,
                                 void* stream);
 int ia2c_prioritize_partners(const ia2c_partner_priority_desc* w, int32_t power, double floor_weight, int32_t reset, void* stream);
+
+/* ------------------------------------------------------------------ frozen seats -- */
+/* Trains an episode with some seats frozen: a frozen seat acts (with its own actor row, a row seated by ia2c_seat_partners
+ * before the call, or its env's pool row), but nothing of it is updated and the update kernels skip it.  With the partner
+ * seats frozen this is training against truly frozen partners; with no pool it trains a best response to fixed co-players.
+ *
+ * Definitions (R runs of N agents, the same mask for every run; `r` NULL is one standalone run):
+ *   mask        bit n of mask[n >> 6] set: seat n is frozen.  No bit at or above N; at least one seat frozen and one trained.
+ *   trained     every byte of every buffer of a trained seat, and the trajectory, ep_return, env state and partner logs, are
+ *               what the same entry point computes with nothing frozen: a seat's critic, actor gradient and beliefs read only
+ *               the trajectory and that seat's own rows.
+ *   frozen      net n = run * N + seat of a frozen seat: actor_params, critic_params, actor_grad, critic_grad, actor_m / v,
+ *               critic_m / v, actor_step, critic_step and actor_grad_accum are byte-unchanged (ia2c_seat_partners, before the
+ *               call, writes actor rows as it always does); loss_out[0, n] and loss_out[1, n] are NaN.
+ *   beliefs     N <= 8: the fused rollout runs every seat's filter as before, so a frozen seat's belief records and
+ *               partner_pred are what they are with nothing frozen.  9 <= N <= 256: the whole-episode belief kernel skips
+ *               frozen rows: their records are untouched and their partner_pred entries (all T + 1 steps) are 0xFF, "no
+ *               prediction"; a standalone episode with parity dumps writes no pred_dump / belief_dump entry of theirs either
+ *               (those slots keep what they held).
+ * Paths: those with whole-episode kernels.  Standalone: N <= 8 with IA2C_FLAG_FUSED_ROLLOUT (with or without
+ * IA2C_FLAG_FUSED_CRITIC), 9 <= N <= 256 with the whole-episode rollout and belief kernels; both with IA2C_FLAG_ACTOR_COLUMNS.
+ * Batches: ia2c_train_episode_runs (N <= 8) and ia2c_train_episode_runs_many (9 <= N <= 256).  p (the per-env pool) and w
+ * (prioritized draws; needs p) may be NULL, as for ia2c_train_episode_env_partners(_prioritized).  The launches are those of
+ * the unfrozen entry point (4 at N <= 8, 6 at 9..256); ia2c_seat_partners before and ia2c_record_partner_returns after the
+ * call stay the caller's.  Kernels: instantiations of the gradient, reduce and whole-episode belief kernels over the trained
+ * seats, whose list the entry point builds from the mask and passes by value; each trained net keeps the partition and the
+ * partial rows of the unfrozen episode, so its fixed-order sums are the same sums.
+ * Refusals, all before the first CUDA call.  IA2C_ERR_INVALID: a NULL mask, a bit at or above N, no seat frozen or none
+ * trained, and whatever the unfrozen entry point refuses.  IA2C_ERR_UNSUPPORTED: IA2C_FLAG_SKIP_ADAM or IA2C_FLAG_GRAD_ONLY,
+ * a multi-GPU shard (env_offset != 0 or E_total != E), IA2C_FLAG_ROLLOUT_PER_STEP or IA2C_FLAG_BELIEF_PER_STEP, N <= 8
+ * without IA2C_FLAG_FUSED_ROLLOUT or a fused instantiation, N > 256 or no whole-episode belief kernel, the pipelined actor
+ * kernel (no IA2C_FLAG_ACTOR_COLUMNS), and injected tapes in a batch. */
+typedef struct ia2c_frozen_seats {
+    uint64_t mask[4];                 /* host memory: bit n set, seat n frozen (N <= 256) */
+} ia2c_frozen_seats;
+int ia2c_train_episode_frozen(const ia2c_episode_desc* d, const ia2c_runs_desc* r, const ia2c_env_partner_desc* p,
+                              const ia2c_partner_priority_desc* w, const ia2c_frozen_seats* f, void* stream);
 
 #ifdef __cplusplus
 }
